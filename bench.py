@@ -1,7 +1,7 @@
 """Benchmark of the per-frame arm-pose estimation hot path (BASELINE.json's metric: MC-sampled arm-pose
 estimates/sec at 1/2/4/8 B200 vs the reference CPU path, and % of roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload (configs[2] of BASELINE.json, the largest single-GPU configuration and the one the throughput metric
@@ -21,6 +21,9 @@ random-init weights.  One step = one frame of every stream = 1024 estimates per 
   cpu_baseline / --impl reference: the oracle's restatement of the reference CPU path (torch.nn.LSTM on the CPU +
              numpy FK, exactly the arithmetic the reference executes) timed on this box's host cores: all cores
              (one single-stream process per core) and a single process with torch's default threads.
+
+--dump-outputs DIR writes what the last timed step of the device-resident leg returned (msg, std, samples, status of rank 0's
+streams) as DIR/<name>.npy in float32: inputs, weights and Philox seed are fixed, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -377,12 +380,14 @@ def run_ours(args, rank, world, local_rank):
         step_ev = []
         ev0.record()
         for f in range(W, W + K):
-            be.step_device(frames_dev[f], raw_ready=True)     # inputs resident in HBM before the timed region
+            last = be.step_device(frames_dev[f], raw_ready=True)     # inputs resident in HBM before the timed region
             if DEBUG_STEPS:
                 step_ev.append(torch.cuda.Event(enable_timing=True))
                 step_ev[-1].record()
         ev1.record()
         barrier()
+    # (copied now: the legs below reuse the estimator's output buffers)
+    dumped = last.host() if args.dump_outputs and rank == 0 else None
     if DEBUG_STEPS:                                           # APE_BENCH_DEBUG=1: completion time of every step of the timed region, per rank
         print(f"rank {rank}: total {ev0.elapsed_time(ev1):.3f} ms; step completions (ms): "
               + " ".join(f"{ev0.elapsed_time(e):.3f}" for e in step_ev), file=sys.stderr, flush=True)
@@ -491,10 +496,21 @@ def run_ours(args, rank, world, local_rank):
                                 "sample": f"{workers} single-stream worker processes (1 thread each) x {args.cpu_frames} frames of the "
                                           f"{args.workload} workload (n={n}); torch.nn.LSTM on CPU + numpy FK; {wall:.1f} s of CPU work",
                                 "single_process": cpu_single_process(kind, n, smooth, 100)}
+    if dumped is not None:
+        dump_outputs(Path(args.dump_outputs), dumped)
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, res):
+    """The arrays of one EstimateBatch as <name>.npy, float32 (status: 0 / 1 flags)."""
+    arrays = {"msg": res.msg, "std": res.std, "samples": res.samples, "status": res.status}
+    assert sum(a.size * 4 for a in arrays.values()) <= 64 << 20, "outputs exceed 64 MB"
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out_dir / f"{name}.npy", np.ascontiguousarray(a, dtype=np.float32))
 
 
 def ffma_peak_fields(N, torch, achieved):
@@ -843,7 +859,12 @@ def main():
     ap.add_argument("--sustained-seconds", type=float, default=2.0)
     ap.add_argument("--no-relabel", action="store_true", help="skip the BASELINE configs[3] relabelling leg")
     ap.add_argument("--lstm", default="auto", choices=["auto", "fp32", "tc"], help="LSTM kernel variant (auto: probe-gated tensor cores)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results: not with --impl reference")
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     # stdout carries the ONE JSON line and nothing else: whatever libraries write to file descriptor 1 (NCCL prints its
