@@ -640,7 +640,8 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
     using namespace ape;
     int rc = check_lstm_args(g);
     if (rc != APE_OK) return rc;
-    if (g->tc_flags == 3) return ape::tcx::run(g, (cudaStream_t)stream);      // split-precision variant (csrc/ape_lstm_tcx.cu)
+    if (g->tc_flags == 3)                                      // split-precision variant (csrc/ape_lstm_tcx.cu, H = 256: ape_lstm_tcxs.cu)
+        return g->H == 256 ? ape::tcxs::run(g, (cudaStream_t)stream) : ape::tcx::run(g, (cudaStream_t)stream);
     if (!ape_mc_lstm_tc_supported(g->I, g->H, g->L, g->O)) return APE_ERR_UNSUPPORTED;
     if (g->all_steps && (g->layer_begin != 0 || g->layer_end != 0)) return APE_ERR_UNSUPPORTED;
     if (g->h0 || g->c0) return APE_ERR_UNSUPPORTED;            // a caller-supplied initial state runs on the fp32 path

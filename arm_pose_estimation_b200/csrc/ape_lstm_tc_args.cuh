@@ -160,4 +160,13 @@ int run(const ape_lstm_args* g, cudaStream_t st);    // all layers of a call (ap
 size_t blob_bytes(int I, int L);
 size_t workspace_bytes(int L, int T, long long E, int n_samples);
 }  // namespace tcx
+
+namespace tcxs {
+// split-precision kernel for H = 256 (ape_lstm_tcxs.cu): the arithmetic and blob layout of tcx, h_t staged through L2 into
+// single-buffered TMEM operands
+bool supported(int H, int I, int O);
+int run(const ape_lstm_args* g, cudaStream_t st);    // all layers of a call (ape_mc_lstm_tc with tc_flags == 3, H = 256)
+size_t blob_bytes(int I, int L);
+size_t workspace_bytes(int L, int T, long long E, int n_samples);
+}  // namespace tcxs
 }  // namespace ape

@@ -42,7 +42,8 @@ extern "C" int ape_pipeline_create(const ape_pipeline_desc* d, ape_pipeline** ou
     for (int s = 0; s < d->n_slots; ++s)
         if (!d->out_dev[s] || !d->raw_host[s] || !d->out_host[s]) return APE_ERR_BAD_ARG;
     if (d->lstm.mask_mode == APE_MASK_INJECTED) return APE_ERR_UNSUPPORTED;      // injected masks change per call: the caller's path
-    if (!(split ? ape_mc_lstm_tcx_supported(d->lstm.I, d->lstm.H, d->lstm.L, d->lstm.O)
+    if (!(split ? (ape_mc_lstm_tcx_supported(d->lstm.I, d->lstm.H, d->lstm.L, d->lstm.O) ||
+                   ape_mc_lstm_tcxs_supported(d->lstm.I, d->lstm.H, d->lstm.L, d->lstm.O))
                 : ape_mc_lstm_tc_supported(d->lstm.I, d->lstm.H, d->lstm.L, d->lstm.O))) return APE_ERR_UNSUPPORTED;
     ape_pipeline* p = new (std::nothrow) ape_pipeline();
     if (!p) return APE_ERR_BAD_ARG;

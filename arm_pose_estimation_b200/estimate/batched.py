@@ -190,8 +190,9 @@ class BatchedEstimator:
             # Tensor cores when the fp16-operand result stays within tc_tolerance_m of the fp32 kernel on a probe batch of
             # THIS model's weights (and the batch has at least tc_min_rows rows: the measured crossover against the fp32
             # kernel is below one row - profiles/r1_crossover.md - so the default does not restrict).
-            # "tcx" = the split-precision tensor-core kernel (csrc/ape_lstm_tcx.cu, H = 128): fp16 pairs hi + lo, three passes per product,
-            # ex2 / rcp cell update - what "auto" takes when the single-pass probe fails, before it falls back to the fp32 kernel.
+            # "tcx" = the split-precision tensor-core kernels (csrc/ape_lstm_tcx.cu, H = 128; csrc/ape_lstm_tcxs.cu, H = 256): fp16 pairs
+            # hi + lo, three passes per product, ex2 / rcp cell update - what "auto" takes when the single-pass probe fails, before it
+            # falls back to the fp32 kernel.
             self.tc_weights = self.tcx_weights = None
             self.tc_probe_error_m = self.tcx_probe_error_m = None
             self.tc_split = False
@@ -199,7 +200,7 @@ class BatchedEstimator:
             if lstm_variant not in ("auto", "fp32", "tc", "tcx"):
                 raise UserWarning(f"lstm_variant must be 'auto', 'fp32', 'tc' or 'tcx', got {lstm_variant!r}")
             tc_ok = N.tc_supported(self.I, self.H, self.L, self.O) and self.T <= 40
-            tcx_ok = N.tcx_supported(self.I, self.H, self.L, self.O) and self.T <= 40
+            tcx_ok = N.split_supported(self.I, self.H, self.L, self.O) and self.T <= 40
             if lstm_variant == "tc" and not tc_ok:
                 raise UserWarning(f"the tensor-core LSTM kernel does not support H={self.H}, L={self.L}")
             if lstm_variant == "tcx" and not tcx_ok:
@@ -216,11 +217,11 @@ class BatchedEstimator:
                     self.lstm_variant = "tc"
             if lstm_variant == "tcx" or (lstm_variant == "auto" and self.lstm_variant != "tc" and tcx_ok and B * nF * self.n >= tc_min_rows):
                 self.tcx_weights = torch.from_numpy(nn_models.pack_lstm_weights_tcx(state)).to(dev)
-                assert self.tcx_weights.numel() == N.tcx_blob_bytes(self.I, self.H, self.L)
+                assert self.tcx_weights.numel() == N.split_blob_bytes(self.I, self.H, self.L)
                 self.tcx_probe_error_m = self._probe_tc_error("tcx")
                 if lstm_variant == "tcx" or self.tcx_probe_error_m <= tc_tolerance_m:
                     self.lstm_variant, self.tc_split, self.tc_flags = "tc", True, 3
-                    ws_x = N.tcx_workspace_bytes(self.I, self.H, self.L, self.T, self.O, B * nF, self.n) + 1024
+                    ws_x = N.split_workspace_bytes(self.I, self.H, self.L, self.T, self.O, B * nF, self.n) + 1024
                     if ws_x > self.workspace.numel():
                         self.workspace = torch.empty(ws_x, dtype=torch.uint8, device=dev)
             # A call of <= 128 rows (one stream x 100 MC samples: the real-time case) can run ALL layers in one launch of one 8-CTA cluster
@@ -345,7 +346,7 @@ class BatchedEstimator:
         g = torch.Generator(device="cpu").manual_seed(1234)
         x = torch.randn((n_est, self.T, self.I), generator=g, dtype=torch.float32).to(dev)
         ws = torch.empty(max(N.workspace_bytes(self.I, self.H, self.L, self.T, self.O, n_est, n_samples),
-                             N.tcx_workspace_bytes(self.I, self.H, self.L, self.T, self.O, n_est, n_samples) if which == "tcx" else
+                             N.split_workspace_bytes(self.I, self.H, self.L, self.T, self.O, n_est, n_samples) if which == "tcx" else
                              N.workspace_bytes(self.I, self.H, self.L, self.T, self.O, n_est, n_samples, tensor_core=True)),
                          dtype=torch.uint8, device=dev)
         outs = []

@@ -123,18 +123,19 @@ def pack_lstm_weights_tc(state):
 
 
 def pack_lstm_weights_tcx(state):
-    """Reference state dict -> the blob of the SPLIT-PRECISION tensor-core kernel (``csrc/ape_lstm_tcx.cu``, H = 128), as uint8 bytes.
+    """Reference state dict -> the blob of the SPLIT-PRECISION tensor-core kernels (``csrc/ape_lstm_tcx.cu``, H = 128, and
+    ``csrc/ape_lstm_tcxs.cu``, H = 256: the same layout at either width), as uint8 bytes.
 
     Every weight enters as an fp16 pair ``hi = fp16(w)``, ``lo = fp16(w - hi)``; the i, f, o columns are halved first (exact), so the
     accumulator is the ex2 argument of the cell update up to one constant.  Per layer, CTA ``r`` of the pair and 32-unit chunk ``c``
     (gate columns as in ``pack_lstm_weights_tc``) four K-major tiles ``[k-group][64][8]``: ``Wx_hi`` with one extra K = 16 step whose
     rows 0 and 1 hold the scaled bias as an fp16 pair (the kernel multiplies it by a tile of ones), ``Wx_lo``, ``Wh_hi``, ``Wh_lo``.
-    After all layers the output layer as in ``pack_lstm_weights_tc`` (fp16 rounding and remainder, 16 columns)."""
+    After all layers the output layer as in ``pack_lstm_weights_tc`` (fp16 rounding and remainder, 16 columns; 32 for H = 256)."""
     st = {k: np.asarray(v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else v, dtype=np.float32)
           for k, v in state.items()}
     I, H, L, O = lstm_dims(st)
-    if H != 128:
-        raise UserWarning("the split-precision tensor-core kernel takes H = 128")
+    if H not in (128, 256):
+        raise UserWarning("the split-precision tensor-core kernels take H = 128 or 256")
     parts, nl = [], np.arange(64)
 
     def tiles(w):                                                  # [cols, K] fp32 -> (hi, lo) K-major uint8 tiles
@@ -165,8 +166,9 @@ def pack_lstm_weights_tcx(state):
                 p1 = tiles(wx[:, : kin_pad])[1]
                 wh_hi, wh_lo = tiles(w_hh[rows] * scale)
                 parts += [p0, p1, wh_hi, wh_lo]
-    w_full = np.zeros((16, H), np.float32)
-    w_full[: min(O, 16)] = st["output_layer.weight"][:16]
+    n_cols = 32 if H > 128 else 16
+    w_full = np.zeros((n_cols, H), np.float32)
+    w_full[: min(O, n_cols)] = st["output_layer.weight"][:n_cols]
     for t in tiles(w_full):
         parts.append(t)
     return np.ascontiguousarray(np.concatenate(parts))

@@ -142,7 +142,8 @@ typedef struct ape_lstm_args {
     /* tensor-core path, H = 128, L >= 3: how consecutive layers >= 1 are launched.  0 = automatic (a pair of layers runs as ONE
        two-layer wavefront launch, csrc/ape_lstm_tcw.cu, when the batch fills the GPU), 1 = one launch per layer always,
        2 = wavefront pairs always, 3 = the SPLIT-PRECISION variant (every operand an fp16 pair hi + lo, three tensor-core passes per
-       product, ex2 / rcp cell update: fp32-grade results at ~1/2 of the single-pass throughput; needs weights_tcx),
+       product, ex2 / rcp cell update: fp32-grade results at ~0.4 of the single-pass throughput; needs weights_tcx; H = 128:
+       csrc/ape_lstm_tcx.cu, H = 256: csrc/ape_lstm_tcxs.cu),
        4 = the SMALL-BATCH kernel (csrc/ape_lstm_tcl.cu: B * nF * n_samples <= 8192 rows, L <= 4: all layers in one launch, one
        8-CTA cluster per 128 rows with the hidden units split across it - the real-time case of one to a few dozen streams; same
        arithmetic as 0..2) */
@@ -156,8 +157,9 @@ typedef struct ape_lstm_args {
        few CTAs of stage 1 + layer 0 of the NEXT call (a high-priority side stream, ape_pipeline_submit) start at once instead of
        waiting for a persistent launch to retire CTAs; 0 = use every SM */
     int reserve_sms;
-    /* split-precision tensor-core variant (tc_flags == 3; csrc/ape_lstm_tcx.cu, H = 128): its weight blob, packed by
-       pack_lstm_weights_tcx() (ape_lstm_tcx_blob_bytes() bytes); the workspace must then hold ape_mc_lstm_tcx_workspace_bytes() */
+    /* split-precision tensor-core variant (tc_flags == 3; csrc/ape_lstm_tcx.cu, H = 128, or csrc/ape_lstm_tcxs.cu, H = 256): its
+       weight blob, packed by pack_lstm_weights_tcx() (ape_lstm_tcx_blob_bytes() / ape_lstm_tcxs_blob_bytes() bytes); the workspace
+       must then hold ape_mc_lstm_tcx_workspace_bytes() / ape_mc_lstm_tcxs_workspace_bytes() */
     const void* weights_tcx;
 } ape_lstm_args;
 
@@ -181,6 +183,12 @@ int ape_mc_lstm_tc(const ape_lstm_args* args, void* stream);
 int ape_mc_lstm_tcx_supported(int I, int H, int L, int O);
 int ape_lstm_tcx_blob_bytes(int I, int H, int L, int64_t* bytes);
 int ape_mc_lstm_tcx_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes);
+/* the same for the H = 256 split-precision kernel (csrc/ape_lstm_tcxs.cu; H = 256, I <= 256, O <= 32, L >= 2), which tc_flags == 3
+   selects for an H = 256 model: its blob (packed by pack_lstm_weights_tcx() as well, the same layout at H = 256) also travels in
+   weights_tcx, and the workspace must hold ape_mc_lstm_tcxs_workspace_bytes() */
+int ape_mc_lstm_tcxs_supported(int I, int H, int L, int O);
+int ape_lstm_tcxs_blob_bytes(int I, int H, int L, int64_t* bytes);
+int ape_mc_lstm_tcxs_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes);
 /* number of kernels ape_mc_lstm_tc launches for these arguments (layer pairs of an H = 128 model count once) */
 int ape_mc_lstm_tc_launch_count(const ape_lstm_args* args, int* launches);
 /*
