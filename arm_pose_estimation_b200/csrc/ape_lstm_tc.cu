@@ -78,7 +78,10 @@ constexpr uint32_t BAR_BLOCK_BYTES = 256;          // barriers + the TMEM base s
 
 __device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 1, %0;" ::"n"(EPI_THREADS) : "memory"); }
 
-template <int H>
+// STATE: a caller-supplied initial state (a.h0, a.c0).  Step 0 of every tile then runs like every later step - x-part, then the
+// recurrent half on h_0 - and the cell starts from c_0; the x-part MMAs keep their order, so h_0 = c_0 = 0 reproduces the
+// stateless kernel bit for bit (the recurrent products only add +0 to the fp32 accumulators).
+template <int H, bool STATE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_layer_tc_kernel(TcLayerArgs a) {
     using namespace umma;
     constexpr int NCH = H / 32, KG = H / 8;
@@ -154,6 +157,31 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
             for (int c = 0; c < NCH; ++c)
 #pragma unroll
                 for (int u = 0; u < 8; ++u) cst[c][u] = 0.0f;
+            if constexpr (STATE) {
+                // h_0 into the operand tile step 0 reads (tile 0), c_0 into the registers.  The tile is free: this warp has drained
+                // every accumulator of the previous tile's last step (and waited for its output product), so every MMA that read
+                // an h tile of that tile has retired.
+                if (warp_live) {
+                    const float4* h0r = reinterpret_cast<const float4*>(a.h0 + (size_t)(valid ? row : 0) * H);
+                    const float4* c0r = reinterpret_cast<const float4*>(a.c0 + (size_t)(valid ? row : 0) * H);
+#pragma unroll
+                    for (int c = 0; c < NCH; ++c) {
+                        const int j = 4 * c + s;
+                        const float4 z = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+                        const float4 h_a = valid ? __ldg(h0r + 2 * j) : z, h_b = valid ? __ldg(h0r + 2 * j + 1) : z;
+                        const float4 c_a = valid ? __ldg(c0r + 2 * j) : z, c_b = valid ? __ldg(c0r + 2 * j + 1) : z;
+                        cst[c][0] = c_a.x; cst[c][1] = c_a.y; cst[c][2] = c_a.z; cst[c][3] = c_a.w;
+                        cst[c][4] = c_b.x; cst[c][5] = c_b.y; cst[c][6] = c_b.z; cst[c][7] = c_b.w;
+                        *reinterpret_cast<uint4*>(sAh + unit_offset(ROWS, row_l, j)) =
+                            make_uint4(pack_half2(h_a.x, h_a.y), pack_half2(h_a.z, h_a.w), pack_half2(h_b.x, h_b.y), pack_half2(h_b.z, h_b.w));
+                    }
+                }
+                fence_proxy_async_smem();
+                __syncwarp();
+                if (lane == 0)
+#pragma unroll
+                    for (int c = 0; c < NCH; ++c) mbar_arrive_leader(&bars[BAR_H_READY + c], rank);
+            }
 
             for (int t = 0; t < T; ++t) {
                 uint8_t* sAh_next = sAh + ((t + 1) & 1) * A_BYTES;
@@ -243,7 +271,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
 #pragma unroll
                         for (int u = 0; u < 4; ++u) {
                             cst[c][4 * half + u] = num[u] * den[u];
-                            num[u] = ex2_approx(cst[c][4 * half + u] * (-2.0f * LOG2E));   // e_c = 2^(-2c log2e), |c| <= T: no overflow
+                            // e_c = 2^(-2c log2e): |c| <= T, no overflow; with a state |c| <= |c_0| + T, clamped
+                            const float pc = cst[c][4 * half + u] * (-2.0f * LOG2E);
+                            num[u] = ex2_approx(STATE ? fminf(pc, EX2_CLAMP) : pc);
                         }
 #pragma unroll
                         for (int u = 0; u < 4; ++u) hv[u] = (1.0f - num[u]) * rcp_approx((1.0f + ev[4 * u + 3]) * (1.0f + num[u]));
@@ -442,6 +472,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
                 ph_xready ^= 1;
                 fence_after_sync();
                 APE_TRACE(2, t, 1);
+                if (STATE && out_pending) {                     // (t == 0) the previous tile's output layer goes first: the
+                    mbar_wait(&bars[BAR_SLOT_FREE + NCH - 1], ph_slot);   // epilogue publishes h_0 only after it has read those outputs
+                    fence_after_sync();
+                    issue_output();
+                }
                 const uint64_t dH = desc_advance(dH0, (t & 1) * A_BYTES);
 #pragma unroll
                 for (int c = 0; c < NCH; ++c) {
@@ -452,9 +487,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
                         const uint64_t wx = desc_advance(dW, c * chunk_bytes);
                         for (int k2 = 0; k2 < kgx / 2; ++k2)
                             mma_f16<2>(tmem + c * 128, desc_advance(dX, k2 * 2 * LBO_A), desc_advance(wx, k2 * 2 * LBO_B), idesc, k2 > 0 ? 1u : 0u);
-                        if (t == 0) commit_pair(&bars[BAR_ACC_READY + c], 0x3);  // h_{-1} = 0: no recurrent half
+                        if (t == 0 && !STATE) commit_pair(&bars[BAR_ACC_READY + c], 0x3);  // h_{-1} = 0: no recurrent half
                         if (c == NCH - 1) commit_pair(&bars[BAR_X_DONE], 0x3);
-                        if (t > 0) {
+                        if (t > 0 || STATE) {
                             const uint64_t wh = desc_advance(wx, (uint32_t)kgx * KG_BYTES_B);
 #pragma unroll
                             for (int cs = 0; cs < c; ++cs)                       // slices published before this chunk drained
@@ -465,7 +500,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
                     }
                     __syncwarp();
                     APE_TRACE(2, t, 3 + 3 * c);
-                    if (t > 0) {
+                    if (t > 0 || STATE) {
                         mbar_wait(&bars[BAR_H_READY + c], ph_hready);           // slice c of h_{t-1}
                         fence_after_sync();
                         APE_TRACE(2, t, 4 + 3 * c);
@@ -484,7 +519,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
                 }
                 APE_TRACE(2, t, 14);
                 if (!first) ph_slot ^= 1;
-                if (t > 0) ph_hready ^= 1;
+                if (t > 0 || STATE) ph_hready ^= 1;
                 first = false;
             }
             out_pending = a.preds != nullptr;
@@ -534,10 +569,11 @@ template <int H> static size_t smem_bytes(int kgx) {
 
 template <int H> static int launch(const TcLayerArgs& a, int sm_count, cudaStream_t st) {
     const size_t smem = smem_bytes<H>(a.kgx);
-    APE_CUDA_TRY(cudaFuncSetAttribute(lstm_layer_tc_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    auto kernel = a.h0 ? lstm_layer_tc_kernel<H, true> : lstm_layer_tc_kernel<H, false>;
+    APE_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int clusters = sm_count / 2;
     if (clusters > a.n_pair_tiles) clusters = a.n_pair_tiles;
-    lstm_layer_tc_kernel<H><<<2 * clusters, THREADS, smem, st>>>(a);
+    kernel<<<2 * clusters, THREADS, smem, st>>>(a);
     return check_launch();
 }
 
@@ -615,8 +651,9 @@ extern "C" int ape_mc_lstm_tc_workspace_bytes_all_steps(int I, int H, int L, int
     return APE_OK;
 }
 
+// (a caller-supplied initial state runs on the one-layer kernels: the wavefront kernel takes none)
 static bool tc_pairs_layers(const ape_lstm_args* g, long long tiles1, int sm_count) {
-    return ape::tcw::supported(g->H, g->T, g->O) && g->tc_flags != 1 && (g->tc_flags == 2 || tiles1 >= sm_count / 2);
+    return ape::tcw::supported(g->H, g->T, g->O) && g->tc_flags != 1 && g->h0 == nullptr && (g->tc_flags == 2 || tiles1 >= sm_count / 2);
 }
 
 // kernels ape_mc_lstm_tc will launch for these arguments (bench.py's gpu_launches; depends on the pairing rule above)
@@ -638,14 +675,18 @@ extern "C" int ape_mc_lstm_tc_launch_count(const ape_lstm_args* g, int* launches
 
 extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
     using namespace ape;
-    int rc = check_lstm_args(g);
+    int rc = check_lstm_args(g);                               // (h0 / c0: both or neither, and n_samples == 1)
     if (rc != APE_OK) return rc;
+    // an initial state runs on the one-layer kernels (tc_flags 0 and 1); the wavefront, split-precision and small-batch kernels take none
+    if (g->h0 && (g->tc_flags == 2 || g->tc_flags == 3 || g->tc_flags == 4)) return APE_ERR_UNSUPPORTED;
+    // the state kernels read h_0 / c_0 rows as float4 (H is a multiple of 32, so every layer's block keeps the base alignment)
+    if (((uintptr_t)g->h0 | (uintptr_t)g->c0) & 15) return APE_ERR_BAD_ARG;
     if (g->tc_flags == 3)                                      // split-precision variant (csrc/ape_lstm_tcx.cu, H = 256: ape_lstm_tcxs.cu)
         return g->H == 256 ? ape::tcxs::run(g, (cudaStream_t)stream) : ape::tcx::run(g, (cudaStream_t)stream);
     if (!ape_mc_lstm_tc_supported(g->I, g->H, g->L, g->O)) return APE_ERR_UNSUPPORTED;
     if (g->all_steps && (g->layer_begin != 0 || g->layer_end != 0)) return APE_ERR_UNSUPPORTED;
-    if (g->h0 || g->c0) return APE_ERR_UNSUPPORTED;            // a caller-supplied initial state runs on the fp32 path
     if (g->T > 40) return APE_ERR_UNSUPPORTED;                 // |c_t| <= t keeps 2^(2 c log2e) finite in fp32 only for T <= 44
+                                                               // (with a state |c_t| <= |c_0| + t: the state kernels clamp it)
     if (!g->weights_tc) return APE_ERR_BAD_ARG;
     const long long E = (long long)g->B * g->nF;
     if (E == 0) return APE_OK;
@@ -754,6 +795,8 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
         a.preds = (last && !all_steps) ? g->preds : nullptr;
         a.pred_ring = g->pred_ring; a.n_out = g->n_samples;
         a.cstate = scratch_region ? (float*)(scratch + (l == 0 ? 0 : scratch_region)) : nullptr;
+        a.h0 = g->h0 ? g->h0 + (size_t)l * E * H : nullptr;   // [L][E][H]: with a state every layer has E rows (n_samples == 1)
+        a.c0 = g->c0 ? g->c0 + (size_t)l * E * H : nullptr;
         a.trace = (g->trace && l == g->trace_layer) ? (long long*)g->trace : nullptr;
         // trace_layer < 0: the CTA timeline of every layer instead, [layer][TC_MAX_SMS CTAs][4]
         a.timeline = (g->trace && g->trace_layer < 0) ? (long long*)g->trace + (size_t)l * TC_MAX_SMS * 4 : nullptr;

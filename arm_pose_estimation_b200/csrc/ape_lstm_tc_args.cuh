@@ -47,6 +47,8 @@ struct TcLayerArgs {
     int pred_ring, n_out;
     int n_pair_tiles;
     float* cstate;             // streamed-weights kernel (H = 256): per-CTA cell-state scratch, tcs::scratch_bytes() bytes
+    const float* h0;           // caller-supplied initial state of THIS layer, [rows][H] float32 each (n == 1), or both null:
+    const float* c0;           //   step 0 of every tile then also runs the recurrent half on h_0 and starts the cell from c_0
     long long* trace;          // debugging: null, or [3 roles][16 steps][16 events] SM-clock stamps of the first tile of CTA 0
     long long* timeline;       // debugging: null, or [CTA][4] = {globaltimer at entry, after the set-up, at exit; SM id} (tools/lanes_timeline.py)
 };
@@ -130,7 +132,7 @@ namespace tcs {
 // streamed-weights kernel (ape_lstm_tcs.cu)
 bool supported(int H);
 size_t scratch_bytes(int H, int sm_count);      // one region of per-CTA cell-state scratch (a launch needs one)
-int launch_layer(int H, const tc::TcLayerArgs& a, int sm_count, cudaStream_t st);
+int launch_layer(int H, const tc::TcLayerArgs& a, int sm_count, cudaStream_t st);    // a.h0 / a.c0: the state variant
 }  // namespace tcs
 
 namespace tcw {

@@ -119,13 +119,31 @@ template <int H> struct Cfg {
 //   acc_done(c) / x_done()              chunk c complete / this slot's share of the x tile has been consumed
 //   out_point()                         (first step of a tile) before the next piece: the output layer of the PREVIOUS tile, one
 //                                       extra ring piece (the W_o tile) multiplied by that tile's h_T into accumulator slot 1
+// Three kinds of step, which index the schedule table: the first step of a tile without an initial state (h_{-1} = 0), a later
+// step, and the first step of a tile with a caller-supplied h_0.
+enum StepKind { STEP_FIRST = 0, STEP_LATER = 1, STEP_FIRST_STATE = 2, N_STEP_KINDS = 3 };
 template <int NCH, class V>
-static void walk_step(bool first_step, int kgx, V& v) {
+static void walk_step(int kind, int kgx, V& v) {
     const int KG = NCH * SLICE_KG;
+    const bool first_step = kind == STEP_FIRST;
     auto range = [&](int c, bool is_h, int kg_lo, int kg_hi, bool first) {      // [kg_lo, kg_hi) in pieces of <= PIECE_KG
         for (int kg0 = kg_lo; kg0 < kg_hi; kg0 += PIECE_KG)
             v.piece(c, is_h, kg0, kg_hi - kg0 < PIECE_KG ? kg_hi - kg0 : PIECE_KG, first && kg0 == kg_lo);
     };
+    if (kind == STEP_FIRST_STATE) {
+        // Every chunk takes its x-part exactly as in STEP_FIRST, then the whole recurrent part on h_0.  The epilogue publishes h_0
+        // only after it has read the previous tile's outputs, so the output piece and both x-parts it sits between go ahead of
+        // the first recurrent piece, in the ring as in the issue order.
+        for (int c = 0; c < NCH; ++c) {
+            v.chunk_begin(c);
+            if (c == 1) v.out_point();
+            range(c, false, 0, kgx, true);
+            if (c >= NCH - NSLOT) v.x_done();
+            if (c == 1) { range(0, true, 0, KG, false); v.acc_done(0); }
+            if (c >= 1) { range(c, true, 0, KG, false); v.acc_done(c); }
+        }
+        return;
+    }
     for (int c = 0; c < NCH; ++c) {
         v.chunk_begin(c);
         if (first_step && c == 1) v.out_point();               // slot 1 is free and the previous tile's h_T is complete by now
@@ -168,9 +186,9 @@ enum : uint32_t {
 };
 constexpr int MAX_ENTRIES = 48;
 
-struct Schedule {                                              // [0]: first step of a tile (no recurrent half), [1]: later steps
-    uint2 e[2][MAX_ENTRIES];                                   // .x see above; .y A-operand offset (x: descriptor units, h: TMEM columns)
-    uint32_t n[2];
+struct Schedule {                                              // indexed by StepKind
+    uint2 e[N_STEP_KINDS][MAX_ENTRIES];                        // .x see above; .y A-operand offset (x: descriptor units, h: TMEM columns)
+    uint32_t n[N_STEP_KINDS];
 };
 
 struct Recorder {
@@ -194,7 +212,9 @@ struct Recorder {
     void x_done() { if (n > 0) tab[n - 1].x |= E_POST_X; }
 };
 
-template <int H>
+// STATE: a caller-supplied initial state (a.h0, a.c0): h_0 goes into the h buffer step 0 reads, the cell starts from c_0 and step 0
+// follows the STEP_FIRST_STATE schedule; h_0 = c_0 = 0 reproduces the stateless kernel bit for bit.
+template <int H, bool STATE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_layer_tcs_kernel(const __grid_constant__ TcLayerArgs a, const __grid_constant__ Schedule sched) {
     using namespace umma;
     using C = Cfg<H>;
@@ -260,6 +280,28 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
         for (int tile = cluster_id; tile < a.n_pair_tiles; tile += n_clusters) {
             const int row = (tile * 2 + (int)rank) * a.rpc + row_l;
             const bool valid = row_l < a.rpc && row < a.rows;
+            const float4* c0r = STATE ? reinterpret_cast<const float4*>(a.c0 + (size_t)(valid ? row : 0) * H) : nullptr;
+            if constexpr (STATE) {
+                // h_0 as fp16 pairs into buffer 0 (the one step 0 reads).  Every MMA that read the buffer has retired: this warp has
+                // drained every accumulator of the previous tile's last step and waited for its output product.
+                if (warp_live) {
+                    const float4* h0r = reinterpret_cast<const float4*>(a.h0 + (size_t)(valid ? row : 0) * H);
+                    const float4 z = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+#pragma unroll
+                    for (int c = 0; c < NCH; ++c) {
+                        const int j = 4 * c + s;
+                        const float4 h_a = valid ? __ldg(h0r + 2 * j) : z, h_b = valid ? __ldg(h0r + 2 * j + 1) : z;
+                        tmem_st_x4(tmem + t_lane + H_COL + (uint32_t)(4 * j), pack_half2(h_a.x, h_a.y), pack_half2(h_a.z, h_a.w),
+                                   pack_half2(h_b.x, h_b.y), pack_half2(h_b.z, h_b.w));
+                    }
+                    tmem_st_wait();
+                }
+                fence_before_sync();
+                __syncwarp();
+                if (lane == 0)
+#pragma unroll
+                    for (int c = 0; c < NCH; ++c) mbar_arrive_leader(&bars[C::BAR_H_READY + c], rank);
+            }
 
             for (int t = 0; t < T; ++t, ++gstep) {
                 const uint32_t h_next = H_COL + (uint32_t)((t + 1) & 1) * H_COLS;     // TMEM columns that receive h_t
@@ -285,6 +327,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
                     cbuf[0] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
                     cbuf[1] = cbuf[0];
                     if (t > 0 && APE_EXP != 8) cbuf[0] = __ldcg(cst + (size_t)((4 * 0 + s) * 2 + 0) * ROWS);
+                    else if (STATE && valid) cbuf[0] = __ldg(c0r + 2 * s);
                     // The bias of half-pass hp+1 is requested at the end of half-pass hp's arithmetic, where few registers are live:
                     // its ~40 cycles of L1 latency used to sit in front of the first FMA of every half-pass (ncu: a fifth of the
                     // kernel's stall samples).
@@ -323,6 +366,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
                         if (hp + 1 < 2 * NCH) {
                             const int c1 = (hp + 1) >> 1, h1 = (hp + 1) & 1;
                             if (t > 0 && APE_EXP != 8) cbuf[(hp + 1) & 1] = __ldcg(cst + (size_t)((4 * c1 + s) * 2 + h1) * ROWS);
+                            else if (STATE && valid) cbuf[(hp + 1) & 1] = __ldg(c0r + 2 * (4 * c1 + s) + h1);
                             // Next chunk: its accumulators are prefetched under this half-pass IF the chunk is already complete -
                             // waiting for it here would tie the pass period to the refill latency of the two-slot ring (drain of
                             // chunk c -> chunk c+2 complete), so an unfinished chunk is waited for at the top of its own pass.
@@ -405,7 +449,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
 #pragma unroll
                         for (int u = 0; u < 4; ++u) {
                             cn[u] = num[u] * den[u];
-                            num[u] = ex2_approx(cn[u] * (-2.0f * LOG2E));   // e_c = 2^(-2c log2e), |c| <= T: no overflow
+                            // e_c = 2^(-2c log2e): |c| <= T, no overflow; with a state |c| <= |c_0| + T, clamped
+                            num[u] = ex2_approx(STATE ? fminf(cn[u] * (-2.0f * LOG2E), EX2_CLAMP) : cn[u] * (-2.0f * LOG2E));
                         }
 #pragma unroll
                         for (int u = 0; u < 4; ++u) hv[u] = (1.0f - num[u]) * rcp_approx((1.0f + ev[4 * u + 3]) * (1.0f + num[u]));
@@ -602,6 +647,11 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
                     mbar_wait_wd(&bars[C::BAR_OUT_DONE], ph_outdone);                  // every epilogue warp has read its outputs
                     ph_outdone ^= 1;
                     fence_after_sync();
+                } else if (STATE) {
+                    // Issuer 0's next H_READY wait (step 0 with a state) is for h_0, whose phase has the parity of the phase BEFORE h_T:
+                    // while h_T is still being published that wait would pass at once and the recurrent MMAs would read the h buffer
+                    // before h_0 is in it.  So it waits for h_T here as issuer 1 does.
+                    mbar_wait_wd(&bars[C::BAR_H_READY + NCH - 1], hphase);
                 }
                 hphase ^= 1;                                   // the last step of a final layer publishes h_T: one more H_READY phase
                 wslot = wslot + 1 == NP ? 0 : wslot + 1;
@@ -616,7 +666,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
                     TCS_TR(if (tr) tr[576] = clock64();)
                     const uint64_t dX = dX0 + xb * (C::A_BYTES >> 4);
                     const uint32_t h_prev = tmem + H_COL + (uint32_t)(t & 1) * H_COLS;   // TMEM columns of h_{t-1}
-                    const int which = t == 0 ? 0 : 1;
+                    const int which = t > 0 ? STEP_LATER : STATE ? STEP_FIRST_STATE : STEP_FIRST;
                     const uint32_t n_ent = sched.n[which];
                     uint32_t h_waited = 0;                     // K-slices of h_{t-1} seen so far in this step
                     uint2 e = sched.e[which][0];
@@ -701,7 +751,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
                         ++gpiece;
                         e = e_next;
                     }
-                    if (t > 0) hphase ^= 1;
+                    if (t > 0 || STATE) hphase ^= 1;
                 }
                 out_pending = a.preds != nullptr;
             }
@@ -717,7 +767,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
             bool out_pending = false;
             for (int tile = cluster_id; tile < a.n_pair_tiles; tile += n_clusters) {
                 for (int t = 0; t < T; ++t) {
-                    const int which = t == 0 ? 0 : 1;
+                    const int which = t > 0 ? STEP_LATER : STATE ? STEP_FIRST_STATE : STEP_FIRST;
                     const uint32_t n_ent = sched.n[which];
 #pragma unroll 1
                     for (uint32_t i = 0; i < n_ent; ++i) {
@@ -745,7 +795,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
         for (int tile = cluster_id; tile < a.n_pair_tiles; tile += n_clusters) {
             for (int t = 0; t < T; ++t) {
                 TCS_TR(long long* tr = (a.trace && blockIdx.x == 0 && tile == cluster_id && t == TRACE_T) ? a.trace : nullptr;)
-                const int which = t == 0 ? 0 : 1;
+                const int which = t > 0 ? STEP_LATER : STATE ? STEP_FIRST_STATE : STEP_FIRST;
                 const uint32_t n_ent = sched.n[which];
 #pragma unroll 1
                 for (uint32_t i = 0; i < n_ent; ++i, ++gpiece) {
@@ -787,18 +837,20 @@ int launch_layer(int H, const TcLayerArgs& a, int sm_count, cudaStream_t st) {
     using C = Cfg<256>;
     if (a.kgx < 2 || a.kgx > C::KG || (a.kgx & 1) || !a.cstate) return APE_ERR_UNSUPPORTED;
     if (a.preds && (!a.Wo16 || a.O > (int)C::OUT_N / 2)) return APE_ERR_UNSUPPORTED;
+    if ((a.h0 != nullptr) != (a.c0 != nullptr)) return APE_ERR_BAD_ARG;
     Schedule sched{};
-    for (int which = 0; which < 2; ++which) {
+    for (int which = 0; which < N_STEP_KINDS; ++which) {
         Recorder r{sched.e[which], 0, a.kgx, C::KG, 0u, false};
-        walk_step<C::NCH>(which == 0, a.kgx, r);
+        walk_step<C::NCH>(which, a.kgx, r);
         if (r.overflow) return APE_ERR_UNSUPPORTED;
         sched.n[which] = (uint32_t)r.n;
     }
     const size_t smem = C::SMEM;
-    APE_CUDA_TRY(cudaFuncSetAttribute(lstm_layer_tcs_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    auto kernel = a.h0 ? lstm_layer_tcs_kernel<256, true> : lstm_layer_tcs_kernel<256, false>;
+    APE_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int clusters = sm_count / 2;
     if (clusters > a.n_pair_tiles) clusters = a.n_pair_tiles;
-    lstm_layer_tcs_kernel<256><<<2 * clusters, THREADS, smem, st>>>(a, sched);
+    kernel<<<2 * clusters, THREADS, smem, st>>>(a, sched);
     return check_launch();
 }
 
@@ -806,14 +858,15 @@ int launch_layer(int H, const TcLayerArgs& a, int sm_count, cudaStream_t st) {
 }  // namespace ape
 
 // Host self-check hook (tests only): the step schedule of the streamed-weights kernel for an x-part of kgx k-groups.
+// first_step: 0 = a later step, 1 = the first step of a tile, 2 = the first step of a tile with a caller-supplied initial state.
 // entries: [n][2] words (.x flags / MMAs / K-slices needed / weight offset, .y A-operand offset), see the E_* bits above.
 extern "C" int ape_selfcheck_tcs_schedule(int kgx, int first_step, uint32_t* entries, int max_entries, int* n_entries) {
     using namespace ape::tcs;
     using C = Cfg<256>;
-    if (!entries || !n_entries || kgx < 2 || kgx > C::KG || (kgx & 1)) return APE_ERR_BAD_ARG;
+    if (!entries || !n_entries || kgx < 2 || kgx > C::KG || (kgx & 1) || first_step < 0 || first_step > 2) return APE_ERR_BAD_ARG;
     Schedule sched{};
     Recorder r{sched.e[0], 0, kgx, C::KG, 0u, false};
-    walk_step<C::NCH>(first_step != 0, kgx, r);
+    walk_step<C::NCH>(first_step == 0 ? STEP_LATER : first_step == 1 ? STEP_FIRST : STEP_FIRST_STATE, kgx, r);
     if (r.overflow || r.n > max_entries) return APE_ERR_UNSUPPORTED;
     for (int i = 0; i < r.n; ++i) { entries[2 * i] = sched.e[0][i].x; entries[2 * i + 1] = sched.e[0][i].y; }
     *n_entries = r.n;

@@ -205,10 +205,14 @@ class DropoutLSTM:
     ``lstm_variant``: ``"fp32"`` = the exact FFMA kernel, ``"tc"`` = the tcgen05 tensor-core kernels (fp16 operands, fp32
     accumulation and state), ``"auto"`` (default) = tensor cores when this model's shape is supported AND a probe on its own
     weights keeps the tensor-core outputs within ``tc_tolerance`` (normalised output units; 2e-4 is ~3e-5 m of hand position)
-    of the fp32 kernel's.  A caller-supplied ``hs`` always takes the fp32 kernel."""
+    of the fp32 kernel's.
+
+    ``hs_variant`` picks the kernel of calls with a caller-supplied ``hs``: ``"fp32"`` (default), ``"tc"`` (the one-layer
+    tensor-core kernels, which start every row from its (h_0, c_0)), or ``"auto"`` = ``"tc"`` when a probe with a random initial
+    state keeps the outputs within ``tc_tolerance`` of the fp32 kernel's (``hs_probe_error``, ``hs_choice``), else ``"fp32"``."""
 
     def __init__(self, input_size, hidden_layer_size, hidden_layer_count, output_size, dropout=0.2,
-                 philox_seed=None, precision="fp32", lstm_variant="auto", tc_tolerance=2e-4):
+                 philox_seed=None, precision="fp32", lstm_variant="auto", tc_tolerance=2e-4, hs_variant="fp32"):
         self.output_size = int(output_size)
         self.input_size = int(input_size)
         self.hidden_layer_size = int(hidden_layer_size)
@@ -218,8 +222,13 @@ class DropoutLSTM:
         if lstm_variant not in ("auto", "fp32", "tc"):
             raise UserWarning(f"lstm_variant must be 'auto', 'fp32' or 'tc', got {lstm_variant!r}")
         self.lstm_variant = lstm_variant
+        if hs_variant not in ("auto", "fp32", "tc"):
+            raise UserWarning(f"hs_variant must be 'auto', 'fp32' or 'tc', got {hs_variant!r}")
+        self.hs_variant = hs_variant
         self.tc_tolerance = float(tc_tolerance)
         self.tc_probe_error = None           # max |tc - fp32| over the probe batch, once measured
+        self.hs_probe_error = None           # the same for calls with hs (hs_variant="auto")
+        self.hs_choice = None                # the kernel hs_variant="auto" picked: "tc" or "fp32"
         self.lstm = _LstmMode()
         self.philox_seed = int(torch.initial_seed() if philox_seed is None else philox_seed) & (2 ** 64 - 1)
         self._calls = 0                      # Philox "frame" counter: fresh masks on every call
@@ -238,6 +247,7 @@ class DropoutLSTM:
         self._state = {k: torch.as_tensor(np.asarray(v.detach().cpu() if isinstance(v, torch.Tensor) else v,
                                                      dtype=np.float32)) for k, v in state.items()}
         self._blob = self._blob_tc = self._tc_ok = None
+        self.hs_choice = self.hs_probe_error = None
         return self
 
     def state_dict(self):
@@ -304,6 +314,31 @@ class DropoutLSTM:
             self._tc_ok = self.tc_probe_error <= self.tc_tolerance
         return self._tc_ok
 
+    def _use_tc_hs(self, T):
+        """Which kernel a call with ``hs`` takes (see the class docstring)."""
+        if self.hs_variant == "fp32":
+            return False
+        if not self._tc_supported(T):
+            if self.hs_variant == "tc":
+                raise UserWarning(f"the tensor-core LSTM kernels do not take (I,H,L,O)={self._dims()} with T={T}")
+            return False
+        if self.hs_variant == "tc":
+            return True
+        if self.hs_choice is None:               # probe: N(0,1) windows, N(0, 0.5^2) states, the same Philox masks through both kernels
+            I, H, L, _ = self._dims()
+            g = torch.Generator(device="cpu").manual_seed(1234)
+            x = torch.randn((128, T, I), generator=g, dtype=torch.float32).cuda()
+            hs = [(0.5 * torch.randn((L, 128, H), generator=g, dtype=torch.float32)).cuda() for _ in range(2)]
+            calls = self._calls
+            outs = []
+            for tc in (False, True):
+                self._calls = 0x5EED
+                outs.append(self._launch(x, 1, N.MASK_PHILOX, None, hs, tc))
+            self._calls = calls
+            self.hs_probe_error = float((outs[0] - outs[1]).abs().max().item())
+            self.hs_choice = "tc" if self.hs_probe_error <= self.tc_tolerance else "fp32"
+        return self.hs_choice == "tc"
+
     def _launch(self, xd, n_kernel, mask_mode, md, hs, tc):
         """One call of the C ABI: ``xd [E, T, I]`` on the device -> ``[E, n_kernel, T, O]``."""
         I, H, L, O = self._dims()
@@ -366,7 +401,7 @@ class DropoutLSTM:
                 xd = xd.repeat_interleave(n_samples, dim=0)
                 if md is not None:                       # [E][L-1][T][n][H] -> [E * n][L-1][T][1][H]
                     md = md.view(E, L - 1, T, n_samples, H).permute(0, 3, 1, 2, 4).contiguous()
-            out = self._launch(xd, 1, mask_mode, md, state, False).reshape(rows, T, O)
+            out = self._launch(xd, 1, mask_mode, md, state, self._use_tc_hs(T)).reshape(rows, T, O)
             self._calls += 1
             return out.cpu() if host_in else out
         preds = self._launch(xd, n_kernel, mask_mode, md, None, self._use_tc(T))

@@ -141,15 +141,17 @@ typedef struct ape_lstm_args {
     int ws_E;
     /* tensor-core path, H = 128, L >= 3: how consecutive layers >= 1 are launched.  0 = automatic (a pair of layers runs as ONE
        two-layer wavefront launch, csrc/ape_lstm_tcw.cu, when the batch fills the GPU), 1 = one launch per layer always,
-       2 = wavefront pairs always, 3 = the SPLIT-PRECISION variant (every operand an fp16 pair hi + lo, three tensor-core passes per
+       2 = wavefront pairs always (no initial state), 3 = the SPLIT-PRECISION variant, no initial state yet (every operand an fp16 pair hi + lo, three tensor-core passes per
        product, ex2 / rcp cell update: fp32-grade results at ~0.4 of the single-pass throughput; needs weights_tcx; H = 128:
        csrc/ape_lstm_tcx.cu, H = 256: csrc/ape_lstm_tcxs.cu),
        4 = the SMALL-BATCH kernel (csrc/ape_lstm_tcl.cu: B * nF * n_samples <= 8192 rows, L <= 4: all layers in one launch, one
        8-CTA cluster per 128 rows with the hidden units split across it - the real-time case of one to a few dozen streams; same
-       arithmetic as 0..2) */
+       arithmetic as 0..2; no initial state) */
     int tc_flags;
-    /* fp32 path: optional initial state (h_0, c_0) of torch.nn.LSTM(x, hs) (nn_models.py:180-189): [L][E][H] float32 each, both
-       or neither; needs n_samples == 1 (a caller with per-sample states passes the samples as estimates) */
+    /* optional initial state (h_0, c_0) of torch.nn.LSTM(x, hs) (nn_models.py:180-189): [L][E][H] float32 each, both or neither
+       (APE_ERR_BAD_ARG); needs n_samples == 1 (APE_ERR_UNSUPPORTED; a caller with per-sample states passes the samples as estimates).
+       Taken by the fp32 path and by the tensor-core path with tc_flags 0 or 1 (the one-layer kernels; tc_flags 0 then never pairs
+       layers; both pointers 16-byte aligned, else APE_ERR_BAD_ARG); tc_flags 2, 3 and 4 refuse it with APE_ERR_UNSUPPORTED */
     const float* h0;
     const float* c0;
     /* ---- ABI 6 ---- */
@@ -170,7 +172,7 @@ int ape_mc_lstm_fma(const ape_lstm_args* args, void* stream);
  * Tensor-core variant (tcgen05, cta_group::2, TMEM accumulators): fp16 operands, fp32 accumulation and cell state.
  * H in {64, 128} (gate weights resident in shared memory; H = 128, L >= 3: pairs of layers >= 1 as one two-layer wavefront launch
  * with weights streamed from L2) or 256 (gate weights streamed from L2 through a cp.async.bulk ring), L >= 2; same arguments and
- * outputs as ape_mc_lstm_fma plus weights_tc (h0 / c0 are not taken: a caller-supplied initial state runs on the fp32 path).
+ * outputs as ape_mc_lstm_fma plus weights_tc, h0 / c0 included (tc_flags 0 and 1 only; see the h0 field).
  * Use when the streams x MC-samples batch is large (>= a few thousand rows); the fp32 variant is the exact path.
  */
 int ape_mc_lstm_tc_supported(int I, int H, int L, int O);
