@@ -24,7 +24,8 @@ KSLICE = 16                      # csrc/ape_lstm_pack.h: APE_KSLICE
 SYMBOLS = (
     "ape_abi_version", "ape_last_cuda_error", "ape_device_info", "ape_lstm_blob_floats", "ape_features", "ape_features_push",
     "ape_mc_lstm_workspace_bytes", "ape_mc_lstm_fma", "ape_mc_lstm_tc_supported", "ape_lstm_tc_blob_bytes",
-    "ape_mc_lstm_tc_workspace_bytes", "ape_mc_lstm_tc_workspace_bytes_all_steps", "ape_mc_lstm_tc", "ape_mc_lstm_tc_launch_count", "ape_mc_lstm_tcx_supported", "ape_lstm_tcx_blob_bytes", "ape_mc_lstm_tcx_workspace_bytes", "ape_mc_lstm_tcxs_supported", "ape_lstm_tcxs_blob_bytes", "ape_mc_lstm_tcxs_workspace_bytes", "ape_philox_masks", "ape_ff_blob_floats", "ape_mc_ff", "ape_dense_act", "ape_fk_reduce", "ape_msg_from_est",
+    "ape_mc_lstm_tc_workspace_bytes", "ape_mc_lstm_tc_workspace_bytes_all_steps", "ape_mc_lstm_tc", "ape_mc_lstm_tc_launch_count", "ape_mc_lstm_tcx_supported", "ape_lstm_tcx_blob_bytes", "ape_mc_lstm_tcx_workspace_bytes", "ape_mc_lstm_tcx_workspace_bytes_all_steps", "ape_mc_lstm_tcxs_supported", "ape_lstm_tcxs_blob_bytes", "ape_mc_lstm_tcxs_workspace_bytes",
+    "ape_mc_lstm_tcxs_workspace_bytes_all_steps", "ape_philox_masks", "ape_ff_blob_floats", "ape_mc_ff", "ape_dense_act", "ape_fk_reduce", "ape_msg_from_est",
     "ape_pipeline_create", "ape_pipeline_destroy", "ape_pipeline_submit", "ape_pipeline_wait", "ape_pipeline_query", "ape_pipeline_sync",
     "ape_pipeline_fence",
     "ape_selfcheck_philox", "ape_selfcheck_keep8", "ape_selfcheck_features", "ape_selfcheck_row_pose", "ape_selfcheck_tcs_schedule",
@@ -146,12 +147,16 @@ def load():
     lib.ape_lstm_tcx_blob_bytes.argtypes = [i32, i32, i32, C.POINTER(C.c_int64)]
     lib.ape_mc_lstm_tcx_workspace_bytes.restype = i32
     lib.ape_mc_lstm_tcx_workspace_bytes.argtypes = [i32, i32, i32, i32, i32, i32, i32, C.POINTER(u64)]
+    lib.ape_mc_lstm_tcx_workspace_bytes_all_steps.restype = i32
+    lib.ape_mc_lstm_tcx_workspace_bytes_all_steps.argtypes = [i32, i32, i32, i32, i32, i32, i32, C.POINTER(u64)]
     lib.ape_mc_lstm_tcxs_supported.restype = i32
     lib.ape_mc_lstm_tcxs_supported.argtypes = [i32, i32, i32, i32]
     lib.ape_lstm_tcxs_blob_bytes.restype = i32
     lib.ape_lstm_tcxs_blob_bytes.argtypes = [i32, i32, i32, C.POINTER(C.c_int64)]
     lib.ape_mc_lstm_tcxs_workspace_bytes.restype = i32
     lib.ape_mc_lstm_tcxs_workspace_bytes.argtypes = [i32, i32, i32, i32, i32, i32, i32, C.POINTER(u64)]
+    lib.ape_mc_lstm_tcxs_workspace_bytes_all_steps.restype = i32
+    lib.ape_mc_lstm_tcxs_workspace_bytes_all_steps.argtypes = [i32, i32, i32, i32, i32, i32, i32, C.POINTER(u64)]
     lib.ape_philox_masks.restype = i32
     lib.ape_philox_masks.argtypes = [u64, u32, i32, i32, i32, i32, i32, i32, i32, f32, vp, vp]
     lib.ape_ff_blob_floats.restype = i32
@@ -254,9 +259,10 @@ def tcx_blob_bytes(I, H, L):
     return out.value
 
 
-def tcx_workspace_bytes(I, H, L, T, O, E, n):
+def tcx_workspace_bytes(I, H, L, T, O, E, n, all_steps=False):
     out = C.c_uint64(0)
-    check(load().ape_mc_lstm_tcx_workspace_bytes(I, H, L, T, O, E, n, C.byref(out)), "ape_mc_lstm_tcx_workspace_bytes")
+    name = "ape_mc_lstm_tcx_workspace_bytes" + ("_all_steps" if all_steps else "")
+    check(getattr(load(), name)(I, H, L, T, O, E, n, C.byref(out)), name)
     return out.value
 
 
@@ -270,9 +276,10 @@ def tcxs_blob_bytes(I, H, L):
     return out.value
 
 
-def tcxs_workspace_bytes(I, H, L, T, O, E, n):
+def tcxs_workspace_bytes(I, H, L, T, O, E, n, all_steps=False):
     out = C.c_uint64(0)
-    check(load().ape_mc_lstm_tcxs_workspace_bytes(I, H, L, T, O, E, n, C.byref(out)), "ape_mc_lstm_tcxs_workspace_bytes")
+    name = "ape_mc_lstm_tcxs_workspace_bytes" + ("_all_steps" if all_steps else "")
+    check(getattr(load(), name)(I, H, L, T, O, E, n, C.byref(out)), name)
     return out.value
 
 
@@ -285,8 +292,10 @@ def split_blob_bytes(I, H, L):
     return tcxs_blob_bytes(I, H, L) if H == 256 else tcx_blob_bytes(I, H, L)
 
 
-def split_workspace_bytes(I, H, L, T, O, E, n):
-    return tcxs_workspace_bytes(I, H, L, T, O, E, n) if H == 256 else tcx_workspace_bytes(I, H, L, T, O, E, n)
+def split_workspace_bytes(I, H, L, T, O, E, n, all_steps=False):
+    """Workspace of a split-precision call; ``all_steps``: a call with per-step outputs (the model API)."""
+    fn = tcxs_workspace_bytes if H == 256 else tcx_workspace_bytes
+    return fn(I, H, L, T, O, E, n, all_steps)
 
 
 def tc_blob_bytes(I, H, L):

@@ -541,26 +541,42 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1) lstm_lay
 // all_steps (the model API, DropoutLSTM.forward / monte_carlo_predictions): the output layer on EVERY step of the last layer's
 // sequence.  units: [pair tile][T][cta][H/8][128 rows] 16-byte units of fp16 h_t (unscaled); Wo: [O][H] then bias [O];
 // preds: [row][T][O] float32.  One thread per output value; rows x T x O x H multiply-adds, negligible next to the layers.
-__global__ void units_output_kernel(const uint4* __restrict__ units, const float* __restrict__ Wo, float* __restrict__ preds,
-                                    int rows, int T, int H, int O) {
+// units_lo (the split-precision kernels, else null): the lo halves of the same units; h = hi + lo is exact in fp32 (the pair
+// carries ~22 bits) and enters the same FMA chain.
+__global__ void units_output_kernel(const uint4* __restrict__ units, const uint4* __restrict__ units_lo, const float* __restrict__ Wo,
+                                    float* __restrict__ preds, int rows, int T, int H, int O) {
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= (long long)rows * T * O) return;
     const int o = (int)(idx % O), t = (int)((idx / O) % T), row = (int)(idx / ((long long)O * T));
     const int tile = row >> 8, cta = (row >> 7) & 1, r = row & 127, KG = H / 8;
-    const uint4* src = units + ((((size_t)tile * T + t) * 2 + cta) * KG) * ROWS + r;
+    const size_t at = ((((size_t)tile * T + t) * 2 + cta) * KG) * ROWS + r;
+    const uint4* src = units + at;
     const float* w = Wo + (size_t)o * H;
     float sum = __ldg(Wo + (size_t)O * H + o);
     for (int j = 0; j < KG; ++j) {
         const uint4 u = __ldg(src + (size_t)j * ROWS);
-        const uint32_t v[4] = {u.x, u.y, u.z, u.w};
+        const uint4 ul = units_lo ? __ldg(units_lo + at + (size_t)j * ROWS) : make_uint4(0, 0, 0, 0);
+        const uint32_t v[4] = {u.x, u.y, u.z, u.w}, vl[4] = {ul.x, ul.y, ul.z, ul.w};
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
-            const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&v[k]));
+            float2 f = __half22float2(*reinterpret_cast<const __half2*>(&v[k]));
+            if (units_lo) {
+                const float2 fl = __half22float2(*reinterpret_cast<const __half2*>(&vl[k]));
+                f.x += fl.x; f.y += fl.y;
+            }
             sum = fmaf(__ldg(w + 8 * j + 2 * k), f.x, sum);
             sum = fmaf(__ldg(w + 8 * j + 2 * k + 1), f.y, sum);
         }
     }
     preds[idx] = sum;
+}
+
+int launch_units_output(const uint4* units, const uint4* units_lo, const float* Wo, float* preds, long long rows, int T, int H, int O,
+                        cudaStream_t st) {
+    const long long total = rows * T * O;
+    const int threads = 256;
+    units_output_kernel<<<(unsigned)((total + threads - 1) / threads), threads, 0, st>>>(units, units_lo, Wo, preds, (int)rows, T, H, O);
+    return check_launch();
 }
 
 template <int H> static size_t smem_bytes(int kgx) {
@@ -677,8 +693,9 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
     using namespace ape;
     int rc = check_lstm_args(g);                               // (h0 / c0: both or neither, and n_samples == 1)
     if (rc != APE_OK) return rc;
-    // an initial state runs on the one-layer kernels (tc_flags 0 and 1); the wavefront, split-precision and small-batch kernels take none
-    if (g->h0 && (g->tc_flags == 2 || g->tc_flags == 3 || g->tc_flags == 4)) return APE_ERR_UNSUPPORTED;
+    // an initial state runs on the one-layer kernels (tc_flags 0 and 1) and on the H = 256 split-precision kernel; the wavefront,
+    // small-batch and H = 128 split-precision kernels take none
+    if (g->h0 && (g->tc_flags == 2 || (g->tc_flags == 3 && g->H != 256) || g->tc_flags == 4)) return APE_ERR_UNSUPPORTED;
     // the state kernels read h_0 / c_0 rows as float4 (H is a multiple of 32, so every layer's block keeps the base alignment)
     if (((uintptr_t)g->h0 | (uintptr_t)g->c0) & 15) return APE_ERR_BAD_ARG;
     if (g->tc_flags == 3)                                      // split-precision variant (csrc/ape_lstm_tcx.cu, H = 256: ape_lstm_tcxs.cu)
@@ -831,11 +848,8 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
         ++l;
     }
     if (all_steps) {                                            // output layer on every step (nn_models.py:189: output_layer(all))
-        const long long total = rows * g->T * g->O;
-        const int threads = 256;
-        tc::units_output_kernel<<<(unsigned)((total + threads - 1) / threads), threads, 0, st>>>(
-            units[(g->L - 2) & 1], g->weights + ape_pack_out_offset(g->I, g->H, g->L), g->preds, (int)rows, g->T, H, g->O);
-        rc = check_launch();
+        rc = tc::launch_units_output(units[(g->L - 2) & 1], nullptr, g->weights + ape_pack_out_offset(g->I, g->H, g->L), g->preds, rows,
+                                     g->T, H, g->O, st);
         if (rc != APE_OK) return rc;
     }
     if (prof) {

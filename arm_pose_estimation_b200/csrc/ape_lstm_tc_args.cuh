@@ -126,6 +126,11 @@ __device__ __forceinline__ void lstm_cell2(F2 pi, F2 pf, F2 pg, F2 po, F2& c, F2
     h = (one - ec) * pk(rcp_approx(lo(d2)), rcp_approx(hi(d2)));
 }
 
+// all_steps: the fp32 output layer on every step of the last layer's kept sequence (units [pair tile][T][cta][H/8][128 rows]);
+// units_lo: the split-precision kernels' lo halves of the same units, or null (ape_lstm_tc.cu)
+int launch_units_output(const uint4* units, const uint4* units_lo, const float* Wo, float* preds, long long rows, int T, int H, int O,
+                        cudaStream_t st);
+
 }  // namespace tc
 
 namespace tcs {
@@ -160,15 +165,15 @@ size_t scratch_bytes(int sm_count);              // per-CTA cell-state scratch o
 int launch_layer(const tc::TcLayerArgs& a, int sm_count, cudaStream_t st);
 int run(const ape_lstm_args* g, cudaStream_t st);    // all layers of a call (ape_mc_lstm_tc with tc_flags == 3)
 size_t blob_bytes(int I, int L);
-size_t workspace_bytes(int L, int T, long long E, int n_samples);
+size_t workspace_bytes(int L, int T, long long E, int n_samples, bool all_steps);
 }  // namespace tcx
 
 namespace tcxs {
 // split-precision kernel for H = 256 (ape_lstm_tcxs.cu): the arithmetic and blob layout of tcx, h_t staged through L2 into
 // single-buffered TMEM operands
 bool supported(int H, int I, int O);
-int run(const ape_lstm_args* g, cudaStream_t st);    // all layers of a call (ape_mc_lstm_tc with tc_flags == 3, H = 256)
+int run(const ape_lstm_args* g, cudaStream_t st);    // all layers of a call (ape_mc_lstm_tc with tc_flags == 3, H = 256; h0 / c0 taken)
 size_t blob_bytes(int I, int L);
-size_t workspace_bytes(int L, int T, long long E, int n_samples);
+size_t workspace_bytes(int L, int T, long long E, int n_samples, bool all_steps);
 }  // namespace tcxs
 }  // namespace ape

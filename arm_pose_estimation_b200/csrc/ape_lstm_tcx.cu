@@ -521,22 +521,25 @@ size_t blob_bytes(int I, int L) {
 }
 
 // workspace: [2 x scratch][layer 0 output: 2 copies x (hi, lo)][layers >= 1 outputs: up to 2 buffers x (hi, lo)]
+// (all_steps: the last layer's sequence is kept too, for the per-step output layer - one more (hi, lo) pair while L < 4)
 struct WsLayout { size_t scratch, u0, u1, total; int n_u1; };
-static WsLayout ws_layout(int L, int T, long long E, int n_samples) {
+static WsLayout ws_layout(int L, int T, long long E, int n_samples, bool all_steps) {
     WsLayout w{};
     w.scratch = scratch_bytes(MAX_SMS);
     const unsigned long long tiles0 = ((unsigned long long)E + 255) / 256, tiles1 = ((unsigned long long)E * n_samples + 255) / 256;
     w.u0 = (size_t)((tiles0 * 256 * T * H * 2 + 255) & ~(unsigned long long)255);
     w.u1 = (size_t)((tiles1 * 256 * T * H * 2 + 255) & ~(unsigned long long)255);
-    w.n_u1 = L - 2 > 2 ? 2 : (L - 2 < 0 ? 0 : L - 2);
+    const int n_u1 = L - 2 + (all_steps ? 1 : 0);
+    w.n_u1 = n_u1 > 2 ? 2 : (n_u1 < 0 ? 0 : n_u1);
     w.total = 2 * w.scratch + 4 * w.u0 + 2 * (size_t)w.n_u1 * w.u1 + 512;
     return w;
 }
-size_t workspace_bytes(int L, int T, long long E, int n_samples) { return ws_layout(L, T, E, n_samples).total; }
+size_t workspace_bytes(int L, int T, long long E, int n_samples, bool all_steps) { return ws_layout(L, T, E, n_samples, all_steps).total; }
 
 int run(const ape_lstm_args* g, cudaStream_t st) {
     if (!supported(g->H, g->I, g->O) || g->L < 2) return APE_ERR_UNSUPPORTED;
-    if (g->all_steps || g->h0 || g->c0) return APE_ERR_UNSUPPORTED;       // the model API's per-step outputs / initial state: fp32 path
+    if (g->h0 || g->c0) return APE_ERR_UNSUPPORTED;                       // an initial state: the fp32 path (or H = 256, ape_lstm_tcxs.cu)
+    if (g->all_steps && (g->layer_begin != 0 || g->layer_end != 0)) return APE_ERR_UNSUPPORTED;
     if (g->T > 40) return APE_ERR_UNSUPPORTED;
     if (!g->weights_tcx || !g->workspace) return APE_ERR_BAD_ARG;
     const long long E = (long long)g->B * g->nF;
@@ -550,7 +553,8 @@ int run(const ape_lstm_args* g, cudaStream_t st) {
     const int sm_big = sm_count - ((g->reserve_sms + 1) & ~1);
     const long long rows = E * g->n_samples;
     const int tiles0 = (int)((E + 255) / 256), tiles1 = (int)((rows + 255) / 256);
-    const WsLayout wl = ws_layout(g->L, g->T, g->ws_E > 0 ? g->ws_E : E, g->n_samples);
+    const bool all_steps = g->all_steps != 0;
+    const WsLayout wl = ws_layout(g->L, g->T, g->ws_E > 0 ? g->ws_E : E, g->n_samples, all_steps);
     char* wsp = (char*)(((uintptr_t)g->workspace + 255) & ~(uintptr_t)255);
     char* scratch = wsp;
     wsp += 2 * wl.scratch;
@@ -598,8 +602,9 @@ int run(const ape_lstm_args* g, cudaStream_t st) {
             a.rows = (int)rows; a.n = g->n_samples;
             a.n_pair_tiles = tiles1;
             a.mask_mode = g->mask_mode;
-            a.out_units = last ? nullptr : u1_hi((l - 1) & 1);
-            a.out_units_lo = last ? nullptr : u1_lo((l - 1) & 1);
+            // (all_steps: the last layer keeps its sequence for the per-step output layer)
+            a.out_units = (last && !all_steps) ? nullptr : u1_hi((l - 1) & 1);
+            a.out_units_lo = (last && !all_steps) ? nullptr : u1_lo((l - 1) & 1);
         }
         a.masks = g->masks; a.gap = l - 1; a.n_gaps = g->L - 1;
         a.seed = g->philox_seed; a.stream_id0 = g->stream_id0;
@@ -610,13 +615,18 @@ int run(const ape_lstm_args* g, cudaStream_t st) {
         a.bo = a.Wo + (size_t)g->O * g->H;
         a.O = g->O;
         a.Wo16 = wo16;
-        a.preds = last ? g->preds : nullptr;
+        a.preds = (last && !all_steps) ? g->preds : nullptr;
         a.pred_ring = g->pred_ring; a.n_out = g->n_samples;
         a.cstate = (float*)(scratch + (l == 0 ? 0 : wl.scratch));
         a.timeline = (g->trace && g->trace_layer < 0) ? (long long*)g->trace + (size_t)l * MAX_SMS * 4 : nullptr;
         const int rc = launch_layer(a, l == 0 ? sm_count : sm_big, st);
         if (rc != APE_OK) return rc;
         if (prof) APE_CUDA_TRY(cudaEventRecord(ev[l + 1], st));
+    }
+    if (all_steps) {                                           // output layer on every step, h = hi + lo against the fp32 W_o
+        const int rc = tc::launch_units_output(u1_hi((g->L - 2) & 1), u1_lo((g->L - 2) & 1), g->weights + ape_pack_out_offset(g->I, g->H, g->L),
+                                               g->preds, rows, g->T, H, g->O, st);
+        if (rc != APE_OK) return rc;
     }
     if (prof) {
         APE_CUDA_TRY(cudaStreamSynchronize(st));
@@ -640,6 +650,13 @@ extern "C" int ape_lstm_tcx_blob_bytes(int I, int H, int L, int64_t* bytes) {
 extern "C" int ape_mc_lstm_tcx_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
     if (!bytes || T < 1 || E < 0 || n_samples < 1) return APE_ERR_BAD_ARG;
     if (!ape_mc_lstm_tcx_supported(I, H, L, O)) return APE_ERR_UNSUPPORTED;
-    *bytes = ape::tcx::workspace_bytes(L, T, E, n_samples);
+    *bytes = ape::tcx::workspace_bytes(L, T, E, n_samples, false);
+    return APE_OK;
+}
+// the same for a call with all_steps != 0 (the model API: the last layer's sequence is kept for the per-step output layer)
+extern "C" int ape_mc_lstm_tcx_workspace_bytes_all_steps(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
+    if (!bytes || T < 1 || E < 0 || n_samples < 1) return APE_ERR_BAD_ARG;
+    if (!ape_mc_lstm_tcx_supported(I, H, L, O)) return APE_ERR_UNSUPPORTED;
+    *bytes = ape::tcx::workspace_bytes(L, T, E, n_samples, true);
     return APE_OK;
 }

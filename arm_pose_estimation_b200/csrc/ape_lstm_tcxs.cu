@@ -58,7 +58,7 @@ constexpr float NEG2LOG2E = -2.0f * 1.4426950408889634f;   // accumulator -> ex2
 
 enum {
     BAR_X_READY = 0, BAR_X_DONE = 1, BAR_ACC_READY = 2, BAR_SLOT_FREE = 4, BAR_H_READY = 6, BAR_OUT_READY = 7, BAR_W_FULL = 8,
-    BAR_W_EMPTY = BAR_W_FULL + NFULL, BAR_COUNT = BAR_W_EMPTY + NP
+    BAR_W_EMPTY = BAR_W_FULL + NFULL, BAR_H0_READY = BAR_W_EMPTY + NP, BAR_COUNT = BAR_H0_READY + 1
 };
 static_assert(BAR_COUNT * 8 + 16 <= BAR_BLOCK_BYTES, "barrier block too small");
 
@@ -67,9 +67,12 @@ __host__ __device__ constexpr uint32_t p0_bytes(int kgx) { return (uint32_t)(kgx
 __host__ __device__ constexpr uint32_t p1_bytes(int kgx) { return (uint32_t)kgx * KG_BYTES_B; }
 constexpr uint32_t PH_BYTES = KG * KG_BYTES_B;
 __host__ __device__ constexpr uint32_t chunk_bytes(int kgx) { return p0_bytes(kgx) + p1_bytes(kgx) + 2 * PH_BYTES; }
-// ring pieces per chunk: x-part pieces (Wx_hi, then the same count of Wx_lo) and, for t > 0, 2 Wh_hi + 2 Wh_lo
+// ring pieces per chunk: x-part pieces (Wx_hi, then the same count of Wx_lo) and, for a step with a recurrent half, 2 Wh_hi + 2 Wh_lo
 __host__ __device__ constexpr int x_pieces(int kgx) { return (kgx + PIECE_KG - 1) / PIECE_KG; }
 constexpr int H_PIECES = KG / PIECE_KG;
+// Ring pieces of one chunk of step t.  A step has a recurrent half when t > 0 or, with a caller-supplied initial state, at t = 0
+// too (on h_0).  The producer, both issuers and the peer's forwarder walk the ring by this one count.
+__host__ __device__ constexpr int chunk_pieces(int kgx, int t, bool state) { return 2 * x_pieces(kgx) + (t > 0 || state ? 2 * H_PIECES : 0); }
 
 // v -> fp16 pair: hi = fp16(v), lo = fp16(v - hi), for two values at once (packed as half2 words)
 __device__ __forceinline__ void split2(float a, float b, uint32_t& hi, uint32_t& lo) {
@@ -80,6 +83,13 @@ __device__ __forceinline__ void split2(float a, float b, uint32_t& hi, uint32_t&
     lo = *reinterpret_cast<const uint32_t*>(&l);
 }
 
+// STATE: a caller-supplied initial state (a.h0, a.c0).  At the start of every tile the epilogue writes h_0 as fp16 pairs into the h
+// buffers step 0 reads and publishes it on BAR_H0_READY; the cell starts from c_0; step 0 runs its recurrent half after the
+// x-part, whose MMAs keep the stateless order and accumulate flags - so h_0 = c_0 = 0 reproduces the stateless kernel bit for bit.
+// h_0 has a barrier of its own (one phase per tile): BAR_H_READY keeps one phase per item, the parity the issuers derive from the
+// item index.  Sharing it, the epilogue could complete the h_T and h_0 phases before issuer 0 (which never waits for h_T) had
+// consumed h_T, and a parity wait can only name the current or the previous phase.
+template <bool STATE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
 lstm_layer_tcxs_kernel(const __grid_constant__ TcLayerArgs a) {
     using namespace umma;
@@ -117,6 +127,7 @@ lstm_layer_tcxs_kernel(const __grid_constant__ TcLayerArgs a) {
         }
         mbar_init(&bars[BAR_H_READY], 2 * EPI_WARPS);
         mbar_init(&bars[BAR_OUT_READY], 1);
+        if (STATE) mbar_init(&bars[BAR_H0_READY], 2 * EPI_WARPS);
         for (int p = 0; p < NFULL; ++p) mbar_init(&bars[BAR_W_FULL + p], rank == 0 ? 2 : 1);   // leader: own copy + the peer's forward
         for (int p = 0; p < NP; ++p) mbar_init(&bars[BAR_W_EMPTY + p], 1);
         mbar_init_fence();
@@ -160,10 +171,36 @@ lstm_layer_tcxs_kernel(const __grid_constant__ TcLayerArgs a) {
         const int NIe = ((npt - cluster_id + n_clusters - 1) / n_clusters) * T;
         uint32_t ph_out = 0;
         int t = -1, tile = cluster_id - n_clusters;
+        const float4* c0r = nullptr;                           // STATE: this row's c_0 (valid rows only)
 
         for (int w = 0; w < NIe; ++w) {
             if (++t == T) t = 0;
             if (t == 0) tile += n_clusters;
+            if constexpr (STATE) {
+                if (t == 0) {
+                    // h_0 as fp16 pairs into h_hi / h_lo (this thread: its row, units 32 cl + 8 s + [0, 8) of every chunk).  Nothing
+                    // reads them any more: this warp has drained every accumulator of the previous tile's last step and, on the last
+                    // layer, waited for its output product (BAR_OUT_READY).
+                    const int row = (tile * 2 + (int)rank) * ROWS + row_l;
+                    const bool valid = row < a.rows;
+                    const float4* h0r = reinterpret_cast<const float4*>(a.h0 + (size_t)(valid ? row : 0) * H) + 2 * s;
+                    c0r = valid ? reinterpret_cast<const float4*>(a.c0 + (size_t)row * H) + 2 * s : nullptr;
+                    const float4 z = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+#pragma unroll
+                    for (int cl = 0; cl < NCH; ++cl) {
+                        const float4 h_a = valid ? __ldg(h0r + 8 * cl) : z, h_b = valid ? __ldg(h0r + 8 * cl + 1) : z;
+                        uint32_t hi[4], lo[4];
+                        split2(h_a.x, h_a.y, hi[0], lo[0]); split2(h_a.z, h_a.w, hi[1], lo[1]);
+                        split2(h_b.x, h_b.y, hi[2], lo[2]); split2(h_b.z, h_b.w, hi[3], lo[3]);
+                        tmem_st_x4(hst0 + HH_COL + (uint32_t)(16 * cl), hi[0], hi[1], hi[2], hi[3]);
+                        tmem_st_x4(hst0 + HL_COL + (uint32_t)(16 * cl), lo[0], lo[1], lo[2], lo[3]);
+                    }
+                    tmem_st_wait();
+                    fence_before_sync();
+                    __syncwarp();
+                    if (lane == 0) arrive_leader(BAR_H0_READY);
+                }
+            }
             const bool final_out = has_out && t == T - 1;
             const bool keep_h = t + 1 < T || final_out;
             uint32_t r[16];
@@ -172,6 +209,7 @@ lstm_layer_tcxs_kernel(const __grid_constant__ TcLayerArgs a) {
             uint32_t hlast[4], llast[4];
             cbuf[0] = cbuf[1] = make_float4(0.0f, 0.0f, 0.0f, 0.0f);
             if (t > 0) cbuf[0] = __ldcg(cst_at(0));
+            else if (STATE && c0r) cbuf[0] = __ldg(c0r);         // c_0 of units 8 s + [0, 4) of chunk 0
             wait_bar(BAR_ACC_READY + 0, 0);                     // slot k serves chunks k, k+2, ...: parity = (chunk >> 1) & 1
             fence_after_sync();
             tmem_ld_x16(acc0, r);
@@ -191,7 +229,10 @@ lstm_layer_tcxs_kernel(const __grid_constant__ TcLayerArgs a) {
                     if (lane == 0) arrive_leader(BAR_SLOT_FREE + slot);
                 }
                 const float cp[4] = {cbuf[hp & 1].x, cbuf[hp & 1].y, cbuf[hp & 1].z, cbuf[hp & 1].w};
-                if (hp + 1 < 2 * NCH) cbuf[(hp + 1) & 1] = t > 0 ? __ldcg(cst_at(hp + 1)) : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+                if (hp + 1 < 2 * NCH)                          // (c_0: units 32 cl + 8 s + 4 half + [0, 4))
+                    cbuf[(hp + 1) & 1] = t > 0 ? __ldcg(cst_at(hp + 1))
+                                               : (STATE && c0r) ? __ldg(c0r + 8 * ((hp + 1) >> 1) + ((hp + 1) & 1))
+                                                                : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
                 if (half == 0) tmem_ld_x16(acc0 + (uint32_t)(slot * 128 + 16), r);
                 float hv[4], cn[4];
 #pragma unroll
@@ -376,8 +417,8 @@ lstm_layer_tcxs_kernel(const __grid_constant__ TcLayerArgs a) {
     } else {
       TCXS_REG_DEC(REGS_MMA);
       // The ring's piece sequence, walked identically by the producer, both issuers and the forwarder: per item (tile, t) and chunk
-      // nxp Wx_hi pieces (the last with the bias K step), nxp Wx_lo pieces, then (t > 0) H_PIECES Wh_hi and H_PIECES Wh_lo pieces;
-      // after the last step of the last layer's tile, one W_o piece.
+      // nxp Wx_hi pieces (the last with the bias K step), nxp Wx_lo pieces, then (t > 0, or STATE) H_PIECES Wh_hi and H_PIECES Wh_lo
+      // pieces (chunk_pieces); after the last step of the last layer's tile, one W_o piece.
       if (warp >= MMA_WARP && warp < MMA_WARP + N_ISSUERS) {
         if (rank == 0) {
             // =============================== MMA issuers (leader CTA): issuer k owns accumulator slot k ========================
@@ -388,7 +429,7 @@ lstm_layer_tcxs_kernel(const __grid_constant__ TcLayerArgs a) {
             const uint32_t bar_full = smem_u32(&bars[BAR_W_FULL]), bar_empty = smem_u32(&bars[BAR_W_EMPTY]);
             const uint32_t d_tmem = tmem + my_slot * 128u;
             const uint32_t hh = tmem + HH_COL, hl = tmem + HL_COL;
-            uint32_t wslot = 0, gpiece = 0, uses = 0;
+            uint32_t wslot = 0, gpiece = 0, uses = 0, h0_par = 1;   // h0_par: parity of this tile's BAR_H0_READY phase (STATE)
             auto ring_next = [&]() { wslot = wslot + 1 == NP ? 0 : wslot + 1; ++gpiece; };
             auto wait_full = [&]() {
                 uint32_t spins = 0;
@@ -400,7 +441,8 @@ lstm_layer_tcxs_kernel(const __grid_constant__ TcLayerArgs a) {
                 ++uses;
             };
             auto chunk = [&](int cl, bool mine, int t, int w) {
-                const int n_pieces = 2 * nxp + (t > 0 ? 2 * H_PIECES : 0);
+                const int n_pieces = chunk_pieces(kgx, t, STATE);
+                const bool recurrent = n_pieces > 2 * nxp;
                 if (!mine) { for (int p = 0; p < n_pieces; ++p) ring_next(); return; }
                 wait_slot();
                 for (int p = 0; p < nxp; ++p) {                // Wx_hi (+ bias rows): x_hi, ones, x_lo
@@ -427,15 +469,16 @@ lstm_layer_tcxs_kernel(const __grid_constant__ TcLayerArgs a) {
                             mma_f16<2>(d_tmem, dXh + (kg0 / 2 + m) * (2 * LBO_A >> 4), bd + m * (2 * LBO_B >> 4), idesc, 1u);
                         commit_pair_addr(bar_empty + wslot * 8, 0x3);
                         if (p == nxp - 1) {
-                            if (t == 0) commit_pair(&bars[BAR_ACC_READY + my_slot], 0x3);
+                            if (!recurrent) commit_pair(&bars[BAR_ACC_READY + my_slot], 0x3);
                             if (cl >= NCH - 2) commit_pair(&bars[BAR_X_DONE], 0x3);   // this issuer's last x-part of the item
                         }
                     }
                     __syncwarp();
                     ring_next();
                 }
-                if (t > 0) {
-                    mbar_wait_wd(&bars[BAR_H_READY], ((uint32_t)(w - 1)) & 1u);    // all of h_{t-1} is in TMEM
+                if (recurrent) {
+                    if (STATE && t == 0) mbar_wait_wd(&bars[BAR_H0_READY], h0_par);  // all of h_0 is in TMEM
+                    else mbar_wait_wd(&bars[BAR_H_READY], ((uint32_t)(w - 1)) & 1u);  // all of h_{t-1} is in TMEM
                     fence_after_sync();
                     for (int p = 0; p < 2 * H_PIECES; ++p) {   // Wh_hi: h_hi, h_lo; then Wh_lo: h_hi
                         const uint32_t c0 = (uint32_t)((p % H_PIECES) * PIECE_KG * 4);   // TMEM column of the piece's first k-group
@@ -478,6 +521,7 @@ lstm_layer_tcxs_kernel(const __grid_constant__ TcLayerArgs a) {
             int t = -1;
             for (int w = 0; w < NI; ++w) {
                 if (++t == T) t = 0;
+                if (STATE && t == 0) h0_par ^= 1;
                 mbar_wait_wd(&bars[BAR_X_READY], (uint32_t)w & 1u);
                 fence_after_sync();
                 for (int cl = 0; cl < NCH; ++cl) chunk(cl, (uint32_t)(cl & 1) == my_slot, t, w);
@@ -494,7 +538,7 @@ lstm_layer_tcxs_kernel(const __grid_constant__ TcLayerArgs a) {
             int t = -1;
             for (int w = 0; w < NI; ++w) {
                 if (++t == T) t = 0;
-                const int n_pieces = NCH * (2 * nxp + (t > 0 ? 2 * H_PIECES : 0)) + (has_out && t == T - 1 ? 1 : 0);
+                const int n_pieces = NCH * chunk_pieces(kgx, t, STATE) + (has_out && t == T - 1 ? 1 : 0);
                 for (int p = 0; p < n_pieces; ++p) forward();
             }
         }
@@ -525,7 +569,7 @@ lstm_layer_tcxs_kernel(const __grid_constant__ TcLayerArgs a) {
                     const int nkg = kgx - p * PIECE_KG < PIECE_KG ? kgx - p * PIECE_KG : PIECE_KG;
                     put(c0 + p0b + (size_t)p * PIECE_KG * KG_BYTES_B, (uint32_t)nkg * KG_BYTES_B);
                 }
-                if (t > 0)
+                if (chunk_pieces(kgx, t, STATE) > 2 * nxp)      // the recurrent half: Wh_hi, Wh_lo
                     for (int p = 0; p < 2 * H_PIECES; ++p) put(c0 + p0b + p1b + (size_t)p * PIECE_KG * KG_BYTES_B, PIECE_KG * KG_BYTES_B);
             }
             if (has_out && t == T - 1) put(a.Wo16 + (size_t)rank * OUT_BYTES, OUT_BYTES);
@@ -551,10 +595,12 @@ int launch_layer(const TcLayerArgs& a, int sm_count, cudaStream_t st) {
     if (unit_mode && (!a.in_lo || a.kgx != KG)) return APE_ERR_BAD_ARG;
     if (a.out_units && !a.out_units_lo) return APE_ERR_BAD_ARG;
     if (a.preds && (!a.Wo16 || a.O > (int)OUT_N / 2)) return APE_ERR_UNSUPPORTED;
-    APE_CUDA_TRY(cudaFuncSetAttribute(lstm_layer_tcxs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
+    if ((a.h0 != nullptr) != (a.c0 != nullptr)) return APE_ERR_BAD_ARG;
+    auto kernel = a.h0 ? lstm_layer_tcxs_kernel<true> : lstm_layer_tcxs_kernel<false>;
+    APE_CUDA_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
     int clusters = sm_count / 2;
     if (clusters > a.n_pair_tiles) clusters = a.n_pair_tiles;
-    lstm_layer_tcxs_kernel<<<2 * clusters, THREADS, SMEM, st>>>(a);
+    kernel<<<2 * clusters, THREADS, SMEM, st>>>(a);
     return check_launch();
 }
 
@@ -568,23 +614,26 @@ size_t blob_bytes(int I, int L) {
 }
 
 // workspace: [2 x scratch][layer 0 output: 2 copies x (hi, lo)][layers >= 1 outputs: up to 2 buffers x (hi, lo)]
+// (all_steps: the last layer's sequence is kept too, for the per-step output layer - one more (hi, lo) pair while L < 4)
 struct WsLayout { size_t scratch, u0, u1, total; int n_u1; };
-static WsLayout ws_layout(int L, int T, long long E, int n_samples) {
+static WsLayout ws_layout(int L, int T, long long E, int n_samples, bool all_steps) {
     WsLayout w{};
     w.scratch = scratch_bytes(MAX_SMS);
     const unsigned long long tiles0 = ((unsigned long long)E + 255) / 256, tiles1 = ((unsigned long long)E * n_samples + 255) / 256;
     w.u0 = (size_t)((tiles0 * 256 * T * H * 2 + 255) & ~(unsigned long long)255);
     w.u1 = (size_t)((tiles1 * 256 * T * H * 2 + 255) & ~(unsigned long long)255);
-    w.n_u1 = L - 2 > 2 ? 2 : (L - 2 < 0 ? 0 : L - 2);
+    const int n_u1 = L - 2 + (all_steps ? 1 : 0);
+    w.n_u1 = n_u1 > 2 ? 2 : (n_u1 < 0 ? 0 : n_u1);
     w.total = 2 * w.scratch + 4 * w.u0 + 2 * (size_t)w.n_u1 * w.u1 + 512;
     return w;
 }
-size_t workspace_bytes(int L, int T, long long E, int n_samples) { return ws_layout(L, T, E, n_samples).total; }
+size_t workspace_bytes(int L, int T, long long E, int n_samples, bool all_steps) { return ws_layout(L, T, E, n_samples, all_steps).total; }
 
 int run(const ape_lstm_args* g, cudaStream_t st) {
     if (!supported(g->H, g->I, g->O) || g->L < 2) return APE_ERR_UNSUPPORTED;
-    if (g->all_steps || g->h0 || g->c0) return APE_ERR_UNSUPPORTED;       // the model API's per-step outputs / initial state: fp32 path
-    if (g->T > 40) return APE_ERR_UNSUPPORTED;
+    // (h0 / c0: both or neither, n_samples == 1 and 16-byte alignment are checked by ape_mc_lstm_tc)
+    if (g->all_steps && (g->layer_begin != 0 || g->layer_end != 0)) return APE_ERR_UNSUPPORTED;
+    if (g->T > 40) return APE_ERR_UNSUPPORTED;                            // (with a state |c_t| <= |c_0| + t: the ex2 arguments are clamped)
     if (!g->weights_tcx || !g->workspace) return APE_ERR_BAD_ARG;
     const long long E = (long long)g->B * g->nF;
     if (E == 0) return APE_OK;
@@ -597,7 +646,8 @@ int run(const ape_lstm_args* g, cudaStream_t st) {
     const int sm_big = sm_count - ((g->reserve_sms + 1) & ~1);
     const long long rows = E * g->n_samples;
     const int tiles0 = (int)((E + 255) / 256), tiles1 = (int)((rows + 255) / 256);
-    const WsLayout wl = ws_layout(g->L, g->T, g->ws_E > 0 ? g->ws_E : E, g->n_samples);
+    const bool all_steps = g->all_steps != 0;
+    const WsLayout wl = ws_layout(g->L, g->T, g->ws_E > 0 ? g->ws_E : E, g->n_samples, all_steps);
     char* wsp = (char*)(((uintptr_t)g->workspace + 255) & ~(uintptr_t)255);
     char* scratch = wsp;
     wsp += 2 * wl.scratch;
@@ -645,8 +695,9 @@ int run(const ape_lstm_args* g, cudaStream_t st) {
             a.rows = (int)rows; a.n = g->n_samples;
             a.n_pair_tiles = tiles1;
             a.mask_mode = g->mask_mode;
-            a.out_units = last ? nullptr : u1_hi((l - 1) & 1);
-            a.out_units_lo = last ? nullptr : u1_lo((l - 1) & 1);
+            // (all_steps: the last layer keeps its sequence for the per-step output layer)
+            a.out_units = (last && !all_steps) ? nullptr : u1_hi((l - 1) & 1);
+            a.out_units_lo = (last && !all_steps) ? nullptr : u1_lo((l - 1) & 1);
         }
         a.masks = g->masks; a.gap = l - 1; a.n_gaps = g->L - 1;
         a.seed = g->philox_seed; a.stream_id0 = g->stream_id0;
@@ -657,13 +708,20 @@ int run(const ape_lstm_args* g, cudaStream_t st) {
         a.bo = a.Wo + (size_t)g->O * g->H;
         a.O = g->O;
         a.Wo16 = wo16;
-        a.preds = last ? g->preds : nullptr;
+        a.preds = (last && !all_steps) ? g->preds : nullptr;
         a.pred_ring = g->pred_ring; a.n_out = g->n_samples;
         a.cstate = (float*)(scratch + (l == 0 ? 0 : wl.scratch));
+        a.h0 = g->h0 ? g->h0 + (size_t)l * E * H : nullptr;   // [L][E][H]: with a state every layer has E rows (n_samples == 1)
+        a.c0 = g->c0 ? g->c0 + (size_t)l * E * H : nullptr;
         a.timeline = (g->trace && g->trace_layer < 0) ? (long long*)g->trace + (size_t)l * MAX_SMS * 4 : nullptr;
         const int rc = launch_layer(a, l == 0 ? sm_count : sm_big, st);
         if (rc != APE_OK) return rc;
         if (prof) APE_CUDA_TRY(cudaEventRecord(ev[l + 1], st));
+    }
+    if (all_steps) {                                           // output layer on every step, h = hi + lo against the fp32 W_o
+        const int rc = tc::launch_units_output(u1_hi((g->L - 2) & 1), u1_lo((g->L - 2) & 1), g->weights + ape_pack_out_offset(g->I, g->H, g->L),
+                                               g->preds, rows, g->T, H, g->O, st);
+        if (rc != APE_OK) return rc;
     }
     if (prof) {
         APE_CUDA_TRY(cudaStreamSynchronize(st));
@@ -687,6 +745,13 @@ extern "C" int ape_lstm_tcxs_blob_bytes(int I, int H, int L, int64_t* bytes) {
 extern "C" int ape_mc_lstm_tcxs_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
     if (!bytes || T < 1 || E < 0 || n_samples < 1) return APE_ERR_BAD_ARG;
     if (!ape_mc_lstm_tcxs_supported(I, H, L, O)) return APE_ERR_UNSUPPORTED;
-    *bytes = ape::tcxs::workspace_bytes(L, T, E, n_samples);
+    *bytes = ape::tcxs::workspace_bytes(L, T, E, n_samples, false);
+    return APE_OK;
+}
+// the same for a call with all_steps != 0 (the model API: the last layer's sequence is kept for the per-step output layer)
+extern "C" int ape_mc_lstm_tcxs_workspace_bytes_all_steps(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
+    if (!bytes || T < 1 || E < 0 || n_samples < 1) return APE_ERR_BAD_ARG;
+    if (!ape_mc_lstm_tcxs_supported(I, H, L, O)) return APE_ERR_UNSUPPORTED;
+    *bytes = ape::tcxs::workspace_bytes(L, T, E, n_samples, true);
     return APE_OK;
 }

@@ -205,11 +205,14 @@ class DropoutLSTM:
     ``lstm_variant``: ``"fp32"`` = the exact FFMA kernel, ``"tc"`` = the tcgen05 tensor-core kernels (fp16 operands, fp32
     accumulation and state), ``"auto"`` (default) = tensor cores when this model's shape is supported AND a probe on its own
     weights keeps the tensor-core outputs within ``tc_tolerance`` (normalised output units; 2e-4 is ~3e-5 m of hand position)
-    of the fp32 kernel's.
+    of the fp32 kernel's.  ``"tcx"`` = the split-precision tensor-core kernels (every operand an fp16 pair, fp32-grade results at
+    ~0.4 of the single-pass throughput; ``csrc/ape_lstm_tcx.cu`` for H = 128, ``csrc/ape_lstm_tcxs.cu`` for H = 256), for a model
+    whose weights make the single-pass probe fail; ``"auto"`` never picks it.
 
     ``hs_variant`` picks the kernel of calls with a caller-supplied ``hs``: ``"fp32"`` (default), ``"tc"`` (the one-layer
-    tensor-core kernels, which start every row from its (h_0, c_0)), or ``"auto"`` = ``"tc"`` when a probe with a random initial
-    state keeps the outputs within ``tc_tolerance`` of the fp32 kernel's (``hs_probe_error``, ``hs_choice``), else ``"fp32"``."""
+    tensor-core kernels, which start every row from its (h_0, c_0)), ``"tcx"`` (the split-precision kernel, H = 256 only), or
+    ``"auto"`` = ``"tc"`` when a probe with a random initial state keeps the outputs within ``tc_tolerance`` of the fp32 kernel's
+    (``hs_probe_error``, ``hs_choice``), else ``"fp32"``."""
 
     def __init__(self, input_size, hidden_layer_size, hidden_layer_count, output_size, dropout=0.2,
                  philox_seed=None, precision="fp32", lstm_variant="auto", tc_tolerance=2e-4, hs_variant="fp32"):
@@ -219,11 +222,11 @@ class DropoutLSTM:
         self.hidden_layer_count = int(hidden_layer_count)
         self.dropout = float(dropout)
         self.precision = precision
-        if lstm_variant not in ("auto", "fp32", "tc"):
-            raise UserWarning(f"lstm_variant must be 'auto', 'fp32' or 'tc', got {lstm_variant!r}")
+        if lstm_variant not in ("auto", "fp32", "tc", "tcx"):
+            raise UserWarning(f"lstm_variant must be 'auto', 'fp32', 'tc' or 'tcx', got {lstm_variant!r}")
         self.lstm_variant = lstm_variant
-        if hs_variant not in ("auto", "fp32", "tc"):
-            raise UserWarning(f"hs_variant must be 'auto', 'fp32' or 'tc', got {hs_variant!r}")
+        if hs_variant not in ("auto", "fp32", "tc", "tcx"):
+            raise UserWarning(f"hs_variant must be 'auto', 'fp32', 'tc' or 'tcx', got {hs_variant!r}")
         self.hs_variant = hs_variant
         self.tc_tolerance = float(tc_tolerance)
         self.tc_probe_error = None           # max |tc - fp32| over the probe batch, once measured
@@ -235,6 +238,7 @@ class DropoutLSTM:
         self._state = None
         self._blob = None                    # device copy of the packed weights (built lazily)
         self._blob_tc = None
+        self._blob_tcx = None
         self._ws = None
         self._tc_ok = None                   # outcome of the probe (None: not run yet)
 
@@ -246,7 +250,7 @@ class DropoutLSTM:
                                f"{(self.input_size, self.hidden_layer_size, self.hidden_layer_count, self.output_size)}")
         self._state = {k: torch.as_tensor(np.asarray(v.detach().cpu() if isinstance(v, torch.Tensor) else v,
                                                      dtype=np.float32)) for k, v in state.items()}
-        self._blob = self._blob_tc = self._tc_ok = None
+        self._blob = self._blob_tc = self._blob_tcx = self._tc_ok = None
         self.hs_choice = self.hs_probe_error = None
         return self
 
@@ -277,12 +281,22 @@ class DropoutLSTM:
             self._blob_tc = torch.from_numpy(pack_lstm_weights_tc(self._state)).cuda()
         return self._blob_tc
 
+    def packed_weights_tcx(self):
+        """Device tensor holding the blob of the split-precision tensor-core kernels."""
+        self.packed_weights()
+        if self._blob_tcx is None:
+            self._blob_tcx = torch.from_numpy(pack_lstm_weights_tcx(self._state)).cuda()
+        return self._blob_tcx
+
     def _dims(self):
         return self.input_size, self.hidden_layer_size, self.hidden_layer_count, self.output_size
 
-    def _workspace(self, T, E, n, tc):
+    def _workspace(self, T, E, n, kernel):
         I, H, L, O = self._dims()
-        need = N.workspace_bytes(I, H, L, T, O, E, n, tensor_core=tc, all_steps=tc)
+        if kernel == "tcx":
+            need = N.split_workspace_bytes(I, H, L, T, O, E, n, all_steps=True)
+        else:
+            need = N.workspace_bytes(I, H, L, T, O, E, n, tensor_core=kernel == "tc", all_steps=kernel == "tc")
         if self._ws is None or self._ws.numel() < need:
             self._ws = torch.empty(need, dtype=torch.uint8, device="cuda")
         return self._ws
@@ -291,39 +305,52 @@ class DropoutLSTM:
         I, H, L, O = self._dims()
         return N.tc_supported(I, H, L, O) and T <= 40
 
-    def _use_tc(self, T):
-        """Which kernel a call without ``hs`` takes (see the class docstring)."""
+    def _split_kernel(self, T, hs):
+        """``"tcx"`` when the split-precision kernels take this call, else ``UserWarning``."""
+        I, H, L, O = self._dims()
+        if not (N.split_supported(I, H, L, O) and T <= 40):
+            raise UserWarning(f"the split-precision tensor-core LSTM kernels do not take (I,H,L,O)={self._dims()} with T={T}")
+        if hs and H != 256:
+            raise UserWarning(f"the split-precision tensor-core LSTM kernels take an initial state at H = 256 only, not H = {H}")
+        return "tcx"
+
+    def _kernel(self, T):
+        """Which kernel a call without ``hs`` takes (see the class docstring): ``"fp32"``, ``"tc"`` or ``"tcx"``."""
         if self.lstm_variant == "fp32":
-            return False
+            return "fp32"
+        if self.lstm_variant == "tcx":
+            return self._split_kernel(T, False)
         if not self._tc_supported(T):
             if self.lstm_variant == "tc":
                 raise UserWarning(f"the tensor-core LSTM kernels do not take (I,H,L,O)={self._dims()} with T={T}")
-            return False
+            return "fp32"
         if self.lstm_variant == "tc":
-            return True
+            return "tc"
         if self._tc_ok is None:                  # probe: N(0,1) windows, dropout active, the same Philox masks through both kernels
             g = torch.Generator(device="cpu").manual_seed(1234)
             x = torch.randn((8, T, self.input_size), generator=g, dtype=torch.float32).cuda()
             calls = self._calls
             outs = []
-            for tc in (False, True):
+            for kernel in ("fp32", "tc"):
                 self._calls = 0x5EED
-                outs.append(self._launch(x, 16, N.MASK_PHILOX, None, None, tc))
+                outs.append(self._launch(x, 16, N.MASK_PHILOX, None, None, kernel))
             self._calls = calls
             self.tc_probe_error = float((outs[0] - outs[1]).abs().max().item())
             self._tc_ok = self.tc_probe_error <= self.tc_tolerance
-        return self._tc_ok
+        return "tc" if self._tc_ok else "fp32"
 
-    def _use_tc_hs(self, T):
-        """Which kernel a call with ``hs`` takes (see the class docstring)."""
+    def _kernel_hs(self, T):
+        """Which kernel a call with ``hs`` takes (see the class docstring): ``"fp32"``, ``"tc"`` or ``"tcx"``."""
         if self.hs_variant == "fp32":
-            return False
+            return "fp32"
+        if self.hs_variant == "tcx":
+            return self._split_kernel(T, True)
         if not self._tc_supported(T):
             if self.hs_variant == "tc":
                 raise UserWarning(f"the tensor-core LSTM kernels do not take (I,H,L,O)={self._dims()} with T={T}")
-            return False
+            return "fp32"
         if self.hs_variant == "tc":
-            return True
+            return "tc"
         if self.hs_choice is None:               # probe: N(0,1) windows, N(0, 0.5^2) states, the same Philox masks through both kernels
             I, H, L, _ = self._dims()
             g = torch.Generator(device="cpu").manual_seed(1234)
@@ -331,22 +358,24 @@ class DropoutLSTM:
             hs = [(0.5 * torch.randn((L, 128, H), generator=g, dtype=torch.float32)).cuda() for _ in range(2)]
             calls = self._calls
             outs = []
-            for tc in (False, True):
+            for kernel in ("fp32", "tc"):
                 self._calls = 0x5EED
-                outs.append(self._launch(x, 1, N.MASK_PHILOX, None, hs, tc))
+                outs.append(self._launch(x, 1, N.MASK_PHILOX, None, hs, kernel))
             self._calls = calls
             self.hs_probe_error = float((outs[0] - outs[1]).abs().max().item())
             self.hs_choice = "tc" if self.hs_probe_error <= self.tc_tolerance else "fp32"
-        return self.hs_choice == "tc"
+        return self.hs_choice
 
-    def _launch(self, xd, n_kernel, mask_mode, md, hs, tc):
-        """One call of the C ABI: ``xd [E, T, I]`` on the device -> ``[E, n_kernel, T, O]``."""
+    def _launch(self, xd, n_kernel, mask_mode, md, hs, kernel):
+        """One call of the C ABI on ``kernel`` ("fp32", "tc" or "tcx"): ``xd [E, T, I]`` on the device -> ``[E, n_kernel, T, O]``."""
         I, H, L, O = self._dims()
         E, T, _ = xd.shape
         preds = torch.empty((E, n_kernel, T, O), dtype=torch.float32, device="cuda")
         a = N.LstmArgs()
         a.weights = self.packed_weights().data_ptr()
-        a.weights_tc = self.packed_weights_tc().data_ptr() if tc else None
+        a.weights_tc = self.packed_weights_tc().data_ptr() if kernel == "tc" else None
+        if kernel == "tcx":                                  # split precision: its own blob, tc_flags = 3
+            a.weights_tcx, a.tc_flags = self.packed_weights_tcx().data_ptr(), 3
         a.I, a.H, a.L, a.T, a.O = I, H, L, T, O
         a.dropout_p = self.dropout
         a.x_dense, a.feat_ring_buf, a.feat_ring = xd.data_ptr(), None, 0
@@ -358,9 +387,9 @@ class DropoutLSTM:
         if hs is not None:
             a.h0, a.c0 = hs[0].data_ptr(), hs[1].data_ptr()
         a.philox_seed, a.stream_id0 = self.philox_seed, 0
-        a.workspace = self._workspace(T, E, n_kernel, tc).data_ptr()
+        a.workspace = self._workspace(T, E, n_kernel, kernel).data_ptr()
         a.preds, a.pred_ring, a.all_steps = preds.data_ptr(), 1, 1
-        fn, what = (N.load().ape_mc_lstm_tc, "ape_mc_lstm_tc") if tc else (N.load().ape_mc_lstm_fma, "ape_mc_lstm_fma")
+        fn, what = (N.load().ape_mc_lstm_fma, "ape_mc_lstm_fma") if kernel == "fp32" else (N.load().ape_mc_lstm_tc, "ape_mc_lstm_tc")
         N.check(fn(a, N.current_stream_ptr()), what)
         return preds
 
@@ -401,10 +430,10 @@ class DropoutLSTM:
                 xd = xd.repeat_interleave(n_samples, dim=0)
                 if md is not None:                       # [E][L-1][T][n][H] -> [E * n][L-1][T][1][H]
                     md = md.view(E, L - 1, T, n_samples, H).permute(0, 3, 1, 2, 4).contiguous()
-            out = self._launch(xd, 1, mask_mode, md, state, self._use_tc_hs(T)).reshape(rows, T, O)
+            out = self._launch(xd, 1, mask_mode, md, state, self._kernel_hs(T)).reshape(rows, T, O)
             self._calls += 1
             return out.cpu() if host_in else out
-        preds = self._launch(xd, n_kernel, mask_mode, md, None, self._use_tc(T))
+        preds = self._launch(xd, n_kernel, mask_mode, md, None, self._kernel(T))
         self._calls += 1
         out = preds.reshape(E * n_kernel, T, O)
         if n_kernel != n_samples:

@@ -141,9 +141,9 @@ typedef struct ape_lstm_args {
     int ws_E;
     /* tensor-core path, H = 128, L >= 3: how consecutive layers >= 1 are launched.  0 = automatic (a pair of layers runs as ONE
        two-layer wavefront launch, csrc/ape_lstm_tcw.cu, when the batch fills the GPU), 1 = one launch per layer always,
-       2 = wavefront pairs always (no initial state), 3 = the SPLIT-PRECISION variant, no initial state yet (every operand an fp16 pair hi + lo, three tensor-core passes per
+       2 = wavefront pairs always (no initial state), 3 = the SPLIT-PRECISION variant, initial state at H = 256 only (every operand an fp16 pair hi + lo, three tensor-core passes per
        product, ex2 / rcp cell update: fp32-grade results at ~0.4 of the single-pass throughput; needs weights_tcx; H = 128:
-       csrc/ape_lstm_tcx.cu, H = 256: csrc/ape_lstm_tcxs.cu),
+       csrc/ape_lstm_tcx.cu, H = 256: csrc/ape_lstm_tcxs.cu; all_steps != 0 needs the _all_steps workspace query),
        4 = the SMALL-BATCH kernel (csrc/ape_lstm_tcl.cu: B * nF * n_samples <= 8192 rows, L <= 4: all layers in one launch, one
        8-CTA cluster per 128 rows with the hidden units split across it - the real-time case of one to a few dozen streams; same
        arithmetic as 0..2; no initial state) */
@@ -151,7 +151,8 @@ typedef struct ape_lstm_args {
     /* optional initial state (h_0, c_0) of torch.nn.LSTM(x, hs) (nn_models.py:180-189): [L][E][H] float32 each, both or neither
        (APE_ERR_BAD_ARG); needs n_samples == 1 (APE_ERR_UNSUPPORTED; a caller with per-sample states passes the samples as estimates).
        Taken by the fp32 path and by the tensor-core path with tc_flags 0 or 1 (the one-layer kernels; tc_flags 0 then never pairs
-       layers; both pointers 16-byte aligned, else APE_ERR_BAD_ARG); tc_flags 2, 3 and 4 refuse it with APE_ERR_UNSUPPORTED */
+       layers) and with tc_flags 3 at H = 256 only (the split-precision kernel csrc/ape_lstm_tcxs.cu); both pointers 16-byte aligned,
+       else APE_ERR_BAD_ARG.  tc_flags 2 and 4, and 3 at H = 128, refuse it with APE_ERR_UNSUPPORTED */
     const float* h0;
     const float* c0;
     /* ---- ABI 6 ---- */
@@ -172,7 +173,7 @@ int ape_mc_lstm_fma(const ape_lstm_args* args, void* stream);
  * Tensor-core variant (tcgen05, cta_group::2, TMEM accumulators): fp16 operands, fp32 accumulation and cell state.
  * H in {64, 128} (gate weights resident in shared memory; H = 128, L >= 3: pairs of layers >= 1 as one two-layer wavefront launch
  * with weights streamed from L2) or 256 (gate weights streamed from L2 through a cp.async.bulk ring), L >= 2; same arguments and
- * outputs as ape_mc_lstm_fma plus weights_tc, h0 / c0 included (tc_flags 0 and 1 only; see the h0 field).
+ * outputs as ape_mc_lstm_fma plus weights_tc, h0 / c0 included (tc_flags 0 and 1, and 3 at H = 256; see the h0 field).
  * Use when the streams x MC-samples batch is large (>= a few thousand rows); the fp32 variant is the exact path.
  */
 int ape_mc_lstm_tc_supported(int I, int H, int L, int O);
@@ -185,12 +186,15 @@ int ape_mc_lstm_tc(const ape_lstm_args* args, void* stream);
 int ape_mc_lstm_tcx_supported(int I, int H, int L, int O);
 int ape_lstm_tcx_blob_bytes(int I, int H, int L, int64_t* bytes);
 int ape_mc_lstm_tcx_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes);
+/* workspace of a split-precision call with all_steps != 0 (keeps the last layer's sequence, hi and lo, for the per-step output layer) */
+int ape_mc_lstm_tcx_workspace_bytes_all_steps(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes);
 /* the same for the H = 256 split-precision kernel (csrc/ape_lstm_tcxs.cu; H = 256, I <= 256, O <= 32, L >= 2), which tc_flags == 3
    selects for an H = 256 model: its blob (packed by pack_lstm_weights_tcx() as well, the same layout at H = 256) also travels in
    weights_tcx, and the workspace must hold ape_mc_lstm_tcxs_workspace_bytes() */
 int ape_mc_lstm_tcxs_supported(int I, int H, int L, int O);
 int ape_lstm_tcxs_blob_bytes(int I, int H, int L, int64_t* bytes);
 int ape_mc_lstm_tcxs_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes);
+int ape_mc_lstm_tcxs_workspace_bytes_all_steps(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes);
 /* number of kernels ape_mc_lstm_tc launches for these arguments (layer pairs of an H = 128 model count once) */
 int ape_mc_lstm_tc_launch_count(const ape_lstm_args* args, int* launches);
 /*

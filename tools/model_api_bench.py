@@ -1,9 +1,11 @@
 """Throughput of DropoutLSTM's model API on the three deployed model shapes (dimensions read by hash, seeded weights): forward(x, hs) at 4096
-rows and monte_carlo_predictions(100, x, hs) under hs_variant fp32 / tc, and forward(x) at 4096 rows under lstm_variant fp32 / tc.
+rows and monte_carlo_predictions(100, x, hs) under hs_variant fp32 / tc / tcx, and forward(x) at 4096 rows under lstm_variant fp32 / tc / tcx.
 Inputs and states stay on the device; each entry is CUDA events around >= 50 warmed calls, repeated --rounds times with the variants
-alternated; the GPU name and power limit are read in the same run.
+alternated; the GPU name and power limit are read in the same run.  A variant that does not take a case (tcx with hs at H = 128) is
+recorded as not supported.
 
-    python tools/model_api_bench.py [--out profiles/model_api_bench.json] [--calls 50] [--rounds 3]
+    python tools/model_api_bench.py [--out profiles/model_api_split_bench.json] [--variants fp32,tc,tcx] [--calls 50] [--rounds 3]
+    (profiles/model_api_bench.json: --variants fp32,tc --out profiles/model_api_bench.json)
 """
 import argparse
 import json
@@ -19,7 +21,6 @@ from arm_pose_estimation_b200.estimate import nn_models  # noqa: E402
 from split256_bench import gpu_info  # noqa: E402
 
 ROWS, NS = 4096, 100
-VARIANTS = ("fp32", "tc")
 
 
 def time_calls(fn, calls):
@@ -34,12 +35,15 @@ def time_calls(fn, calls):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--out", default="profiles/model_api_bench.json")
+    ap.add_argument("--out", default="profiles/model_api_split_bench.json")
+    ap.add_argument("--variants", default="fp32,tc,tcx", help="comma-separated, fp32 first")
     ap.add_argument("--calls", type=int, default=50)
     ap.add_argument("--rounds", type=int, default=3)
     args = ap.parse_args()
     assert torch.cuda.is_available(), "needs a GPU"
     assert args.calls >= 50, "time at least 50 warmed calls"
+    variants = tuple(args.variants.split(","))
+    assert variants[0] == "fp32" and set(variants) <= {"fp32", "tc", "tcx"}, variants
     torch.cuda.set_device(0)
     result = {"gpu": gpu_info(), "calls": args.calls, "rounds": args.rounds,
               "workload": f"forward(x, hs) and forward(x) at {ROWS} rows, monte_carlo_predictions({NS}, x, hs); device-resident"}
@@ -48,7 +52,7 @@ def main():
         I, H, L, T, O = spec["I"], spec["H"], spec["L"], spec["T"], spec["O"]
         state = syn.synth_state_dict(I, H, L, O, 1234 + kind)
         models = {v: nn_models.DropoutLSTM(I, H, L, O, spec["p"], philox_seed=5, lstm_variant=v, hs_variant=v).load_state_dict(state).eval()
-                  for v in VARIANTS}
+                  for v in variants}
         g = torch.Generator(device="cpu").manual_seed(kind)
         x = torch.randn((ROWS, T, I), generator=g).cuda()
         hs = tuple((0.5 * torch.randn((L, ROWS, H), generator=g)).cuda() for _ in range(2))
@@ -60,24 +64,33 @@ def main():
         }
         entry = {"model": f"seeded weights of the deployed {syn.KIND_NAMES[kind]} shape ({spec['hash'][:8]}): I{I} H{H} L{L} T{T} O{O}"}
         for case, (rows, fn) in cases.items():
-            ms = {v: [] for v in VARIANTS}
-            for v in VARIANTS:                                  # warm-up (module load, workspace, probes)
-                for _ in range(3):
-                    fn(models[v])
+            e, run = {}, []
+            for v in variants:                                  # warm-up (module load, workspace, probes)
+                try:
+                    for _ in range(3):
+                        fn(models[v])
+                    run.append(v)
+                except UserWarning as w:                        # e.g. tcx with hs at H = 128: no split kernel takes a state there
+                    e[v] = {"not_supported": str(w)}
                 models[v].eval()
             torch.cuda.synchronize()
+            ms = {v: [] for v in run}
             for _ in range(args.rounds):
-                for v in VARIANTS:
+                for v in run:
                     ms[v].append(time_calls(lambda: fn(models[v]), args.calls))
                     models[v].eval()                            # (monte_carlo_predictions leaves the LSTM in train mode)
-            e = {}
-            for v in VARIANTS:
+            for v in run:
                 med = float(np.median(ms[v]))
                 e[v] = {"ms_per_call_median": med, "ms_per_call_all": ms[v], "rows_per_s": rows / med * 1e3}
-            e["tc_over_fp32"] = e["tc"]["rows_per_s"] / e["fp32"]["rows_per_s"]
+            line = f"{syn.KIND_NAMES[kind]} {case}: fp32 {e['fp32']['rows_per_s']:.4g} rows/s"
+            for v in variants[1:]:
+                if v in run:
+                    e[f"{v}_over_fp32"] = e[v]["rows_per_s"] / e["fp32"]["rows_per_s"]
+                    line += f", {v} {e[v]['rows_per_s']:.4g} rows/s ({e[f'{v}_over_fp32']:.2f}x)"
+                else:
+                    line += f", {v} not supported"
             entry[case] = e
-            print(f"{syn.KIND_NAMES[kind]} {case}: fp32 {e['fp32']['rows_per_s']:.4g} rows/s, tc {e['tc']['rows_per_s']:.4g} rows/s "
-                  f"({e['tc_over_fp32']:.2f}x)", flush=True)
+            print(line, flush=True)
         result[syn.KIND_NAMES[kind]] = entry
         del models
         torch.cuda.empty_cache()
