@@ -480,24 +480,15 @@ extern "C" int ape_mc_lstm_fma(const ape_lstm_args* g, void* stream) {
     float* seq0 = (float*)wsp;
     float* seq1[2] = {(float*)(wsp + p.seq0_bytes), (float*)(wsp + p.seq0_bytes + p.seq1_bytes)};
 
-    cudaEvent_t ev[17] = {};
-    const bool prof = g->layer_ms != nullptr && g->L <= 16;
-    if (prof) for (int l = 0; l <= g->L; ++l) APE_CUDA_TRY(cudaEventCreate(&ev[l]));
-    if (prof) APE_CUDA_TRY(cudaEventRecord(ev[0], st));
-
-    for (int l = 0; l < g->L; ++l) {
+    LayerTimer timer(g->layer_ms, g->L, st);
+    rc = timer.start();
+    for (int l = 0; l < g->L && rc == APE_OK; ++l) {
         const float* seq_in = l == 0 ? nullptr : (l == 1 ? seq0 : seq1[(l - 2) & 1]);
         float* seq_out = l == 0 ? seq0 : seq1[(l - 1) & 1];
         rc = fma_launch_layer(g, l, p, seq_in, seq_out, st);
-        if (rc != APE_OK) return rc;
-        if (prof) APE_CUDA_TRY(cudaEventRecord(ev[l + 1], st));
+        if (rc == APE_OK) rc = timer.mark(l + 1);
     }
-    if (prof) {
-        APE_CUDA_TRY(cudaStreamSynchronize(st));
-        for (int l = 0; l < g->L; ++l) APE_CUDA_TRY(cudaEventElapsedTime(&g->layer_ms[l], ev[l], ev[l + 1]));
-        for (int l = 0; l <= g->L; ++l) cudaEventDestroy(ev[l]);
-    }
-    return APE_OK;
+    return rc == APE_OK ? timer.finish() : rc;
 }
 
 extern "C" int ape_philox_masks(uint64_t philox_seed, uint32_t stream_id0, int B, int nF, int frame0, int L, int T,

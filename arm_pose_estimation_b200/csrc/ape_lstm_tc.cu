@@ -596,22 +596,31 @@ template <int H> static int launch(const TcLayerArgs& a, int sm_count, cudaStrea
 }  // namespace tc
 }  // namespace ape
 
-// rows per CTA of layer 0 (one row per estimate): a small batch is spread over more CTA pairs, 32 rows each
 constexpr int TC_MAX_SMS = 160;                    // cell-state scratch is sized for this many CTAs (B200: 148)
+// rows per CTA of layer 0 (one row per estimate): a small batch is spread over more CTA pairs, 32 rows each; the split-precision
+// kernels (tc_flags == 3) take 128 rows always
 // (128 rows from 512 estimates on: a 32-row CTA takes as long per step as a full one - its 4 live epilogue warps share one SM quarter -
 // so spreading layer 0 of a large batch over 4x the SMs only takes them away from the big layers that run beside it: +1 % per step)
-static int tc_rpc0(long long E) { return E >= 512 ? 128 : 32; }
+static int tc_rpc0(bool split, long long E) { return split || E >= 512 ? 128 : 32; }
 static int tc_kgx(int layer, int I, int H) { return layer == 0 ? ape_pack_kin_pad(0, I, H) / 8 : H / 8; }
 static size_t tc_layer_bytes(int layer, int I, int H) {
     return (size_t)2 * (H / 32) * (tc_kgx(layer, I, H) + H / 8) * 64 * 16 + (size_t)4 * H * 4;
 }
+// fp16 output-layer tiles (TcLayerArgs::Wo16) after the layers: 2 CTAs x [H/8][16 | 32 (H = 256) columns][8] halfs
+static size_t tc_wo16_bytes(int H) { return (size_t)2 * (H / 8) * (H > 128 ? 32 : 16) * 16; }
+// bytes of layer l in the single-pass blob (weights_tc) or in the split-precision blob (weights_tcx: per layer the pieces of
+// ape_lstm_tcx.cu, H = 256 ape_lstm_tcxs.cu, then the kernel's output-layer tiles)
+static size_t blob_layer_bytes(bool split, int layer, int I, int H) {
+    return !split ? tc_layer_bytes(layer, I, H) : H == 256 ? ape::tcxs::layer_bytes(layer, I) : ape::tcx::layer_bytes(layer, I);
+}
 
-// bytes of the fp16 weight blob of the tensor-core path: per layer the two CTAs' weight tiles, then the scaled bias
+// bytes of the fp16 weight blob of the tensor-core path: per layer the two CTAs' weight tiles, then the scaled bias; then the
+// output-layer tiles and (L >= 3) the wavefront kernel's pieces of layers >= 1
 extern "C" int ape_lstm_tc_blob_bytes(int I, int H, int L, int64_t* bytes) {
     if (!bytes || I < 1 || H < 32 || H % 32 != 0 || L < 1) return APE_ERR_BAD_ARG;
     int64_t total = 0;
     for (int l = 0; l < L; ++l) total += (int64_t)tc_layer_bytes(l, I, H);
-    total += (int64_t)2 * (H / 8) * (H > 128 ? 32 : 16) * 16;              // fp16 output-layer tiles: 2 CTAs x [H/8][16 | 32 (H = 256) columns][8] halfs
+    total += (int64_t)tc_wo16_bytes(H);
     if (L >= 3) total += (int64_t)(L - 1) * (int64_t)ape::tcw::layer_bytes(H);   // wavefront kernel's pieces of layers >= 1 (H = 128)
     *bytes = total;
     return APE_OK;
@@ -623,29 +632,40 @@ extern "C" int ape_mc_lstm_tc_supported(int I, int H, int L, int O) {
             ape_pack_kin_pad(0, I, H) <= H && O >= 1) ? 1 : 0;
 }
 
+// shapes of the split-precision kernels (tc_flags == 3)
+static bool split_supported(int I, int H, int L, int O) {
+    return L >= 2 && I >= 1 && O >= 1 && (H == 256 ? ape::tcxs::supported(H, I, O) : ape::tcx::supported(H, I, O));
+}
+
 // Workspace layout of the tensor-core path, computed from the LARGEST call that will use the workspace (ws_E) so that calls of
 // different sizes in flight on different streams agree on every offset:
 //   [2 x scratch region][layer 0 output, copy 0][copy 1][units of layers >= 1, up to 2 buffers (+ 1 for all_steps)]
+// Split precision: every units buffer is a (hi, lo) pair, the lo halves behind the hi halves.
 struct TcWsLayout { size_t scratch_region, u0, u1, total; };
-static size_t tc_u0_bytes(long long E, int T, int H) {
-    const unsigned long long rpc0 = tc_rpc0(E), tiles0 = ((unsigned long long)E + 2 * rpc0 - 1) / (2 * rpc0);
+static size_t tc_u0_bytes(bool split, long long E, int T, int H) {
+    const unsigned long long rpc0 = tc_rpc0(split, E), tiles0 = ((unsigned long long)E + 2 * rpc0 - 1) / (2 * rpc0);
     return (size_t)((tiles0 * 256 * T * H * 2 + 255) & ~(unsigned long long)255);
 }
-static TcWsLayout tc_ws_layout(int H, int L, int T, long long E, int n_samples, bool all_steps) {
+static TcWsLayout tc_ws_layout(bool split, int H, int L, int T, long long E, int n_samples, bool all_steps) {
     TcWsLayout w{};
-    // a short call (< 512 estimates) spreads layer 0 over 32-row CTAs and needs up to 4x the row slots per estimate
-    w.u0 = tc_u0_bytes(E, T, H);
-    if (E > 511) { const size_t small = tc_u0_bytes(511, T, H); if (small > w.u0) w.u0 = small; }
+    // a short call (< 512 estimates) spreads layer 0 over 32-row CTAs and needs up to 4x the row slots per estimate (single pass)
+    w.u0 = tc_u0_bytes(split, E, T, H);
+    if (E > 511) { const size_t small = tc_u0_bytes(split, 511, T, H); if (small > w.u0) w.u0 = small; }
     const unsigned long long tiles1 = ((unsigned long long)E * n_samples + 255) / 256;
     w.u1 = (size_t)((tiles1 * 256 * T * H * 2 + 255) & ~(unsigned long long)255);
     // per-CTA cell-state scratch: two regions (layer 0 of the next call may run on a side stream under a layer >= 1 of this one);
-    // streamed-weights kernel (H = 256) and two-layer wavefront kernel (H = 128, L >= 3)
-    w.scratch_region = ape::tcs::scratch_bytes(H, TC_MAX_SMS);
-    if (L >= 3) { const size_t s2 = ape::tcw::scratch_bytes(H, TC_MAX_SMS); if (s2 > w.scratch_region) w.scratch_region = s2; }
+    // streamed-weights kernel (H = 256), two-layer wavefront kernel (H = 128, L >= 3) and split-precision kernels
+    if (split) {
+        w.scratch_region = H == 256 ? ape::tcxs::scratch_bytes(TC_MAX_SMS) : ape::tcx::scratch_bytes(TC_MAX_SMS);
+    } else {
+        w.scratch_region = ape::tcs::scratch_bytes(H, TC_MAX_SMS);
+        if (L >= 3) { const size_t s2 = ape::tcw::scratch_bytes(H, TC_MAX_SMS); if (s2 > w.scratch_region) w.scratch_region = s2; }
+    }
     const int n_u1 = L - 2 + (all_steps ? 1 : 0);
-    w.total = 2 * w.scratch_region + 2 * w.u0 + (size_t)(n_u1 > 2 ? 2 : (n_u1 < 0 ? 0 : n_u1)) * w.u1 + 512;
+    const size_t planes = split ? 2 : 1;
+    w.total = 2 * w.scratch_region + 2 * planes * w.u0 + (size_t)(n_u1 > 2 ? 2 : (n_u1 < 0 ? 0 : n_u1)) * planes * w.u1 + 512;
     // the small-batch cluster kernel (tc_flags == 4) keeps its exchange buffers where the layer kernels keep their units: one set per cluster
-    if (!all_steps && (H == 128 || H == 256) && E * n_samples <= 128LL * 64) {
+    if (!split && !all_steps && (H == 128 || H == 256) && E * n_samples <= 128LL * 64) {
         const size_t need = 2 * w.scratch_region + ape::tcl::workspace_bytes(H, T, E * n_samples) + 512;
         if (need > w.total) w.total = need;
     }
@@ -655,7 +675,7 @@ static TcWsLayout tc_ws_layout(int H, int L, int T, long long E, int n_samples, 
 extern "C" int ape_mc_lstm_tc_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
     if (!bytes || I < 1 || H < 1 || L < 1 || T < 1 || O < 1 || E < 0 || n_samples < 1) return APE_ERR_BAD_ARG;
     if (!ape_mc_lstm_tc_supported(I, H, L, O)) return APE_ERR_UNSUPPORTED;
-    *bytes = tc_ws_layout(H, L, T, E, n_samples, false).total;
+    *bytes = tc_ws_layout(false, H, L, T, E, n_samples, false).total;
     return APE_OK;
 }
 
@@ -663,16 +683,53 @@ extern "C" int ape_mc_lstm_tc_workspace_bytes(int I, int H, int L, int T, int O,
 extern "C" int ape_mc_lstm_tc_workspace_bytes_all_steps(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
     if (!bytes || I < 1 || H < 1 || L < 1 || T < 1 || O < 1 || E < 0 || n_samples < 1) return APE_ERR_BAD_ARG;
     if (!ape_mc_lstm_tc_supported(I, H, L, O)) return APE_ERR_UNSUPPORTED;
-    *bytes = tc_ws_layout(H, L, T, E, n_samples, true).total;
+    *bytes = tc_ws_layout(false, H, L, T, E, n_samples, true).total;
     return APE_OK;
 }
 
-// (a caller-supplied initial state runs on the one-layer kernels: the wavefront kernel takes none)
-static bool tc_pairs_layers(const ape_lstm_args* g, long long tiles1, int sm_count) {
-    return ape::tcw::supported(g->H, g->T, g->O) && g->tc_flags != 1 && g->h0 == nullptr && (g->tc_flags == 2 || tiles1 >= sm_count / 2);
+// The split-precision queries: the tcx_* symbols answer for the H = 128 kernel, the tcxs_* symbols for the H = 256 one.
+static int split_blob_query(int kernel_H, int I, int H, int L, int64_t* bytes) {
+    if (!bytes || H != kernel_H || !split_supported(I, H, L, 1)) return APE_ERR_BAD_ARG;
+    int64_t total = (int64_t)(H == 256 ? ape::tcxs::wo16_bytes() : ape::tcx::wo16_bytes());
+    for (int l = 0; l < L; ++l) total += (int64_t)blob_layer_bytes(true, l, I, H);
+    *bytes = total;
+    return APE_OK;
+}
+static int split_workspace_query(int kernel_H, int I, int H, int L, int T, int O, int E, int n_samples, bool all_steps, uint64_t* bytes) {
+    if (!bytes || T < 1 || E < 0 || n_samples < 1) return APE_ERR_BAD_ARG;
+    if (H != kernel_H || !split_supported(I, H, L, O)) return APE_ERR_UNSUPPORTED;
+    *bytes = tc_ws_layout(true, H, L, T, E, n_samples, all_steps).total;
+    return APE_OK;
+}
+extern "C" int ape_mc_lstm_tcx_supported(int I, int H, int L, int O) { return H == 128 && split_supported(I, H, L, O); }
+extern "C" int ape_mc_lstm_tcxs_supported(int I, int H, int L, int O) { return H == 256 && split_supported(I, H, L, O); }
+extern "C" int ape_lstm_tcx_blob_bytes(int I, int H, int L, int64_t* bytes) { return split_blob_query(128, I, H, L, bytes); }
+extern "C" int ape_lstm_tcxs_blob_bytes(int I, int H, int L, int64_t* bytes) { return split_blob_query(256, I, H, L, bytes); }
+extern "C" int ape_mc_lstm_tcx_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
+    return split_workspace_query(128, I, H, L, T, O, E, n_samples, false, bytes);
+}
+extern "C" int ape_mc_lstm_tcx_workspace_bytes_all_steps(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
+    return split_workspace_query(128, I, H, L, T, O, E, n_samples, true, bytes);
+}
+extern "C" int ape_mc_lstm_tcxs_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
+    return split_workspace_query(256, I, H, L, T, O, E, n_samples, false, bytes);
+}
+extern "C" int ape_mc_lstm_tcxs_workspace_bytes_all_steps(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
+    return split_workspace_query(256, I, H, L, T, O, E, n_samples, true, bytes);
 }
 
-// kernels ape_mc_lstm_tc will launch for these arguments (bench.py's gpu_launches; depends on the pairing rule above)
+// Two consecutive layers >= 1 of an H = 128 model run as ONE wavefront launch (ape_lstm_tcw.cu) when the batch gives every CTA pair
+// at least one tile (below that a lone tile is faster through two one-layer launches: its two layers cannot overlap on the epilogue
+// warps of one pair); tc_flags 1 / 2 force either way.  (A caller-supplied initial state runs on the one-layer kernels: the wavefront
+// kernel takes none; the split-precision kernels have no wavefront form.)
+static bool tc_pairs_layers(const ape_lstm_args* g, long long tiles1, int sm_count) {
+    return ape::tcw::supported(g->H, g->T, g->O) && g->tc_flags != 1 && g->tc_flags != 3 && g->h0 == nullptr &&
+           (g->tc_flags == 2 || tiles1 >= sm_count / 2);
+}
+// layers of the launch that starts at layer l of the range [.., l_end)
+static int layers_in_launch(bool pair_ok, int l, int l_end) { return pair_ok && l >= 1 && l + 1 < l_end ? 2 : 1; }
+
+// kernels ape_mc_lstm_tc will launch for these arguments (bench.py's gpu_launches)
 extern "C" int ape_mc_lstm_tc_launch_count(const ape_lstm_args* g, int* launches) {
     if (!g || !launches) return APE_ERR_BAD_ARG;
     int dev = 0, sm_count = 0;
@@ -682,9 +739,9 @@ extern "C" int ape_mc_lstm_tc_launch_count(const ape_lstm_args* g, int* launches
     const int l_begin = (g->layer_begin == 0 && g->layer_end == 0) ? 0 : g->layer_begin;
     const int l_end = (g->layer_begin == 0 && g->layer_end == 0) ? g->L : g->layer_end;
     if (g->tc_flags == 4) { *launches = 1; return APE_OK; }
-    const bool pair_ok = g->tc_flags != 3 && tc_pairs_layers(g, (rows + 255) / 256, sm_count);
+    const bool pair_ok = tc_pairs_layers(g, (rows + 255) / 256, sm_count);
     int n = 0;
-    for (int l = l_begin; l < l_end;) { ++n; l += (pair_ok && l >= 1 && l + 1 < l_end) ? 2 : 1; }
+    for (int l = l_begin; l < l_end; l += layers_in_launch(pair_ok, l, l_end)) ++n;
     *launches = n + (g->all_steps ? 1 : 0);
     return APE_OK;
 }
@@ -698,36 +755,33 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
     if (g->h0 && (g->tc_flags == 2 || (g->tc_flags == 3 && g->H != 256) || g->tc_flags == 4)) return APE_ERR_UNSUPPORTED;
     // the state kernels read h_0 / c_0 rows as float4 (H is a multiple of 32, so every layer's block keeps the base alignment)
     if (((uintptr_t)g->h0 | (uintptr_t)g->c0) & 15) return APE_ERR_BAD_ARG;
-    if (g->tc_flags == 3)                                      // split-precision variant (csrc/ape_lstm_tcx.cu, H = 256: ape_lstm_tcxs.cu)
-        return g->H == 256 ? ape::tcxs::run(g, (cudaStream_t)stream) : ape::tcx::run(g, (cudaStream_t)stream);
-    if (!ape_mc_lstm_tc_supported(g->I, g->H, g->L, g->O)) return APE_ERR_UNSUPPORTED;
+    // tc_flags == 3: the split-precision kernels (csrc/ape_lstm_tcx.cu, H = 256: ape_lstm_tcxs.cu) and their blob, weights_tcx
+    const bool split = g->tc_flags == 3;
+    if (!(split ? split_supported(g->I, g->H, g->L, g->O) : ape_mc_lstm_tc_supported(g->I, g->H, g->L, g->O))) return APE_ERR_UNSUPPORTED;
     if (g->all_steps && (g->layer_begin != 0 || g->layer_end != 0)) return APE_ERR_UNSUPPORTED;
     if (g->T > 40) return APE_ERR_UNSUPPORTED;                 // |c_t| <= t keeps 2^(2 c log2e) finite in fp32 only for T <= 44
                                                                // (with a state |c_t| <= |c_0| + t: the state kernels clamp it)
-    if (!g->weights_tc) return APE_ERR_BAD_ARG;
+    const uint8_t* blob = (const uint8_t*)(split ? g->weights_tcx : g->weights_tc);
+    if (!blob || (split && !g->workspace)) return APE_ERR_BAD_ARG;     // (a split call needs the workspace even when it is empty)
     const long long E = (long long)g->B * g->nF;
     if (E == 0) return APE_OK;
-    if (!g->workspace) return APE_ERR_BAD_ARG;
+    if (!g->workspace || (g->ws_E != 0 && g->ws_E < E)) return APE_ERR_BAD_ARG;
     cudaStream_t st = (cudaStream_t)stream;
     int dev = 0, sm_count = 0;
     APE_CUDA_TRY(cudaGetDevice(&dev));
     APE_CUDA_TRY(cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev));
 
+    const int H = g->H;
     const long long rows = E * g->n_samples;
-    const int rpc0 = tc_rpc0(E);
+    const int rpc0 = tc_rpc0(split, E);
     const int tiles0 = (int)((E + 2 * rpc0 - 1) / (2 * rpc0)), tiles1 = (int)((rows + 255) / 256);
-    if (g->ws_E != 0 && g->ws_E < E) return APE_ERR_BAD_ARG;
-    const TcWsLayout wl_ = tc_ws_layout(g->H, g->L, g->T, g->ws_E > 0 ? g->ws_E : E, g->n_samples, g->all_steps != 0);
-    const size_t u0 = wl_.u0, u1 = wl_.u1;
+    const bool all_steps = g->all_steps != 0;
+    const TcWsLayout wl = tc_ws_layout(split, H, g->L, g->T, g->ws_E > 0 ? g->ws_E : E, g->n_samples, all_steps);
     char* wsp = (char*)(((uintptr_t)g->workspace + 255) & ~(uintptr_t)255);
     // per-CTA cell-state scratch at the front (a position that does not depend on the call's size)
     char* scratch = wsp;
-    const size_t scratch_region = wl_.scratch_region;
-    if (scratch_region && sm_count > TC_MAX_SMS) return APE_ERR_UNSUPPORTED;
-    wsp += 2 * scratch_region;
-    uint4* units0 = (uint4*)(wsp + (g->ws_parity & 1) * u0);            // layer 0 output, one row per estimate (two copies)
-    // layers >= 1 outputs, one row per (estimate, sample) (all_steps: the last layer's sequence is kept too, for the per-step output layer)
-    uint4* units[2] = {(uint4*)(wsp + 2 * u0), (uint4*)(wsp + 2 * u0 + u1)};
+    if (wl.scratch_region && sm_count > TC_MAX_SMS) return APE_ERR_UNSUPPORTED;
+    wsp += 2 * wl.scratch_region;
     const int l_begin = (g->layer_begin == 0 && g->layer_end == 0) ? 0 : g->layer_begin;
     const int l_end = (g->layer_begin == 0 && g->layer_end == 0) ? g->L : g->layer_end;
     if (l_begin < 0 || l_end > g->L || l_begin >= l_end) return APE_ERR_BAD_ARG;
@@ -737,46 +791,49 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
         if (l_begin != 0 || l_end != g->L || g->L > 4) return APE_ERR_UNSUPPORTED;
         const uint8_t* lw[4] = {};
         const float* lb[4] = {};
-        const uint8_t* p = (const uint8_t*)g->weights_tc;
+        const uint8_t* p = blob;
         for (int l = 0; l < g->L; ++l) {
             lw[l] = p;
             p += tc_layer_bytes(l, g->I, g->H);
             lb[l] = (const float*)(p - (size_t)4 * g->H * 4);
         }
-        cudaEvent_t e0 = nullptr, e1 = nullptr;
-        if (g->layer_ms) { APE_CUDA_TRY(cudaEventCreate(&e0)); APE_CUDA_TRY(cudaEventCreate(&e1)); APE_CUDA_TRY(cudaEventRecord(e0, st)); }
-        rc = ape::tcl::run(g, lw, lb, p, wsp, st);
-        if (rc != APE_OK) return rc;
-        if (g->layer_ms) {                                  // the one launch is reported as layer 0's time
-            APE_CUDA_TRY(cudaEventRecord(e1, st));
-            APE_CUDA_TRY(cudaStreamSynchronize(st));
-            for (int l = 0; l < g->L; ++l) g->layer_ms[l] = 0.0f;
-            APE_CUDA_TRY(cudaEventElapsedTime(&g->layer_ms[0], e0, e1));
-            cudaEventDestroy(e0); cudaEventDestroy(e1);
-        }
-        return APE_OK;
+        LayerTimer timer(g->layer_ms, g->L, st);               // the one launch is reported as layer 0's time
+        rc = timer.start();
+        if (rc == APE_OK) rc = ape::tcl::run(g, lw, lb, p, wsp, st);
+        if (rc == APE_OK) rc = timer.mark(g->L);
+        return rc == APE_OK ? timer.finish() : rc;
     }
+    // SMs the launches of layers >= 1 leave free (a whole number of SM pairs): a concurrent stage 1 + layer 0 of the NEXT call - a few
+    // CTAs on a high-priority stream - then never has to wait for a persistent launch to retire CTAs
+    if (g->reserve_sms < 0 || g->reserve_sms > sm_count - 2) return APE_ERR_BAD_ARG;
+    const int sm_big = sm_count - ((g->reserve_sms + 1) & ~1);
 
-    cudaEvent_t ev[17] = {};
-    const bool prof = g->layer_ms != nullptr && g->L <= 16 && l_begin == 0 && l_end == g->L;
-    if (prof) for (int l = 0; l <= g->L; ++l) APE_CUDA_TRY(cudaEventCreate(&ev[l]));
-    if (prof) APE_CUDA_TRY(cudaEventRecord(ev[0], st));
-
-    const int H = g->H;
-    const uint8_t* wl = (const uint8_t*)g->weights_tc;
-    const uint8_t* wo16 = wl;                                               // the fp16 output-layer tile sits after all layers,
-    for (int l = 0; l < g->L; ++l) wo16 += tc_layer_bytes(l, g->I, g->H);
-    const size_t ww_layer = g->L >= 3 ? ape::tcw::layer_bytes(g->H) : 0;     // ... then the wavefront kernel's pieces of layers 1 .. L-1
-    const uint8_t* ww = wo16 + (size_t)2 * (g->H / 8) * (g->H > 128 ? 32 : 16) * 16;
+    // units between layers: layer 0's output (two copies, one row per estimate), the outputs of layers >= 1 (one row per (estimate,
+    // sample); all_steps: the last layer's sequence is kept too, for the per-step output layer); split: the lo halves behind the hi
+    struct Units { uint4 *hi, *lo; };
+    const size_t planes = split ? 2 : 1;
+    auto units_at = [&](char* p, size_t bytes) { return Units{(uint4*)p, split ? (uint4*)(p + bytes) : nullptr}; };
+    const Units units0 = units_at(wsp + (g->ws_parity & 1) * planes * wl.u0, wl.u0);
+    const Units units[2] = {units_at(wsp + 2 * planes * wl.u0, wl.u1), units_at(wsp + 2 * planes * wl.u0 + planes * wl.u1, wl.u1)};
+    auto layer_w = [&](int l) {                                            // layer l's weights inside the blob
+        const uint8_t* p = blob;
+        for (int k = 0; k < l; ++k) p += blob_layer_bytes(split, k, g->I, H);
+        return p;
+    };
+    const uint8_t* wo16 = layer_w(g->L);                                    // the fp16 output-layer tile sits after all layers,
+    const size_t ww_layer = !split && g->L >= 3 ? tcw::layer_bytes(H) : 0;  // ... then the wavefront kernel's pieces of layers 1 .. L-1
+    const uint8_t* ww = wo16 + tc_wo16_bytes(H);
     const float scale = g->mask_mode == APE_MASK_NONE ? 1.0f : 1.0f / (1.0f - g->dropout_p);
-    const bool all_steps = g->all_steps != 0;
-    // argument block of layer l (`wl_l`: its weights inside the fp16 blob)
-    auto layer_args = [&](int l, const uint8_t* wl_l) {
+    auto layer_args = [&](int l) {
         const bool last = l == g->L - 1;
         tc::TcLayerArgs a{};
-        a.W = wl_l;
-        a.bias_s = (const float*)(wl_l + tc_layer_bytes(l, g->I, H) - (size_t)4 * H * 4);
-        a.Ww = (ww_layer && l >= 1) ? ww + (size_t)(l - 1) * ww_layer : nullptr;
+        if (split) {
+            a.Ww = layer_w(l);                                              // the split kernels stream all of a layer's pieces
+        } else {
+            a.W = layer_w(l);
+            a.bias_s = (const float*)(a.W + tc_layer_bytes(l, g->I, H) - (size_t)4 * H * 4);
+            a.Ww = (ww_layer && l >= 1) ? ww + (size_t)(l - 1) * ww_layer : nullptr;
+        }
         a.T = g->T;
         a.kgx = tc_kgx(l, g->I, H);
         a.Kin = l == 0 ? g->I : H;
@@ -788,16 +845,17 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
             a.rpc = rpc0;
             a.n_pair_tiles = tiles0;
             a.mask_mode = APE_MASK_NONE;
-            a.out_units = units0;
+            a.out_units = units0.hi; a.out_units_lo = units0.lo;
         } else {
+            const Units& in = l == 1 ? units0 : units[(l - 2) & 1];
             a.in_mode = l == 1 ? tc::IN_SHARED_UNITS : tc::IN_UNITS;
-            a.in = l == 1 ? (const void*)units0 : (const void*)units[(l - 2) & 1];
+            a.in = in.hi; a.in_lo = in.lo;
             a.rows = (int)rows; a.n = g->n_samples;
             a.rpc = 128;
             a.in_rpc_shift = rpc0 == 128 ? 7 : 5;
             a.n_pair_tiles = tiles1;
             a.mask_mode = g->mask_mode;
-            a.out_units = (last && !all_steps) ? nullptr : units[(l - 1) & 1];
+            if (!last || all_steps) { a.out_units = units[(l - 1) & 1].hi; a.out_units_lo = units[(l - 1) & 1].lo; }
         }
         a.masks = g->masks; a.gap = l - 1; a.n_gaps = g->L - 1;
         a.seed = g->philox_seed; a.stream_id0 = g->stream_id0;
@@ -811,7 +869,7 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
         a.Wo16 = wo16;
         a.preds = (last && !all_steps) ? g->preds : nullptr;
         a.pred_ring = g->pred_ring; a.n_out = g->n_samples;
-        a.cstate = scratch_region ? (float*)(scratch + (l == 0 ? 0 : scratch_region)) : nullptr;
+        a.cstate = wl.scratch_region ? (float*)(scratch + (l == 0 ? 0 : wl.scratch_region)) : nullptr;
         a.h0 = g->h0 ? g->h0 + (size_t)l * E * H : nullptr;   // [L][E][H]: with a state every layer has E rows (n_samples == 1)
         a.c0 = g->c0 ? g->c0 + (size_t)l * E * H : nullptr;
         a.trace = (g->trace && l == g->trace_layer) ? (long long*)g->trace : nullptr;
@@ -819,43 +877,21 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
         a.timeline = (g->trace && g->trace_layer < 0) ? (long long*)g->trace + (size_t)l * TC_MAX_SMS * 4 : nullptr;
         return a;
     };
-    // Two consecutive layers >= 1 of an H = 128 model run as ONE wavefront launch (ape_lstm_tcw.cu) when the batch gives every
-    // CTA pair at least one tile (below that a lone tile is faster through two one-layer launches: its two layers cannot overlap
-    // on the epilogue warps of one pair); tc_flags forces either way.
     const bool pair_ok = tc_pairs_layers(g, tiles1, sm_count);
-    // SMs the launches of layers >= 1 leave free (a whole number of SM pairs): a concurrent stage 1 + layer 0 of the NEXT call - a few
-    // CTAs on a high-priority stream - then never has to wait for a persistent launch to retire CTAs
-    if (g->reserve_sms < 0 || g->reserve_sms > sm_count - 2) return APE_ERR_BAD_ARG;
-    const int sm_big = sm_count - ((g->reserve_sms + 1) & ~1);
-    for (int l = 0; l < l_end;) {
-        const uint8_t* wl_l = wl;
-        wl += tc_layer_bytes(l, g->I, H);
-        if (l < l_begin) { ++l; continue; }
-        const tc::TcLayerArgs a = layer_args(l, wl_l);
-        if (pair_ok && l >= 1 && l + 1 < l_end) {
-            const tc::TcLayerArgs b = layer_args(l + 1, wl);
-            wl += tc_layer_bytes(l + 1, g->I, H);
-            rc = tcw::launch_pair(a, b, sm_big, st);
-            if (rc != APE_OK) return rc;
-            if (prof) { APE_CUDA_TRY(cudaEventRecord(ev[l + 1], st)); APE_CUDA_TRY(cudaEventRecord(ev[l + 2], st)); }   // layer_ms[l] = the pair, [l+1] = 0
-            l += 2;
-            continue;
-        }
+    LayerTimer timer(l_begin == 0 && l_end == g->L ? g->layer_ms : nullptr, g->L, st);   // (a pair's time goes to its first layer)
+    rc = timer.start();
+    for (int l = l_begin, n; l < l_end && rc == APE_OK; l += n) {
+        n = layers_in_launch(pair_ok, l, l_end);
+        const tc::TcLayerArgs a = layer_args(l);
         const int sms = l == 0 ? sm_count : sm_big;
-        rc = H == 128 ? tc::launch<128>(a, sms, st) : H == 64 ? tc::launch<64>(a, sms, st) : tcs::launch_layer(H, a, sms, st);
-        if (rc != APE_OK) return rc;
-        if (prof) APE_CUDA_TRY(cudaEventRecord(ev[l + 1], st));
-        ++l;
+        if (n == 2)     rc = tcw::launch_pair(a, layer_args(l + 1), sm_big, st);
+        else if (split) rc = H == 256 ? tcxs::launch_layer(a, sms, st) : tcx::launch_layer(a, sms, st);
+        else            rc = H == 128 ? tc::launch<128>(a, sms, st) : H == 64 ? tc::launch<64>(a, sms, st) : tcs::launch_layer(H, a, sms, st);
+        if (rc == APE_OK) rc = timer.mark(l + n);
     }
-    if (all_steps) {                                            // output layer on every step (nn_models.py:189: output_layer(all))
-        rc = tc::launch_units_output(units[(g->L - 2) & 1], nullptr, g->weights + ape_pack_out_offset(g->I, g->H, g->L), g->preds, rows,
-                                     g->T, H, g->O, st);
-        if (rc != APE_OK) return rc;
+    if (rc == APE_OK && all_steps) {                           // output layer on every step (nn_models.py:189: output_layer(all)); split: hi + lo
+        const Units& seq = units[(g->L - 2) & 1];
+        rc = tc::launch_units_output(seq.hi, seq.lo, g->weights + ape_pack_out_offset(g->I, g->H, g->L), g->preds, rows, g->T, H, g->O, st);
     }
-    if (prof) {
-        APE_CUDA_TRY(cudaStreamSynchronize(st));
-        for (int l = 0; l < g->L; ++l) APE_CUDA_TRY(cudaEventElapsedTime(&g->layer_ms[l], ev[l], ev[l + 1]));
-        for (int l = 0; l <= g->L; ++l) cudaEventDestroy(ev[l]);
-    }
-    return APE_OK;
+    return rc == APE_OK ? timer.finish() : rc;
 }

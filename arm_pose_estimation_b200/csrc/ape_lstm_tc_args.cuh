@@ -1,6 +1,8 @@
-// Shared between the two tensor-core MC-LSTM layer kernels: ape_lstm_tc.cu (gate weights resident in shared memory,
-// H <= 128) and ape_lstm_tcs.cu (gate weights streamed from L2 through a TMA ring, H = 256): the per-layer argument
-// block, the input modes and the transcendental helpers of the cell update.
+// Shared by the tensor-core MC-LSTM kernels and by ape_mc_lstm_tc (ape_lstm_tc.cu), whose one host-side layer walk launches them:
+// the per-layer argument block, the input modes, the transcendental helpers of the cell update, and each kernel's host entry
+// points - ape_lstm_tc.cu (gate weights resident in shared memory, H <= 128), ape_lstm_tcs.cu (gate weights streamed from L2
+// through a TMA ring, H = 256), ape_lstm_tcw.cu (two layers per launch, H = 128), ape_lstm_tcx.cu / ape_lstm_tcxs.cu (split
+// precision, H = 128 / 256) and ape_lstm_tcl.cu (all layers of a small call in one launch).
 #pragma once
 #include "ape_f32x2.cuh"
 #include "ape_common.cuh"
@@ -161,19 +163,18 @@ namespace tcx {
 // split-precision kernel (ape_lstm_tcx.cu): every operand an fp16 pair hi + lo, three tensor-core passes per product, ex2 / rcp cell
 bool supported(int H, int I, int O);
 size_t layer_bytes(int layer, int I);            // bytes of one layer's pieces (TcLayerArgs::Ww), both CTAs
+size_t wo16_bytes();                             // bytes of the output-layer tiles after the last layer (TcLayerArgs::Wo16), both CTAs
 size_t scratch_bytes(int sm_count);              // per-CTA cell-state scratch of one launch
 int launch_layer(const tc::TcLayerArgs& a, int sm_count, cudaStream_t st);
-int run(const ape_lstm_args* g, cudaStream_t st);    // all layers of a call (ape_mc_lstm_tc with tc_flags == 3)
-size_t blob_bytes(int I, int L);
-size_t workspace_bytes(int L, int T, long long E, int n_samples, bool all_steps);
 }  // namespace tcx
 
 namespace tcxs {
 // split-precision kernel for H = 256 (ape_lstm_tcxs.cu): the arithmetic and blob layout of tcx, h_t staged through L2 into
 // single-buffered TMEM operands
 bool supported(int H, int I, int O);
-int run(const ape_lstm_args* g, cudaStream_t st);    // all layers of a call (ape_mc_lstm_tc with tc_flags == 3, H = 256; h0 / c0 taken)
-size_t blob_bytes(int I, int L);
-size_t workspace_bytes(int L, int T, long long E, int n_samples, bool all_steps);
+size_t layer_bytes(int layer, int I);
+size_t wo16_bytes();
+size_t scratch_bytes(int sm_count);              // per-CTA cell state and h_t staging of one launch
+int launch_layer(const tc::TcLayerArgs& a, int sm_count, cudaStream_t st);    // a.h0 / a.c0: the state variant
 }  // namespace tcxs
 }  // namespace ape

@@ -604,154 +604,7 @@ int launch_layer(const TcLayerArgs& a, int sm_count, cudaStream_t st) {
     return check_launch();
 }
 
-constexpr int MAX_SMS = 160;                       // the scratch is sized for this many CTAs (B200: 148)
-constexpr size_t WO16_BYTES = (size_t)2 * OUT_BYTES;
-
-size_t blob_bytes(int I, int L) {
-    size_t total = WO16_BYTES;
-    for (int l = 0; l < L; ++l) total += layer_bytes(l, I);
-    return total;
-}
-
-// workspace: [2 x scratch][layer 0 output: 2 copies x (hi, lo)][layers >= 1 outputs: up to 2 buffers x (hi, lo)]
-// (all_steps: the last layer's sequence is kept too, for the per-step output layer - one more (hi, lo) pair while L < 4)
-struct WsLayout { size_t scratch, u0, u1, total; int n_u1; };
-static WsLayout ws_layout(int L, int T, long long E, int n_samples, bool all_steps) {
-    WsLayout w{};
-    w.scratch = scratch_bytes(MAX_SMS);
-    const unsigned long long tiles0 = ((unsigned long long)E + 255) / 256, tiles1 = ((unsigned long long)E * n_samples + 255) / 256;
-    w.u0 = (size_t)((tiles0 * 256 * T * H * 2 + 255) & ~(unsigned long long)255);
-    w.u1 = (size_t)((tiles1 * 256 * T * H * 2 + 255) & ~(unsigned long long)255);
-    const int n_u1 = L - 2 + (all_steps ? 1 : 0);
-    w.n_u1 = n_u1 > 2 ? 2 : (n_u1 < 0 ? 0 : n_u1);
-    w.total = 2 * w.scratch + 4 * w.u0 + 2 * (size_t)w.n_u1 * w.u1 + 512;
-    return w;
-}
-size_t workspace_bytes(int L, int T, long long E, int n_samples, bool all_steps) { return ws_layout(L, T, E, n_samples, all_steps).total; }
-
-int run(const ape_lstm_args* g, cudaStream_t st) {
-    if (!supported(g->H, g->I, g->O) || g->L < 2) return APE_ERR_UNSUPPORTED;
-    // (h0 / c0: both or neither, n_samples == 1 and 16-byte alignment are checked by ape_mc_lstm_tc)
-    if (g->all_steps && (g->layer_begin != 0 || g->layer_end != 0)) return APE_ERR_UNSUPPORTED;
-    if (g->T > 40) return APE_ERR_UNSUPPORTED;                            // (with a state |c_t| <= |c_0| + t: the ex2 arguments are clamped)
-    if (!g->weights_tcx || !g->workspace) return APE_ERR_BAD_ARG;
-    const long long E = (long long)g->B * g->nF;
-    if (E == 0) return APE_OK;
-    if (g->ws_E != 0 && g->ws_E < E) return APE_ERR_BAD_ARG;
-    int dev = 0, sm_count = 0;
-    APE_CUDA_TRY(cudaGetDevice(&dev));
-    APE_CUDA_TRY(cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev));
-    if (sm_count > MAX_SMS) return APE_ERR_UNSUPPORTED;
-    if (g->reserve_sms < 0 || g->reserve_sms > sm_count - 2) return APE_ERR_BAD_ARG;
-    const int sm_big = sm_count - ((g->reserve_sms + 1) & ~1);
-    const long long rows = E * g->n_samples;
-    const int tiles0 = (int)((E + 255) / 256), tiles1 = (int)((rows + 255) / 256);
-    const bool all_steps = g->all_steps != 0;
-    const WsLayout wl = ws_layout(g->L, g->T, g->ws_E > 0 ? g->ws_E : E, g->n_samples, all_steps);
-    char* wsp = (char*)(((uintptr_t)g->workspace + 255) & ~(uintptr_t)255);
-    char* scratch = wsp;
-    wsp += 2 * wl.scratch;
-    uint4* u0_hi = (uint4*)(wsp + (size_t)(g->ws_parity & 1) * 2 * wl.u0);
-    uint4* u0_lo = (uint4*)((char*)u0_hi + wl.u0);
-    char* u1_base = wsp + 4 * wl.u0;
-    auto u1_hi = [&](int k) { return (uint4*)(u1_base + (size_t)k * 2 * wl.u1); };
-    auto u1_lo = [&](int k) { return (uint4*)(u1_base + (size_t)k * 2 * wl.u1 + wl.u1); };
-    const int l_begin = (g->layer_begin == 0 && g->layer_end == 0) ? 0 : g->layer_begin;
-    const int l_end = (g->layer_begin == 0 && g->layer_end == 0) ? g->L : g->layer_end;
-    if (l_begin < 0 || l_end > g->L || l_begin >= l_end) return APE_ERR_BAD_ARG;
-
-    cudaEvent_t ev[17] = {};
-    const bool prof = g->layer_ms != nullptr && g->L <= 16 && l_begin == 0 && l_end == g->L;
-    if (prof) for (int l = 0; l <= g->L; ++l) APE_CUDA_TRY(cudaEventCreate(&ev[l]));
-    if (prof) APE_CUDA_TRY(cudaEventRecord(ev[0], st));
-
-    const uint8_t* wl_ptr = (const uint8_t*)g->weights_tcx;
-    const uint8_t* wo16 = wl_ptr;
-    for (int l = 0; l < g->L; ++l) wo16 += layer_bytes(l, g->I);
-    const float scale = g->mask_mode == APE_MASK_NONE ? 1.0f : 1.0f / (1.0f - g->dropout_p);
-    for (int l = 0; l < l_end; ++l) {
-        const uint8_t* w_l = wl_ptr;
-        wl_ptr += layer_bytes(l, g->I);
-        if (l < l_begin) continue;
-        const bool last = l == g->L - 1;
-        tc::TcLayerArgs a{};
-        a.Ww = w_l;
-        a.T = g->T;
-        a.kgx = l == 0 ? ape_pack_kin_pad(0, g->I, H) / 8 : KG;
-        a.Kin = l == 0 ? g->I : H;
-        a.rpc = ROWS;
-        a.feat_ring = g->feat_ring; a.nF = g->nF; a.frame0 = g->frame0; a.stream_frames = g->stream_frames;
-        if (l == 0) {
-            a.in_mode = g->x_dense ? tc::IN_DENSE_F32 : tc::IN_WINDOW_F32;
-            a.in = g->x_dense ? (const void*)g->x_dense : (const void*)g->feat_ring_buf;
-            a.rows = (int)E; a.n = 1;
-            a.n_pair_tiles = tiles0;
-            a.mask_mode = APE_MASK_NONE;
-            a.out_units = u0_hi; a.out_units_lo = u0_lo;
-        } else {
-            a.in_mode = l == 1 ? tc::IN_SHARED_UNITS : tc::IN_UNITS;
-            a.in = l == 1 ? (const void*)u0_hi : (const void*)u1_hi((l - 2) & 1);
-            a.in_lo = l == 1 ? (const void*)u0_lo : (const void*)u1_lo((l - 2) & 1);
-            a.rows = (int)rows; a.n = g->n_samples;
-            a.n_pair_tiles = tiles1;
-            a.mask_mode = g->mask_mode;
-            // (all_steps: the last layer keeps its sequence for the per-step output layer)
-            a.out_units = (last && !all_steps) ? nullptr : u1_hi((l - 1) & 1);
-            a.out_units_lo = (last && !all_steps) ? nullptr : u1_lo((l - 1) & 1);
-        }
-        a.masks = g->masks; a.gap = l - 1; a.n_gaps = g->L - 1;
-        a.seed = g->philox_seed; a.stream_id0 = g->stream_id0;
-        a.rk = philox_round_keys(g->philox_seed);
-        a.keep_thr16 = keep_threshold16(g->dropout_p);
-        a.out_scale = last ? 1.0f : scale;
-        a.Wo = g->weights + ape_pack_out_offset(g->I, g->H, g->L);
-        a.bo = a.Wo + (size_t)g->O * g->H;
-        a.O = g->O;
-        a.Wo16 = wo16;
-        a.preds = (last && !all_steps) ? g->preds : nullptr;
-        a.pred_ring = g->pred_ring; a.n_out = g->n_samples;
-        a.cstate = (float*)(scratch + (l == 0 ? 0 : wl.scratch));
-        a.h0 = g->h0 ? g->h0 + (size_t)l * E * H : nullptr;   // [L][E][H]: with a state every layer has E rows (n_samples == 1)
-        a.c0 = g->c0 ? g->c0 + (size_t)l * E * H : nullptr;
-        a.timeline = (g->trace && g->trace_layer < 0) ? (long long*)g->trace + (size_t)l * MAX_SMS * 4 : nullptr;
-        const int rc = launch_layer(a, l == 0 ? sm_count : sm_big, st);
-        if (rc != APE_OK) return rc;
-        if (prof) APE_CUDA_TRY(cudaEventRecord(ev[l + 1], st));
-    }
-    if (all_steps) {                                           // output layer on every step, h = hi + lo against the fp32 W_o
-        const int rc = tc::launch_units_output(u1_hi((g->L - 2) & 1), u1_lo((g->L - 2) & 1), g->weights + ape_pack_out_offset(g->I, g->H, g->L),
-                                               g->preds, rows, g->T, H, g->O, st);
-        if (rc != APE_OK) return rc;
-    }
-    if (prof) {
-        APE_CUDA_TRY(cudaStreamSynchronize(st));
-        for (int l = 0; l < g->L; ++l) APE_CUDA_TRY(cudaEventElapsedTime(&g->layer_ms[l], ev[l], ev[l + 1]));
-        for (int l = 0; l <= g->L; ++l) cudaEventDestroy(ev[l]);
-    }
-    return APE_OK;
-}
+size_t wo16_bytes() { return (size_t)2 * OUT_BYTES; }
 
 }  // namespace tcxs
 }  // namespace ape
-
-extern "C" int ape_mc_lstm_tcxs_supported(int I, int H, int L, int O) {
-    return (ape::tcxs::supported(H, I, O) && L >= 2) ? 1 : 0;
-}
-extern "C" int ape_lstm_tcxs_blob_bytes(int I, int H, int L, int64_t* bytes) {
-    if (!bytes || !ape_mc_lstm_tcxs_supported(I, H, L, 1)) return APE_ERR_BAD_ARG;
-    *bytes = (int64_t)ape::tcxs::blob_bytes(I, L);
-    return APE_OK;
-}
-extern "C" int ape_mc_lstm_tcxs_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
-    if (!bytes || T < 1 || E < 0 || n_samples < 1) return APE_ERR_BAD_ARG;
-    if (!ape_mc_lstm_tcxs_supported(I, H, L, O)) return APE_ERR_UNSUPPORTED;
-    *bytes = ape::tcxs::workspace_bytes(L, T, E, n_samples, false);
-    return APE_OK;
-}
-// the same for a call with all_steps != 0 (the model API: the last layer's sequence is kept for the per-step output layer)
-extern "C" int ape_mc_lstm_tcxs_workspace_bytes_all_steps(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
-    if (!bytes || T < 1 || E < 0 || n_samples < 1) return APE_ERR_BAD_ARG;
-    if (!ape_mc_lstm_tcxs_supported(I, H, L, O)) return APE_ERR_UNSUPPORTED;
-    *bytes = ape::tcxs::workspace_bytes(L, T, E, n_samples, true);
-    return APE_OK;
-}
