@@ -27,7 +27,7 @@ SYMBOLS = (
     "ape_mc_lstm_tc_workspace_bytes", "ape_mc_lstm_tc_workspace_bytes_all_steps", "ape_mc_lstm_tc", "ape_mc_lstm_tc_launch_count", "ape_mc_lstm_tcx_supported", "ape_lstm_tcx_blob_bytes", "ape_mc_lstm_tcx_workspace_bytes", "ape_mc_lstm_tcx_workspace_bytes_all_steps", "ape_mc_lstm_tcxs_supported", "ape_lstm_tcxs_blob_bytes", "ape_mc_lstm_tcxs_workspace_bytes",
     "ape_mc_lstm_tcxs_workspace_bytes_all_steps", "ape_philox_masks", "ape_ff_blob_floats", "ape_mc_ff", "ape_dense_act", "ape_fk_reduce", "ape_msg_from_est",
     "ape_pipeline_create", "ape_pipeline_destroy", "ape_pipeline_submit", "ape_pipeline_wait", "ape_pipeline_query", "ape_pipeline_sync",
-    "ape_pipeline_fence",
+    "ape_pipeline_fence", "ape_pipeline_stream",
     "ape_selfcheck_philox", "ape_selfcheck_keep8", "ape_selfcheck_features", "ape_selfcheck_row_pose", "ape_selfcheck_tcs_schedule",
     "ape_selftest_umma", "ape_selftest_ffma_peak",
 )
@@ -183,6 +183,8 @@ def load():
     lib.ape_pipeline_sync.argtypes = [vp]
     lib.ape_pipeline_fence.restype = i32
     lib.ape_pipeline_fence.argtypes = [vp, vp]
+    lib.ape_pipeline_stream.restype = i32
+    lib.ape_pipeline_stream.argtypes = [vp, i32, C.POINTER(vp)]
     # host self-check hooks: used by tests/ only
     lib.ape_selfcheck_philox.restype = i32
     lib.ape_selfcheck_philox.argtypes = [C.POINTER(u32), C.POINTER(u32), C.POINTER(u32)]

@@ -10,6 +10,11 @@
 // estimate/batched.py drives the same sequence call by call through torch streams and events (it still does, for profiling legs,
 // injected masks and the CUDA-graph path); at 0.3 ms of device time per call the ~40 Python-level stream / event operations of one
 // submit() had become what the GPU waited for.  This object owns nothing but CUDA streams and events: every buffer is the caller's.
+//
+// Nothing orders the last LSTM layer of call k behind stage 3 of call k-1 (the other lane) as long as every stream's frames move
+// forward: the prediction ring holds two calls' frames plus the smoothing window, so call k writes no slot call k-1 still reads.
+// A stream's counter may go back (a restarted stream, a shared counter reset with calls in flight), or jump; when call k then
+// writes a slot of call k-1's smoothing window (pred_window_alias), its layers >= 1 wait for call k-1's stage 3.
 #include <cstring>
 #include <new>
 
@@ -18,6 +23,15 @@
 
 namespace {
 constexpr int MAX_SLOTS = APE_PIPELINE_MAX_SLOTS;
+
+// Do frames f .. f + nF - 1 of a stream share a slot of a ring of `ring` frames with the smoothing windows of a call of nF1 frames
+// from frame f1 (frames f1 - smooth + 1 .. f1 + nF1 - 1, those before 0 read as frame 0)?  (estimate/batched.py: the same rule)
+bool pred_window_alias(long long f, int nF, long long f1, int nF1, int smooth, int ring) {
+    const long long lo = f1 - smooth + 1 > 0 ? f1 - smooth + 1 : 0;           // oldest frame read
+    long long o = (f - lo) % ring;                             // where the written frames start, counted from its slot
+    if (o < 0) o += ring;
+    return o < f1 + nF1 - lo || o + nF > ring;
+}
 }
 
 struct ape_pipeline {
@@ -28,6 +42,10 @@ struct ape_pipeline {
     bool done_valid[4], lstm_done_valid, slot_busy[MAX_SLOTS];
     int last_lane;
     long long calls, submits;
+    // the previous call, while its stage 3 may still be running: its frames (shared frame0, or per-stream counters in
+    // frames_host[prev_slot], which the next n_slots - 1 calls leave alone)
+    bool prev_valid, prev_sf;
+    int prev_nF, prev_frame0, prev_slot;
 };
 
 #define PIPE_TRY(expr) do { int _rc = (expr); if (_rc != APE_OK) return _rc; } while (0)
@@ -63,6 +81,7 @@ extern "C" int ape_pipeline_create(const ape_pipeline_desc* d, ape_pipeline** ou
     p->lstm_done_valid = false;
     p->last_lane = 0;
     p->calls = p->submits = 0;
+    p->prev_valid = false;
     *out = p;
     return APE_OK;
 }
@@ -87,6 +106,15 @@ extern "C" int ape_pipeline_sync(ape_pipeline* p) {
     APE_CUDA_TRY(cudaStreamSynchronize(p->lane[1]));
     APE_CUDA_TRY(cudaStreamSynchronize(p->copy));
     for (int i = 0; i < MAX_SLOTS; ++i) p->slot_busy[i] = false;
+    p->prev_valid = false;                                     // (everything has drained: the next call follows nothing)
+    return APE_OK;
+}
+
+// the pipeline's streams, for a caller that orders its own work against one of them: 0 side, 1 lane 0, 2 lane 1, 3 copy
+extern "C" int ape_pipeline_stream(ape_pipeline* p, int which, void** stream) {
+    if (!p || !stream || which < 0 || which > 3) return APE_ERR_BAD_ARG;
+    const cudaStream_t s[4] = {p->side, p->lane[0], p->lane[1], p->copy};
+    *stream = (void*)s[which];
     return APE_OK;
 }
 
@@ -167,6 +195,21 @@ extern "C" int ape_pipeline_submit(ape_pipeline* p, const float* rows_host, cons
     APE_CUDA_TRY(cudaEventRecord(p->ev0[bufset], side));
 
     APE_CUDA_TRY(cudaStreamWaitEvent(lane, p->ev0[bufset], 0));
+    // a stream whose counter went back (or jumped) may write a prediction slot that stage 3 of call k-1 (the other lane) still reads;
+    // call k-2 ran on this lane, so only call k-1 needs the check.  A change between the shared and the per-stream counters fences too.
+    if (p->prev_valid) {
+        const int ring = d.lstm.pred_ring;
+        bool alias = p->prev_sf != (sf_dev != nullptr);
+        if (!alias && !sf_dev) {
+            alias = pred_window_alias(frame0, nF, p->prev_frame0, p->prev_nF, d.smooth, ring);
+        } else if (!alias) {
+            const int32_t* prev = d.frames_host[p->prev_slot];
+            for (int b = 0; b < d.B && !alias; ++b)
+                alias = prev[b] >= 0 && stream_frames_host[b] >= 0 &&
+                        pred_window_alias(stream_frames_host[b], nF, prev[b], p->prev_nF, d.smooth, ring);
+        }
+        if (alias) APE_CUDA_TRY(cudaStreamWaitEvent(lane, p->done[(k - 1) & 3], 0));
+    }
     a.layer_begin = 1; a.layer_end = a.L;
     PIPE_TRY(ape_mc_lstm_tc(&a, lane));
     // the smoothing window of stage 3 reaches into the previous call's predictions (written on the other lane)
@@ -196,6 +239,9 @@ extern "C" int ape_pipeline_submit(ape_pipeline* p, const float* rows_host, cons
         APE_CUDA_TRY(cudaEventRecord(p->slot_ev[slot], p->copy));
         p->slot_busy[slot] = true;
     }
+    p->prev_valid = true;
+    p->prev_sf = sf_dev != nullptr;
+    p->prev_nF = nF; p->prev_frame0 = frame0; p->prev_slot = slot;
     p->calls += 1;
     p->submits += 1;
     *slot_out = slot;

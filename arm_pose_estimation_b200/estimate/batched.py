@@ -70,6 +70,16 @@ def ring_slots(n_frames_per_call, history):
     return max(1, n_frames_per_call) + max(1, history) - 1
 
 
+def pred_window_alias(f, nF, f1, nF1, smooth, ring):
+    """Do frames ``f .. f + nF - 1`` of a stream share a slot of a prediction ring of ``ring`` frames with the smoothing windows of
+    a call of ``nF1`` frames from frame ``f1`` (frames ``f1 - smooth + 1 .. f1 + nF1 - 1``, those before 0 read as frame 0)?
+    Element-wise over arrays; the cross-call pipeline's ordering rule (csrc/ape_pipeline.cu has the same)."""
+    f1 = np.asarray(f1, np.int64)
+    lo = np.maximum(f1 - smooth + 1, 0)                   # oldest frame read
+    o = (np.asarray(f, np.int64) - lo) % ring             # where the written frames start, counted from its slot
+    return (o < f1 + nF1 - lo) | (o + nF > ring)
+
+
 @dataclass
 class EstimateBatch:
     """Results of one ``BatchedEstimator.step``; tensors live on the estimator's device until ``.host()``."""
@@ -255,6 +265,7 @@ class BatchedEstimator:
             self.lane_ws = [self.workspace, torch.empty_like(self.workspace)] if self.lanes else None
             self.l1_done = [None] * 4             # completion of the last call that used buffer set (call & 3)
             self.lstm_done = None             # last LSTM layer of the previous call (its predictions feed this call's smoothing window)
+            self._prev_call = None            # (stage-3 event, frames, nF) of the previous pipelined call: frame0, host counters or None
             # The same pipeline as ONE C call per batch (csrc/ape_pipeline.cu: ape_pipeline_submit): used for every call that needs
             # nothing call-specific from Python (no injected masks, no profiling / trace leg, no caller-owned frame counters).  The
             # Python-level pipeline below remains for those, and as the A/B switch (native_pipeline=False | APE_NATIVE_PIPELINE=0).
@@ -462,7 +473,11 @@ class BatchedEstimator:
         promises that ``raw`` is already materialised (not pending on the current stream), which lets the pipelined path
         start stage 1 + layer 0 of this call under the previous call's kernels.  ``stream_frames``: optional device int32
         tensor ``[B]`` of per-stream absolute frame numbers for streams that do not advance in lock-step (a negative entry
-        skips the stream in this call: its rings and outputs stay untouched); the shared frame counter is then not used."""
+        skips the stream in this call: its rings and outputs stay untouched); the shared frame counter is then not used.
+        With the lanes, a call whose frames go back (a restarted stream, ``reset()`` with calls in flight) or jump orders its LSTM
+        layers >= 1 behind the previous call's stage 3, which may still read the prediction slots this call writes; counters that
+        exist only on the device (``stream_frames`` without a host copy) cannot be inspected without a sync, so such a call is
+        always ordered so."""
         nF = int(raw.shape[1]) if n_frames is None else int(n_frames)
         self._g_stale = self._g_stale or not _plain
         if raw.shape[0] != self.B or nF > self.nF_max or raw.shape[2] != self.ncols or not raw.is_contiguous():
@@ -537,6 +552,9 @@ class BatchedEstimator:
             lane.wait_event(ev0)
             if self.copy_done[self.out_slot] is not None:
                 lane.wait_event(self.copy_done[self.out_slot])   # this output buffer has been read back (submit(), call k-2)
+            frames = frame0 if sf is None else (None if _frames_from is None else _frames_from.numpy().copy())
+            if self.lanes and self._prev_call is not None and self._writes_prev_window(frames, nF):
+                lane.wait_event(self._prev_call[0])      # the previous call's stage 3 (the other lane) has read its window
             with torch.cuda.stream(lane):
                 lp = C_void(lane.cuda_stream)
                 a.layer_begin, a.layer_end = 1, self.L
@@ -549,6 +567,7 @@ class BatchedEstimator:
                 done = torch.cuda.Event()
                 done.record(lane)
             self.l1_done[bufset] = done
+            self._prev_call = (done, frames, nF)
             if self.lanes:
                 main.wait_event(done)                    # the caller's stream sees the results, as without the lanes
         else:
@@ -566,6 +585,17 @@ class BatchedEstimator:
                             self._view(self.status, nF), self.frame)
         self.frame += nF
         return out
+
+    def _writes_prev_window(self, frames, nF):
+        """Would a call of ``nF`` frames from ``frames`` (the shared frame0, host counters [B], or None: device counters only) write a
+        prediction slot that the previous pipelined call's smoothing window reads?  A change of counter mode counts as yes."""
+        _, prev, prev_nF = self._prev_call
+        if frames is None or prev is None or isinstance(frames, int) != isinstance(prev, int):
+            return True
+        if isinstance(frames, int):
+            return bool(pred_window_alias(frames, nF, prev, prev_nF, self.smooth, self.pred_ring))
+        both = (frames >= 0) & (prev >= 0)                # a stream the previous call skipped has no window there
+        return bool(pred_window_alias(frames[both], nF, prev[both], prev_nF, self.smooth, self.pred_ring).any())
 
     def _view(self, buf, nF):
         """The kernels pack a call's E = B * nF estimates densely: view the front of a [B, nF_max, ...] buffer."""

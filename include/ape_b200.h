@@ -301,7 +301,9 @@ int ape_pipeline_destroy(ape_pipeline* p);
  * One call of B x nF estimates starting at absolute frame frame0 (or at stream_frames_host[b] per stream, host int32 [B], negative:
  * the stream sits this call out).  Exactly one of rows_host (any host memory, copied into the slot's pinned staging here) and
  * rows_dev (device rows, read in place) is non-null.  *slot = the result slot used (out_dev / out_host index); a slot is
- * reused after n_slots calls, after its previous results have landed.
+ * reused after n_slots calls, after its previous results have landed.  A stream's counter may go back (a restarted stream, frame0
+ * back to 0 after a reset) or jump while earlier calls are in flight: when this call would write a prediction-ring slot that the
+ * previous call's smoothing window reads, its LSTM layers >= 1 wait for the previous call's stage 3.
  */
 int ape_pipeline_submit(ape_pipeline* p, const float* rows_host, const float* rows_dev, int nF, int frame0,
                         const int32_t* stream_frames_host, int flags, void* caller_stream, int* slot);
@@ -309,6 +311,9 @@ int ape_pipeline_wait(ape_pipeline* p, int slot);              /* host-blocking:
 int ape_pipeline_query(ape_pipeline* p, int slot, int* landed);/* non-blocking form */
 int ape_pipeline_sync(ape_pipeline* p);                        /* host-blocking drain of all four streams */
 int ape_pipeline_fence(ape_pipeline* p, void* stream);         /* later submits wait for what `stream` holds now */
+/* The pipeline's CUDA streams (which: 0 side, 1 lane 0, 2 lane 1, 3 copy) as cudaStream_t, for a caller that orders its own work
+   against one of them; the pipeline keeps owning them.  APE_ERR_BAD_ARG for a null pointer or another `which`. */
+int ape_pipeline_stream(ape_pipeline* p, int which, void** stream);
 
 /* ---- host self-check hooks (tests only; one row per call, never used by the product path) ------ */
 /* The __host__ __device__ row math of the kernels, compiled for the host so a CPU-only box can pin it. */
