@@ -738,7 +738,7 @@ extern "C" int ape_mc_lstm_tc_launch_count(const ape_lstm_args* g, int* launches
     const long long rows = (long long)g->B * g->nF * g->n_samples;
     const int l_begin = (g->layer_begin == 0 && g->layer_end == 0) ? 0 : g->layer_begin;
     const int l_end = (g->layer_begin == 0 && g->layer_end == 0) ? g->L : g->layer_end;
-    if (g->tc_flags == 4) { *launches = 1; return APE_OK; }
+    if (g->tc_flags == 4 || g->tc_flags == 5) { *launches = 1; return APE_OK; }
     const bool pair_ok = tc_pairs_layers(g, (rows + 255) / 256, sm_count);
     int n = 0;
     for (int l = l_begin; l < l_end; l += layers_in_launch(pair_ok, l, l_end)) ++n;
@@ -746,10 +746,35 @@ extern "C" int ape_mc_lstm_tc_launch_count(const ape_lstm_args* g, int* launches
     return APE_OK;
 }
 
+// Workspace of the split-precision small-batch kernel (tc_flags == 5): the exchange buffer and layer sequences (hi and lo) of one
+// cluster per 128 rows of the largest call
+extern "C" int ape_mc_lstm_tcxl_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
+    if (!bytes || T < 1 || E < 0 || n_samples < 1) return APE_ERR_BAD_ARG;
+    if (!ape::tcxl::supported(H, I, L, T, O, E, n_samples)) return APE_ERR_UNSUPPORTED;
+    *bytes = ape::tcxl::workspace_bytes(T, (long long)E * n_samples);
+    return APE_OK;
+}
+
+// tc_flags == 5: every layer of a call of <= 8192 rows of a split-precision H = 128 model in ONE launch (csrc/ape_lstm_tcxl.cu).  Every
+// refusal comes before the first CUDA call.
+static int tcxl_call(const ape_lstm_args* g, cudaStream_t st) {
+    const long long E = (long long)g->B * g->nF;
+    if (g->h0 || g->all_steps || g->layer_begin != 0 || g->layer_end != 0) return APE_ERR_UNSUPPORTED;
+    if (!ape::tcxl::supported(g->H, g->I, g->L, g->T, g->O, E, g->n_samples)) return APE_ERR_UNSUPPORTED;
+    if (!g->weights_tcx || !g->workspace || (g->ws_E != 0 && g->ws_E < E)) return APE_ERR_BAD_ARG;
+    if (E == 0) return APE_OK;
+    ape::LayerTimer timer(g->layer_ms, g->L, st);              // the one launch is reported as layer 0's time
+    int rc = timer.start();
+    if (rc == APE_OK) rc = ape::tcxl::run(g, (const uint8_t*)g->weights_tcx, g->workspace, st);
+    if (rc == APE_OK) rc = timer.mark(g->L);
+    return rc == APE_OK ? timer.finish() : rc;
+}
+
 extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
     using namespace ape;
     int rc = check_lstm_args(g);                               // (h0 / c0: both or neither, and n_samples == 1)
     if (rc != APE_OK) return rc;
+    if (g->tc_flags == 5) return tcxl_call(g, (cudaStream_t)stream);
     // an initial state runs on the one-layer kernels (tc_flags 0 and 1) and on the H = 256 split-precision kernel; the wavefront,
     // small-batch and H = 128 split-precision kernels take none
     if (g->h0 && (g->tc_flags == 2 || (g->tc_flags == 3 && g->H != 256) || g->tc_flags == 4)) return APE_ERR_UNSUPPORTED;
@@ -785,7 +810,7 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
     const int l_begin = (g->layer_begin == 0 && g->layer_end == 0) ? 0 : g->layer_begin;
     const int l_end = (g->layer_begin == 0 && g->layer_end == 0) ? g->L : g->layer_end;
     if (l_begin < 0 || l_end > g->L || l_begin >= l_end) return APE_ERR_BAD_ARG;
-    if (g->tc_flags < 0 || g->tc_flags > 4) return APE_ERR_BAD_ARG;
+    if (g->tc_flags < 0 || g->tc_flags > 5) return APE_ERR_BAD_ARG;
     if (g->tc_flags == 4) {
         // small-batch kernel: every layer of a call of <= 128 rows in ONE launch of one 8-CTA cluster (csrc/ape_lstm_tcl.cu)
         if (l_begin != 0 || l_end != g->L || g->L > 4) return APE_ERR_UNSUPPORTED;

@@ -132,7 +132,7 @@ class BatchedEstimator:
                  smooth=1, dropout=0.2, bonemap=None, frames_per_call=1, emit_samples=True, normalize=True,
                  mask_mode=N.MASK_PHILOX, philox_seed=0, first_stream=0, device=None,
                  lstm_variant="auto", tc_min_rows=1, tc_tolerance_m=5e-5, pipeline=True, lanes=True, tc_flags=None,
-                 native_pipeline=None, small_batch_kernel=True):
+                 native_pipeline=None, small_batch_kernel=True, split_small_batch_kernel=False):
         if not torch.cuda.is_available():
             raise RuntimeError("BatchedEstimator needs a CUDA device (sm_100a); there is no CPU fallback")
         self.lib = N.load()
@@ -244,6 +244,15 @@ class BatchedEstimator:
                                 and self.L <= 4 and self.H in (128, 256) and self.T <= 40 and B * nF * self.n <= self.SMALL_BATCH_ROWS)
             if self.small_batch:
                 self.tc_flags = 4
+            # The same for a model on the split-precision kernels (H = 128: csrc/ape_lstm_tcxl.cu, tc_flags = 5): the layer kernels' arithmetic
+            # and MMA order per accumulator, so the results are bit-identical to them (tests/test_gpu_tcxl.py).  Off by default; the
+            # single-stream estimator classes (estimator.py) turn it on.
+            if (split_small_batch_kernel and self.tc_split and self.H == 128 and self.L <= 4 and self.T <= 40
+                    and B * nF * self.n <= self.SMALL_BATCH_ROWS):
+                self.small_batch, self.tc_flags = True, 5
+                ws_xl = N.tcxl_workspace_bytes(self.I, self.H, self.L, self.T, self.O, B * nF, self.n)
+                if ws_xl > self.workspace.numel():
+                    self.workspace = torch.empty(ws_xl, dtype=torch.uint8, device=dev)
             # cross-call software pipeline (tensor-core path), two levels:
             #  * stage 1 + LSTM layer 0 of call k+1 (a few dozen CTAs) run on a side stream under call k's big layer kernels;
             #    layer 0's output is double-buffered by call parity;

@@ -291,4 +291,4 @@ class _NNEstimator(Estimator):
             kind=self._kind, layout=self._layout, state=self._nn_model.state_dict(), seq_len=self._sequence_len,
             y_targets=self._y_targets, stats=stats, n_streams=1, mc_samples=self._mc_samples, smooth=self._smooth,
             dropout=self._nn_model.dropout, bonemap=self._bonemap, frames_per_call=1, emit_samples=True,
-            normalize=self._normalize, mask_mode=mask_mode, philox_seed=self._philox_seed)
+            normalize=self._normalize, mask_mode=mask_mode, philox_seed=self._philox_seed, split_small_batch_kernel=True)

@@ -146,7 +146,10 @@ typedef struct ape_lstm_args {
        csrc/ape_lstm_tcx.cu, H = 256: csrc/ape_lstm_tcxs.cu; all_steps != 0 needs the _all_steps workspace query),
        4 = the SMALL-BATCH kernel (csrc/ape_lstm_tcl.cu: B * nF * n_samples <= 8192 rows, L <= 4: all layers in one launch, one
        8-CTA cluster per 128 rows with the hidden units split across it - the real-time case of one to a few dozen streams; same
-       arithmetic as 0..2; no initial state) */
+       arithmetic as 0..2; no initial state),
+       5 = the SPLIT-PRECISION SMALL-BATCH kernel (csrc/ape_lstm_tcxl.cu: the arithmetic of 3 at H = 128 - bit-identical results - in
+       the launch structure of 4: B * nF * n_samples <= 8192 rows, 2 <= L <= 4, T <= 40, O <= 16; needs weights_tcx and a workspace of
+       ape_mc_lstm_tcxl_workspace_bytes(); no initial state, no all_steps, no layer range: APE_ERR_UNSUPPORTED) */
     int tc_flags;
     /* optional initial state (h_0, c_0) of torch.nn.LSTM(x, hs) (nn_models.py:180-189): [L][E][H] float32 each, both or neither
        (APE_ERR_BAD_ARG); needs n_samples == 1 (APE_ERR_UNSUPPORTED; a caller with per-sample states passes the samples as estimates).
@@ -195,7 +198,10 @@ int ape_mc_lstm_tcxs_supported(int I, int H, int L, int O);
 int ape_lstm_tcxs_blob_bytes(int I, int H, int L, int64_t* bytes);
 int ape_mc_lstm_tcxs_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes);
 int ape_mc_lstm_tcxs_workspace_bytes_all_steps(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes);
-/* number of kernels ape_mc_lstm_tc launches for these arguments (layer pairs of an H = 128 model count once) */
+/* workspace of a call on the split-precision small-batch kernel (tc_flags == 5: H = 128, 2 <= L <= 4, T <= 40, O <= 16,
+   E * n_samples <= 8192): the h_t exchange buffer and the layer sequences, hi and lo, of one cluster per 128 rows */
+int ape_mc_lstm_tcxl_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes);
+/* number of kernels ape_mc_lstm_tc launches for these arguments (layer pairs of an H = 128 model count once; tc_flags 4 and 5: 1) */
 int ape_mc_lstm_tc_launch_count(const ape_lstm_args* args, int* launches);
 /*
  * The Bernoulli keep-masks APE_MASK_PHILOX draws, written out as bytes in the APE_MASK_INJECTED layout
