@@ -25,7 +25,8 @@ SYMBOLS = (
     "ape_abi_version", "ape_last_cuda_error", "ape_device_info", "ape_lstm_blob_floats", "ape_features", "ape_features_push",
     "ape_mc_lstm_workspace_bytes", "ape_mc_lstm_fma", "ape_mc_lstm_tc_supported", "ape_lstm_tc_blob_bytes",
     "ape_mc_lstm_tc_workspace_bytes", "ape_mc_lstm_tc_workspace_bytes_all_steps", "ape_mc_lstm_tc", "ape_mc_lstm_tc_launch_count", "ape_mc_lstm_tcx_supported", "ape_lstm_tcx_blob_bytes", "ape_mc_lstm_tcx_workspace_bytes", "ape_mc_lstm_tcx_workspace_bytes_all_steps", "ape_mc_lstm_tcxs_supported", "ape_lstm_tcxs_blob_bytes", "ape_mc_lstm_tcxs_workspace_bytes",
-    "ape_mc_lstm_tcxs_workspace_bytes_all_steps", "ape_mc_lstm_tcxl_workspace_bytes", "ape_philox_masks", "ape_ff_blob_floats", "ape_mc_ff", "ape_dense_act", "ape_fk_reduce", "ape_msg_from_est",
+    "ape_mc_lstm_tcxs_workspace_bytes_all_steps", "ape_mc_lstm_tcxl_workspace_bytes", "ape_mc_lstm_tcxsl", "ape_mc_lstm_tcxsl_workspace_bytes",
+    "ape_mc_lstm_tcxsl_max_active_clusters", "ape_philox_masks", "ape_ff_blob_floats", "ape_mc_ff", "ape_dense_act", "ape_fk_reduce", "ape_msg_from_est",
     "ape_pipeline_create", "ape_pipeline_destroy", "ape_pipeline_submit", "ape_pipeline_wait", "ape_pipeline_query", "ape_pipeline_sync",
     "ape_pipeline_fence", "ape_pipeline_stream",
     "ape_selfcheck_philox", "ape_selfcheck_keep8", "ape_selfcheck_features", "ape_selfcheck_row_pose", "ape_selfcheck_tcs_schedule",
@@ -159,6 +160,12 @@ def load():
     lib.ape_mc_lstm_tcxs_workspace_bytes_all_steps.argtypes = [i32, i32, i32, i32, i32, i32, i32, C.POINTER(u64)]
     lib.ape_mc_lstm_tcxl_workspace_bytes.restype = i32
     lib.ape_mc_lstm_tcxl_workspace_bytes.argtypes = [i32, i32, i32, i32, i32, i32, i32, C.POINTER(u64)]
+    lib.ape_mc_lstm_tcxsl.restype = i32
+    lib.ape_mc_lstm_tcxsl.argtypes = [C.POINTER(LstmArgs), vp]
+    lib.ape_mc_lstm_tcxsl_workspace_bytes.restype = i32
+    lib.ape_mc_lstm_tcxsl_workspace_bytes.argtypes = [i32, i32, i32, i32, i32, i32, i32, C.POINTER(u64)]
+    lib.ape_mc_lstm_tcxsl_max_active_clusters.restype = i32
+    lib.ape_mc_lstm_tcxsl_max_active_clusters.argtypes = [C.POINTER(i32)]
     lib.ape_philox_masks.restype = i32
     lib.ape_philox_masks.argtypes = [u64, u32, i32, i32, i32, i32, i32, i32, i32, f32, vp, vp]
     lib.ape_ff_blob_floats.restype = i32
@@ -306,6 +313,21 @@ def tcxl_workspace_bytes(I, H, L, T, O, E, n):
     """Workspace of a call on the split-precision small-batch kernel (tc_flags = 5: H = 128, L <= 4, T <= 40, E * n <= 8192 rows)."""
     out = C.c_uint64(0)
     check(load().ape_mc_lstm_tcxl_workspace_bytes(I, H, L, T, O, E, n, C.byref(out)), "ape_mc_lstm_tcxl_workspace_bytes")
+    return out.value
+
+
+def tcxsl_workspace_bytes(I, H, L, T, O, E, n):
+    """Workspace of a call on the H = 256 split-precision small-batch kernel (ape_mc_lstm_tcxsl: L <= 4, T <= 40, O <= 32,
+    E * n <= 8192 rows)."""
+    out = C.c_uint64(0)
+    check(load().ape_mc_lstm_tcxsl_workspace_bytes(I, H, L, T, O, E, n, C.byref(out)), "ape_mc_lstm_tcxsl_workspace_bytes")
+    return out.value
+
+
+def tcxsl_max_active_clusters():
+    """16-CTA clusters of the H = 256 split-precision small-batch kernel the current device holds at once (0: it cannot run there)."""
+    out = C.c_int(0)
+    check(load().ape_mc_lstm_tcxsl_max_active_clusters(C.byref(out)), "ape_mc_lstm_tcxsl_max_active_clusters")
     return out.value
 
 

@@ -920,3 +920,42 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
     }
     return rc == APE_OK ? timer.finish() : rc;
 }
+
+// Workspace of the H = 256 split-precision small-batch kernel (ape_mc_lstm_tcxsl): the exchange buffer and layer sequences (hi and lo)
+// of one 16-CTA cluster per 128 rows of the largest call
+extern "C" int ape_mc_lstm_tcxsl_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
+    if (!bytes || T < 1 || E < 0 || n_samples < 1) return APE_ERR_BAD_ARG;
+    if (!ape::tcxsl::supported(H, I, L, T, O, E, n_samples)) return APE_ERR_UNSUPPORTED;
+    *bytes = ape::tcxsl::workspace_bytes(T, (long long)E * n_samples);
+    return APE_OK;
+}
+
+extern "C" int ape_mc_lstm_tcxsl_max_active_clusters(int* clusters) {
+    if (!clusters) return APE_ERR_BAD_ARG;
+    *clusters = 0;
+    return ape::tcxsl::max_active_clusters(clusters);
+}
+
+// Every layer of a call of <= 8192 rows of a split-precision H = 256 model in ONE launch (csrc/ape_lstm_tcxsl.cu), tc_flags == 5.
+// Every refusal comes before the first CUDA call; then a device that cannot hold one 16-CTA cluster of the kernel refuses the call.
+extern "C" int ape_mc_lstm_tcxsl(const ape_lstm_args* g, void* stream) {
+    using namespace ape;
+    int rc = check_lstm_args(g);
+    if (rc != APE_OK) return rc;
+    if (g->tc_flags != 5) return APE_ERR_BAD_ARG;
+    const long long E = (long long)g->B * g->nF;
+    if (g->h0 || g->all_steps || g->layer_begin != 0 || g->layer_end != 0) return APE_ERR_UNSUPPORTED;
+    if (!tcxsl::supported(g->H, g->I, g->L, g->T, g->O, E, g->n_samples)) return APE_ERR_UNSUPPORTED;
+    if (!g->weights_tcx || !g->workspace || (g->ws_E != 0 && g->ws_E < E)) return APE_ERR_BAD_ARG;
+    if (E == 0) return APE_OK;
+    int clusters = 0;
+    rc = tcxsl::max_active_clusters(&clusters);
+    if (rc != APE_OK) return rc;
+    if (clusters < 1) return APE_ERR_UNSUPPORTED;
+    cudaStream_t st = (cudaStream_t)stream;
+    LayerTimer timer(g->layer_ms, g->L, st);                   // the one launch is reported as layer 0's time
+    rc = timer.start();
+    if (rc == APE_OK) rc = tcxsl::run(g, (const uint8_t*)g->weights_tcx, g->workspace, st);
+    if (rc == APE_OK) rc = timer.mark(g->L);
+    return rc == APE_OK ? timer.finish() : rc;
+}

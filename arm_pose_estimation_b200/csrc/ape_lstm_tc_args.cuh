@@ -2,8 +2,8 @@
 // the per-layer argument block, the input modes, the transcendental helpers of the cell update, and each kernel's host entry
 // points - ape_lstm_tc.cu (gate weights resident in shared memory, H <= 128), ape_lstm_tcs.cu (gate weights streamed from L2
 // through a TMA ring, H = 256), ape_lstm_tcw.cu (two layers per launch, H = 128), ape_lstm_tcx.cu / ape_lstm_tcxs.cu (split
-// precision, H = 128 / 256), ape_lstm_tcl.cu (all layers of a small call in one launch) and ape_lstm_tcxl.cu (the same at split
-// precision, H = 128).
+// precision, H = 128 / 256), ape_lstm_tcl.cu (all layers of a small call in one launch) and ape_lstm_tcxl.cu / ape_lstm_tcxsl.cu (the
+// same at split precision, H = 128 / 256).
 #pragma once
 #include "ape_f32x2.cuh"
 #include "ape_common.cuh"
@@ -186,4 +186,13 @@ bool supported(int H, int I, int L, int T, int O, long long E, int n);
 size_t workspace_bytes(int T, long long rows);             // rows = E * n_samples of the largest call (one cluster per 128 rows)
 int run(const ape_lstm_args* g, const uint8_t* blob, void* workspace, cudaStream_t st);
 }  // namespace tcxl
+
+namespace tcxsl {
+// split-precision small-batch kernel for H = 256 (ape_lstm_tcxsl.cu): all layers of a call in one launch, one 16-CTA cluster per
+// 128 rows, the arithmetic of tcxs on the tcx blob
+bool supported(int H, int I, int L, int T, int O, long long E, int n);
+size_t workspace_bytes(int T, long long rows);             // rows = E * n_samples of the largest call (one cluster per 128 rows)
+int max_active_clusters(int* clusters);                    // 16-CTA clusters of this launch the current device holds at once
+int run(const ape_lstm_args* g, const uint8_t* blob, void* workspace, cudaStream_t st);
+}  // namespace tcxsl
 }  // namespace ape

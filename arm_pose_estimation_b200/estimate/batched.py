@@ -125,6 +125,11 @@ class _GraphCall:
 class BatchedEstimator:
     # largest call (streams x frames x MC samples) that runs on the cluster kernel (one 8-CTA cluster per 128 rows, csrc/ape_lstm_tcl.cu)
     SMALL_BATCH_ROWS = int(os.environ.get("APE_SMALL_BATCH_ROWS", "2048"))
+    # largest call of an H = 256 model on the split-precision small-batch kernel (16-CTA clusters, csrc/ape_lstm_tcxsl.cu).  A B200 holds
+    # 7 of its clusters at once, so calls above 896 rows run in waves; measured per single call (n = 128, B200 at 1000 W,
+    # profiles/split_small256_bench.json) it still beats the split layer kernels at 3072 rows (pocket 0.334 / 0.349 ms, watch-only
+    # 0.418 / 0.452) and loses at 4096 (0.408 / 0.352, 0.512 / 0.455): the crossover lies above SMALL_BATCH_ROWS, which stays the bound
+    SPLIT256_SMALL_BATCH_ROWS = min(SMALL_BATCH_ROWS, 2048)
     N_SLOTS = int(os.environ.get("APE_N_SLOTS", "8"))      # staging / result buffer sets: up to N_SLOTS - 1 submitted calls may be outstanding while the next is staged
                      # (measured end to end, uarm 1024 x 100: 3 outstanding 0.413 ms/step, 5 outstanding 0.392, 7 outstanding 0.391)
 
@@ -244,13 +249,16 @@ class BatchedEstimator:
                                 and self.L <= 4 and self.H in (128, 256) and self.T <= 40 and B * nF * self.n <= self.SMALL_BATCH_ROWS)
             if self.small_batch:
                 self.tc_flags = 4
-            # The same for a model on the split-precision kernels (H = 128: csrc/ape_lstm_tcxl.cu, tc_flags = 5): the layer kernels' arithmetic
-            # and MMA order per accumulator, so the results are bit-identical to them (tests/test_gpu_tcxl.py).  Off by default; the
-            # single-stream estimator classes (estimator.py) turn it on.
-            if (split_small_batch_kernel and self.tc_split and self.H == 128 and self.L <= 4 and self.T <= 40
-                    and B * nF * self.n <= self.SMALL_BATCH_ROWS):
+            # The same for a model on the split-precision kernels (tc_flags = 5; H = 128: csrc/ape_lstm_tcxl.cu, H = 256:
+            # csrc/ape_lstm_tcxsl.cu, its own entry point, on a device that holds one of its 16-CTA clusters): the layer kernels'
+            # arithmetic and MMA order per accumulator, so the results are bit-identical to them (tests/test_gpu_tcxl.py,
+            # tests/test_gpu_tcxsl.py).  Off by default; the single-stream estimator classes (estimator.py) turn it on.
+            if (split_small_batch_kernel and self.tc_split and self.L <= 4 and self.T <= 40
+                    and ((self.H == 128 and B * nF * self.n <= self.SMALL_BATCH_ROWS)
+                         or (self.H == 256 and B * nF * self.n <= self.SPLIT256_SMALL_BATCH_ROWS and self._tcxsl_available()))):
                 self.small_batch, self.tc_flags = True, 5
-                ws_xl = N.tcxl_workspace_bytes(self.I, self.H, self.L, self.T, self.O, B * nF, self.n)
+                ws_fn = N.tcxl_workspace_bytes if self.H == 128 else N.tcxsl_workspace_bytes
+                ws_xl = ws_fn(self.I, self.H, self.L, self.T, self.O, B * nF, self.n)
                 if ws_xl > self.workspace.numel():
                     self.workspace = torch.empty(ws_xl, dtype=torch.uint8, device=dev)
             # cross-call software pipeline (tensor-core path), two levels:
@@ -346,7 +354,18 @@ class BatchedEstimator:
                 self._pipe_busy = False
             self._py_dirty = True
 
+    @staticmethod
+    def _tcxsl_available():
+        """Can the current device run the H = 256 split-precision small-batch kernel (at least one of its 16-CTA clusters at once)?
+        A failed availability query counts as "no": the estimator then stays on the split layer kernels, which need no cluster of 16."""
+        try:
+            return N.tcxsl_max_active_clusters() >= 1
+        except UserWarning:
+            return False
+
     def _lstm_fn(self, variant=None):
+        if variant is None and self.tc_flags == 5 and self.H == 256:
+            return self.lib.ape_mc_lstm_tcxsl                  # the H = 256 split-precision small-batch kernel has its own entry point
         return self.lib.ape_mc_lstm_tc if (variant or self.lstm_variant) in ("tc", "tcx") else self.lib.ape_mc_lstm_fma
 
     def _lstm_launches(self, a):

@@ -149,7 +149,8 @@ typedef struct ape_lstm_args {
        arithmetic as 0..2; no initial state),
        5 = the SPLIT-PRECISION SMALL-BATCH kernel (csrc/ape_lstm_tcxl.cu: the arithmetic of 3 at H = 128 - bit-identical results - in
        the launch structure of 4: B * nF * n_samples <= 8192 rows, 2 <= L <= 4, T <= 40, O <= 16; needs weights_tcx and a workspace of
-       ape_mc_lstm_tcxl_workspace_bytes(); no initial state, no all_steps, no layer range: APE_ERR_UNSUPPORTED) */
+       ape_mc_lstm_tcxl_workspace_bytes(); no initial state, no all_steps, no layer range: APE_ERR_UNSUPPORTED; the same call of an
+       H = 256 model goes to ape_mc_lstm_tcxsl, csrc/ape_lstm_tcxsl.cu) */
     int tc_flags;
     /* optional initial state (h_0, c_0) of torch.nn.LSTM(x, hs) (nn_models.py:180-189): [L][E][H] float32 each, both or neither
        (APE_ERR_BAD_ARG); needs n_samples == 1 (APE_ERR_UNSUPPORTED; a caller with per-sample states passes the samples as estimates).
@@ -201,6 +202,21 @@ int ape_mc_lstm_tcxs_workspace_bytes_all_steps(int I, int H, int L, int T, int O
 /* workspace of a call on the split-precision small-batch kernel (tc_flags == 5: H = 128, 2 <= L <= 4, T <= 40, O <= 16,
    E * n_samples <= 8192): the h_t exchange buffer and the layer sequences, hi and lo, of one cluster per 128 rows */
 int ape_mc_lstm_tcxl_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes);
+/*
+ * Split-precision small-batch kernel for H = 256 (csrc/ape_lstm_tcxsl.cu): the arithmetic and MMA order of tc_flags == 3 at H = 256 -
+ * bit-identical results - with every layer of a call in ONE launch, one 16-CTA cluster per 128 rows (a non-portable cluster size).
+ * Same arguments as ape_mc_lstm_tc with tc_flags == 5 (else APE_ERR_BAD_ARG) and the blob in weights_tcx.  APE_ERR_UNSUPPORTED for
+ * an initial state, all_steps, a layer range, H != 256, L outside 2..4, O > 32, T > 40, I > 256 or B * nF * n_samples > 8192;
+ * APE_ERR_BAD_ARG for a missing blob or workspace or ws_E < B * nF - all before any CUDA call; an empty call returns APE_OK.  Then
+ * APE_ERR_UNSUPPORTED when the device cannot hold one cluster of the kernel (ape_mc_lstm_tcxsl_max_active_clusters() == 0).
+ * layer_ms reports the one launch as layer 0.  The workspace must hold ape_mc_lstm_tcxsl_workspace_bytes() (the h_t exchange buffer
+ * and the layer sequences, hi and lo, of one cluster per 128 rows).
+ */
+int ape_mc_lstm_tcxsl(const ape_lstm_args* args, void* stream);
+int ape_mc_lstm_tcxsl_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes);
+/* 16-CTA clusters of ape_mc_lstm_tcxsl's launch the current device holds at once (cudaOccupancyMaxActiveClusters, cached per device);
+   0 = the kernel cannot run there */
+int ape_mc_lstm_tcxsl_max_active_clusters(int* clusters);
 /* number of kernels ape_mc_lstm_tc launches for these arguments (layer pairs of an H = 128 model count once; tc_flags 4 and 5: 1) */
 int ape_mc_lstm_tc_launch_count(const ape_lstm_args* args, int* launches);
 /*

@@ -1,6 +1,8 @@
-"""Real-time latency of a split-precision model (uarm, I38 H128 L3 T6, weights x4 + forget-gate bias: the single-pass probe fails) on the
-split-precision small-batch kernel (csrc/ape_lstm_tcxl.cu, tc_flags = 5) against the split layer kernels (tc_flags = 3), with the
-single-pass cluster kernel on the unscaled weights (tc_flags = 4) as the floor.
+"""Real-time latency of a split-precision model (weights x4 + forget-gate bias: the single-pass probe fails) on the split-precision
+small-batch kernel (tc_flags = 5) against the split layer kernels (tc_flags = 3), with the single-pass cluster kernel on the unscaled
+weights (tc_flags = 4) as the floor.  --kind uarm (I38 H128 L3 T6, the default): csrc/ape_lstm_tcxl.cu; --kind pocket (I22 H256 L2 T6)
+and / or watch_only (I20 H256 L2 T8): csrc/ape_lstm_tcxsl.cu (ape_mc_lstm_tcxsl), with the number of its 16-CTA clusters the device
+holds at once.
 
   * workloads: 1, 4 and 16 streams x 100 MC samples, one frame per call, Philox masks;
   * per eager call (``step``: H2D of the rows, three stages, D2H of the results, host clock around a synchronised call) and per
@@ -11,7 +13,10 @@ single-pass cluster kernel on the unscaled weights (tc_flags = 4) as the floor.
   * the outputs of the two split paths are compared bitwise in the same run; the GPU name, power limit and maximum SM clock are read
     in the same run.
 
-    python tools/split_small_bench.py [--out profiles/split_small_bench.json] [--rounds 3]
+    python tools/split_small_bench.py [--kind uarm | pocket watch_only] [--out profiles/split_small_bench.json] [--rounds 3]
+
+The bitwise comparison and the latencies run the new kernel on every shape listed, above the estimator's row bound too (this tool
+measures the kernels, not the routing).
 """
 import argparse
 import json
@@ -27,7 +32,9 @@ sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
 from arm_pose_estimation_b200 import _native as N, synthetic as syn  # noqa: E402
 from arm_pose_estimation_b200.estimate.batched import BatchedEstimator  # noqa: E402
 
-KIND, NS = syn.KIND_UARM, 100
+NS = 100
+KINDS = {"uarm": syn.KIND_UARM, "pocket": syn.KIND_POCKET, "watch_only": syn.KIND_WATCH_ONLY}
+KIND = syn.KIND_UARM               # the model being measured (main() sets it per --kind)
 VARIANTS = {                       # name: (scaled weights, BatchedEstimator keywords, expected tc_flags)
     "split_layer_kernels": (True, dict(split_small_batch_kernel=False), 3),
     "split_small_batch_kernel": (True, dict(split_small_batch_kernel=True), 5),
@@ -66,6 +73,8 @@ def make(B, n, name):
                           stats=spec["stats"], n_streams=B, mc_samples=n, smooth=1, dropout=spec["p"], frames_per_call=1,
                           mask_mode=N.MASK_PHILOX, philox_seed=7, **kw)
     assert be.tc_flags == flags and be.tc_split == scaled, (name, be.tc_flags, be.tc_split)
+    if flags == 5:
+        assert be._lstm_fn() == (be.lib.ape_mc_lstm_tcxsl if be.H == 256 else be.lib.ape_mc_lstm_tc)
     return be
 
 
@@ -112,7 +121,7 @@ def latency(rounds, calls, frames):
 
 def bitwise(calls=8):
     res = {}
-    for B, n in ((1, 100), (4, 100), (16, 100), (16, 128)):
+    for B, n in ((1, 100), (4, 100), (16, 100), (16, 128), (64, 128)) if syn.kind_spec(KIND)["H"] == 256 else ((1, 100), (4, 100), (16, 100), (16, 128)):
         rows = syn.synth_rows(KIND, B, calls, config_id=5)
         a, b = make(B, n, "split_small_batch_kernel"), make(B, n, "split_layer_kernels")
         same = True
@@ -127,7 +136,6 @@ def bitwise(calls=8):
 
 def crossover():
     n, res = 128, {}
-    BatchedEstimator.SMALL_BATCH_ROWS = 1 << 20
     for B in (1, 2, 4, 8, 12, 16, 24, 32, 48, 64):
         rows = syn.synth_rows(KIND, B, 64, config_id=2)
         dev = [torch.from_numpy(np.ascontiguousarray(rows[:, f:f + 1])).cuda() for f in range(64)]
@@ -139,7 +147,7 @@ def crossover():
             be = BatchedEstimator(kind=KIND, layout=spec["layout"], state=state_for(True), seq_len=spec["T"], y_targets=spec["y_targets"],
                                   stats=spec["stats"], n_streams=B, mc_samples=n, smooth=1, dropout=spec["p"], frames_per_call=1,
                                   mask_mode=N.MASK_PHILOX, philox_seed=7, **kw)
-            assert be.tc_split and be.tc_flags == (5 if kw["split_small_batch_kernel"] else 3)
+            assert be.tc_split and be.tc_flags == (5 if kw["split_small_batch_kernel"] else 3), (B, be.tc_flags)
             for f in range(8):
                 be.step_device(dev[f], raw_ready=True)
             torch.cuda.synchronize()
@@ -156,13 +164,26 @@ def crossover():
             del be
         res[B * n] = line
         print("rows", B * n, json.dumps(line), flush=True)
-    BatchedEstimator.SMALL_BATCH_ROWS = 2048
     return res
 
 
+def measure_model(args):
+    spec = syn.kind_spec(KIND)
+    result = {"model": f"{syn.KIND_NAMES[KIND]} I{spec['I']} H{spec['H']} L{spec['L']} T{spec['T']} O{spec['O']}, LSTM weights x4 + "
+              "forget-gate bias +1 (single-pass probe fails); floor: the same model unscaled on the single-pass cluster kernel",
+              "mc_samples": NS, "masks": "Philox"}
+    result["bitwise_equal_split_paths"] = bitwise()
+    print("bitwise", result["bitwise_equal_split_paths"], flush=True)
+    result["latency"] = latency(args.rounds, args.calls, args.frames)
+    result["crossover_rows_n128"] = crossover()
+    return result
+
+
 def main():
+    global KIND
     ap = argparse.ArgumentParser()
-    ap.add_argument("--out", default="profiles/split_small_bench.json")
+    ap.add_argument("--kind", nargs="+", choices=list(KINDS), default=["uarm"])
+    ap.add_argument("--out", default=None, help="default: profiles/split_small_bench.json (uarm), profiles/split_small256_bench.json")
     ap.add_argument("--rounds", type=int, default=3)
     ap.add_argument("--calls", type=int, default=200)
     ap.add_argument("--frames", type=int, default=400)
@@ -170,17 +191,29 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("split_small_bench.py measures on the GPU; there is no CPU mode")
     torch.cuda.set_device(0)
-    result = {"gpu": gpu_info(), "model": "uarm I38 H128 L3 T6 O14, LSTM weights x4 + forget-gate bias +1 (single-pass probe fails); "
-              "floor: the same model unscaled on the single-pass cluster kernel", "mc_samples": NS, "masks": "Philox"}
-    result["bitwise_equal_split_paths"] = bitwise()
-    print("bitwise", result["bitwise_equal_split_paths"], flush=True)
-    result["latency"] = latency(args.rounds, args.calls, args.frames)
-    result["crossover_rows_n128"] = crossover()
+    h256 = [k for k in args.kind if syn.kind_spec(KINDS[k])["H"] == 256]
+    if h256 and len(h256) != len(args.kind):
+        raise SystemExit("--kind: uarm (H = 128) or the H = 256 models, not both in one run")
+    out = args.out or ("profiles/split_small256_bench.json" if h256 else "profiles/split_small_bench.json")
+    bounds = BatchedEstimator.SMALL_BATCH_ROWS, BatchedEstimator.SPLIT256_SMALL_BATCH_ROWS
+    BatchedEstimator.SMALL_BATCH_ROWS = BatchedEstimator.SPLIT256_SMALL_BATCH_ROWS = 1 << 20    # every shape on the new kernel
+    if not h256:                       # (the uarm run keeps the layout of its earlier measurements)
+        KIND = syn.KIND_UARM
+        result = {"gpu": gpu_info(), **measure_model(args)}
+        same = result["bitwise_equal_split_paths"]
+    else:
+        result = {"gpu": gpu_info(), "max_active_clusters": N.tcxsl_max_active_clusters(), "models": {}}
+        print("max_active_clusters", result["max_active_clusters"], flush=True)
+        for k in h256:
+            KIND = KINDS[k]
+            result["models"][k] = measure_model(args)
+        same = {f"{k} {s}": v for k in h256 for s, v in result["models"][k]["bitwise_equal_split_paths"].items()}
+    BatchedEstimator.SMALL_BATCH_ROWS, BatchedEstimator.SPLIT256_SMALL_BATCH_ROWS = bounds
     result["gpu_after"] = gpu_info()
-    Path(args.out).parent.mkdir(parents=True, exist_ok=True)
-    Path(args.out).write_text(json.dumps(result, indent=1) + "\n")
-    assert all(result["bitwise_equal_split_paths"].values()), "the two split paths differ"
-    print("wrote", args.out)
+    Path(out).parent.mkdir(parents=True, exist_ok=True)
+    Path(out).write_text(json.dumps(result, indent=1) + "\n")
+    assert all(same.values()), "the two split paths differ"
+    print("wrote", out)
 
 
 if __name__ == "__main__":
