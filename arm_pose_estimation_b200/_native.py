@@ -26,7 +26,7 @@ SYMBOLS = (
     "ape_mc_lstm_workspace_bytes", "ape_mc_lstm_fma", "ape_mc_lstm_tc_supported", "ape_lstm_tc_blob_bytes",
     "ape_mc_lstm_tc_workspace_bytes", "ape_mc_lstm_tc_workspace_bytes_all_steps", "ape_mc_lstm_tc", "ape_mc_lstm_tc_launch_count", "ape_mc_lstm_tcx_supported", "ape_lstm_tcx_blob_bytes", "ape_mc_lstm_tcx_workspace_bytes", "ape_mc_lstm_tcx_workspace_bytes_all_steps", "ape_mc_lstm_tcxs_supported", "ape_lstm_tcxs_blob_bytes", "ape_mc_lstm_tcxs_workspace_bytes",
     "ape_mc_lstm_tcxs_workspace_bytes_all_steps", "ape_mc_lstm_tcxl_workspace_bytes", "ape_mc_lstm_tcxsl", "ape_mc_lstm_tcxsl_workspace_bytes",
-    "ape_mc_lstm_tcxsl_max_active_clusters", "ape_philox_masks", "ape_ff_blob_floats", "ape_mc_ff", "ape_dense_act", "ape_fk_reduce", "ape_msg_from_est",
+    "ape_mc_lstm_tcxsl_max_active_clusters", "ape_philox_masks", "ape_ff_blob_floats", "ape_mc_ff", "ape_mc_ff_ring", "ape_dense_act", "ape_fk_reduce", "ape_msg_from_est",
     "ape_pipeline_create", "ape_pipeline_destroy", "ape_pipeline_submit", "ape_pipeline_wait", "ape_pipeline_query", "ape_pipeline_sync",
     "ape_pipeline_fence", "ape_pipeline_stream",
     "ape_selfcheck_philox", "ape_selfcheck_keep8", "ape_selfcheck_features", "ape_selfcheck_row_pose", "ape_selfcheck_tcs_schedule",
@@ -174,6 +174,8 @@ def load():
     lib.ape_dense_act.argtypes = [vp, vp, vp, vp, i32, i32, i32, i32, vp]
     lib.ape_mc_ff.restype = i32
     lib.ape_mc_ff.argtypes = [vp, i32, i32, i32, i32, f32, vp, i32, i32, i32, vp, u64, u32, u32, vp, vp]
+    lib.ape_mc_ff_ring.restype = i32
+    lib.ape_mc_ff_ring.argtypes = [vp, i32, i32, i32, i32, i32, f32, vp, i32, i32, i32, i32, vp, i32, i32, vp, u64, u32, vp, i32, vp]
     lib.ape_fk_reduce.restype = i32
     lib.ape_fk_reduce.argtypes = [vp, i32, vp, vp, vp, i32, i32, i32, i32, i32, vp, i32, i32, vp, vp, vp, vp, vp, vp]
     lib.ape_msg_from_est.restype = i32

@@ -3,6 +3,7 @@
 // evaluated once per input row, and only  y_s = W_o (mask_s * h) / (1 - p) + b_o  runs per sample.  fp32 FFMA throughout.
 // Two kernels: the batched one (8 rows per CTA, below) for the usual shapes, and a generic one-CTA-per-row kernel (threads over output
 // units for the dense layers, then one warp per MC sample with a warp-shuffle reduction per output) for everything else.
+// ape_mc_ff_ring runs the batched kernel on the rings of the batched path (BatchedEstimator with a feed-forward state dict).
 // Not on the deployed models' path.
 #include "ape_common.cuh"
 
@@ -20,7 +21,11 @@ struct FfArgs {
     uint64_t seed;
     uint32_t stream_id0, frame0, keep_thr16;
     float keep_scale;
-    float* preds;            // [rows][n][O]
+    float* preds;            // [rows][n][O]; ring mode: [B][pred_ring][n][O]
+    // ring mode (ape_mc_ff_ring): row e = b * nF + j is frame f = stream_frame0(stream_frames, frame0, b) + j of stream b, its input
+    // the window of frames f - T + 1 .. f (time-major, I = T * Ifr) of the feature ring x = [B][feat_ring][Ifr]
+    const int32_t* stream_frames;
+    int Ifr, T, feat_ring, nF, pred_ring;
 };
 
 __global__ void __launch_bounds__(FF_THREADS) mc_ff_row_kernel(FfArgs a) {
@@ -90,9 +95,11 @@ __global__ void __launch_bounds__(FF_THREADS) mc_ff_row_kernel(FfArgs a) {
 // hidden vector swept against W_o^T in shared memory (every lane reads the same weights: broadcast loads, OP FMAs per unit).
 // The row kernel above re-read every weight per row and left half of its threads idle in the hidden stack: 0.252 ms for 1024 rows x 100
 // samples (I = 110, H = 128, two hidden layers) against 0.050 ms here (8192 rows: 0.21 ms = 0.24 of the measured fp32 FMA peak).
+// RING: the rows are windows of the feature ring and the outputs go to the prediction ring (ape_mc_ff_ring); only the addressing
+// of the input tile, the Philox counters (stream b, frame f instead of stream_id0 + row, frame0) and the store differ.
 constexpr int FF_TR = 8, FF_KC = 32, FF_HB = 128;
 
-template <int OP>
+template <int OP, bool RING>
 __global__ void __launch_bounds__(FF_THREADS) mc_ff_kernel(FfArgs a, PhiloxRoundKeys rk) {
     extern __shared__ __align__(16) float sh[];
     const int KM = ((a.I > a.H ? a.I : a.H) + FF_KC - 1) / FF_KC * FF_KC;     // tile row: k-chunks never read past it
@@ -104,7 +111,18 @@ __global__ void __launch_bounds__(FF_THREADS) mc_ff_kernel(FfArgs a, PhiloxRound
     const int nr = min(FF_TR, a.rows - row0);
     for (int i = tid; i < FF_TR * KM; i += FF_THREADS) {
         const int r = i / KM, k = i - r * KM;
-        act0[i] = (r < nr && k < a.I) ? a.x[(size_t)(row0 + r) * a.I + k] : 0.0f;
+        float v = 0.0f;
+        if (r < nr && k < a.I) {
+            if constexpr (RING) {                      // frames before 0 read frame 0 (estimator.py:96-97, as ape_lstm_fma.cu)
+                const int e = row0 + r, b = e / a.nF, t = k / a.Ifr;
+                int fw = stream_frame0(a.stream_frames, (int)a.frame0, b) + e % a.nF - a.T + 1 + t;
+                fw = fw < 0 ? 0 : fw;
+                v = __ldg(a.x + ((size_t)b * a.feat_ring + fw % a.feat_ring) * a.Ifr + (k - t * a.Ifr));
+            } else {
+                v = a.x[(size_t)(row0 + r) * a.I + k];
+            }
+        }
+        act0[i] = v;
     }
     const float* w = a.blob;
     int K = a.I;
@@ -170,6 +188,13 @@ __global__ void __launch_bounds__(FF_THREADS) mc_ff_kernel(FfArgs a, PhiloxRound
     __syncthreads();
     for (int p = tid; p < nr * a.n; p += FF_THREADS) {
         const int rr = p / a.n, s = p - rr * a.n, row = row0 + rr;
+        uint32_t sid = a.stream_id0 + (uint32_t)row, frm = a.frame0;
+        int fb = 0;
+        if constexpr (RING) {
+            fb = stream_frame0(a.stream_frames, (int)a.frame0, row / a.nF);
+            sid = a.stream_id0 + (uint32_t)(row / a.nF);
+            frm = (uint32_t)(fb + row % a.nF);
+        }
         const float* h = cur + rr * KM;
         float acc[OP];
 #pragma unroll
@@ -182,7 +207,7 @@ __global__ void __launch_bounds__(FF_THREADS) mc_ff_kernel(FfArgs a, PhiloxRound
 #pragma unroll
                 for (int j = 0; j < 4; ++j) keep |= (((mm.x >> (8 * j)) & 0xFFu) ? 1u : 0u) << j | (((mm.y >> (8 * j)) & 0xFFu) ? 1u : 0u) << (4 + j);
             } else if (a.mask_mode == APE_MASK_PHILOX) {   // gap id 15 is reserved for the feed-forward output dropout
-                const uint4 f = philox_keep_flags_rk(rk, a.stream_id0 + (uint32_t)row, a.frame0, (uint32_t)s, 15u, 0u, (uint32_t)g, a.keep_thr16);
+                const uint4 f = philox_keep_flags_rk(rk, sid, frm, (uint32_t)s, 15u, 0u, (uint32_t)g, a.keep_thr16);
                 const uint32_t fw[4] = {f.x, f.y, f.z, f.w};
                 keep = 0;
 #pragma unroll
@@ -203,6 +228,10 @@ __global__ void __launch_bounds__(FF_THREADS) mc_ff_kernel(FfArgs a, PhiloxRound
             }
         }
         float* dst = a.preds + ((size_t)row * a.n + s) * a.O;
+        if constexpr (RING) {
+            if (fb < 0) continue;                      // the stream sits this call out: its prediction ring stays untouched
+            dst = a.preds + (((size_t)(row / a.nF) * a.pred_ring + frm % (uint32_t)a.pred_ring) * a.n + s) * a.O;
+        }
 #pragma unroll
         for (int o = 0; o < OP; ++o)
             if (o < a.O) dst[o] = acc[o] + __ldg(bo + o);
@@ -280,7 +309,8 @@ extern "C" int ape_mc_ff(const float* blob, int I, int H, int Lh, int O, float d
     if (mask_mode != APE_MASK_NONE && !(dropout_p >= 0.0f && dropout_p < 1.0f)) return APE_ERR_BAD_ARG;
     if (rows == 0) return APE_OK;
     FfArgs a{blob, I, H, Lh, O, x, rows, n_samples, mask_mode, masks, philox_seed, stream_id0, frame0,
-             keep_threshold16(dropout_p), mask_mode == APE_MASK_NONE ? 1.0f : 1.0f / (1.0f - dropout_p), preds};
+             keep_threshold16(dropout_p), mask_mode == APE_MASK_NONE ? 1.0f : 1.0f / (1.0f - dropout_p), preds,
+             nullptr, I, 1, 1, 1, 1};
     // the batched kernel wants 16-byte rows of W^T / the masks (H % 8 == 0, aligned pointers) and its tiles in shared memory
     const int OP = O <= 16 ? 16 : 20;
     const size_t bsmem = ff_batched_smem(I, H, OP);
@@ -289,11 +319,11 @@ extern "C" int ape_mc_ff(const float* blob, int I, int H, int Lh, int O, float d
         const PhiloxRoundKeys rk = philox_round_keys(philox_seed);
         const int grid = (rows + FF_TR - 1) / FF_TR;
         if (OP == 16) {
-            if (bsmem > 48 * 1024) APE_CUDA_TRY(cudaFuncSetAttribute(mc_ff_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem));
-            mc_ff_kernel<16><<<grid, FF_THREADS, bsmem, (cudaStream_t)stream>>>(a, rk);
+            if (bsmem > 48 * 1024) APE_CUDA_TRY(cudaFuncSetAttribute(mc_ff_kernel<16, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem));
+            mc_ff_kernel<16, false><<<grid, FF_THREADS, bsmem, (cudaStream_t)stream>>>(a, rk);
         } else {
-            if (bsmem > 48 * 1024) APE_CUDA_TRY(cudaFuncSetAttribute(mc_ff_kernel<20>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem));
-            mc_ff_kernel<20><<<grid, FF_THREADS, bsmem, (cudaStream_t)stream>>>(a, rk);
+            if (bsmem > 48 * 1024) APE_CUDA_TRY(cudaFuncSetAttribute(mc_ff_kernel<20, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem));
+            mc_ff_kernel<20, false><<<grid, FF_THREADS, bsmem, (cudaStream_t)stream>>>(a, rk);
         }
         return check_launch();
     }
@@ -302,5 +332,39 @@ extern "C" int ape_mc_ff(const float* blob, int I, int H, int Lh, int O, float d
     if (smem > 48 * 1024)
         APE_CUDA_TRY(cudaFuncSetAttribute(mc_ff_row_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     mc_ff_row_kernel<<<rows, FF_THREADS, smem, (cudaStream_t)stream>>>(a);
+    return check_launch();
+}
+
+extern "C" int ape_mc_ff_ring(const float* blob, int I, int T, int H, int Lh, int O, float dropout_p,
+                              const float* feats, int feat_ring, int B, int nF, int frame0, const int32_t* stream_frames,
+                              int n_samples, int mask_mode, const uint8_t* masks, uint64_t philox_seed, uint32_t stream_id0,
+                              float* preds, int pred_ring, void* stream) {
+    using namespace ape;
+    if (!blob || !feats || !preds || I < 1 || T < 1 || H < 1 || Lh < 0 || O < 1 || O > 20 || B < 0 || nF < 1 || n_samples < 1)
+        return APE_ERR_BAD_ARG;
+    if (feat_ring < nF + T - 1 || frame0 < 0 || pred_ring < nF) return APE_ERR_BAD_ARG;
+    if (mask_mode < APE_MASK_NONE || mask_mode > APE_MASK_PHILOX) return APE_ERR_BAD_ARG;
+    if (mask_mode == APE_MASK_INJECTED && !masks) return APE_ERR_BAD_ARG;
+    if (mask_mode != APE_MASK_NONE && !(dropout_p >= 0.0f && dropout_p < 1.0f)) return APE_ERR_BAD_ARG;
+    if ((int64_t)I * T > (1 << 20) || (int64_t)B * nF > (1 << 30)) return APE_ERR_BAD_ARG;
+    // the batched kernel only (no ring form of the one-CTA-per-row kernel): 16-byte rows of W^T / the masks, tiles in shared memory
+    const int OP = O <= 16 ? 16 : 20;
+    const size_t bsmem = ff_batched_smem(I * T, H, OP);
+    const bool aligned = H % 8 == 0 && ((uintptr_t)blob & 15) == 0 && (mask_mode != APE_MASK_INJECTED || ((uintptr_t)masks & 7) == 0);
+    if (!aligned || bsmem > 200 * 1024) return APE_ERR_UNSUPPORTED;
+    const int rows = B * nF;
+    if (rows == 0) return APE_OK;
+    FfArgs a{blob, I * T, H, Lh, O, feats, rows, n_samples, mask_mode, masks, philox_seed, stream_id0, (uint32_t)frame0,
+             keep_threshold16(dropout_p), mask_mode == APE_MASK_NONE ? 1.0f : 1.0f / (1.0f - dropout_p), preds,
+             stream_frames, I, T, feat_ring, nF, pred_ring};
+    const PhiloxRoundKeys rk = philox_round_keys(philox_seed);
+    const int grid = (rows + FF_TR - 1) / FF_TR;
+    if (OP == 16) {
+        if (bsmem > 48 * 1024) APE_CUDA_TRY(cudaFuncSetAttribute(mc_ff_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem));
+        mc_ff_kernel<16, true><<<grid, FF_THREADS, bsmem, (cudaStream_t)stream>>>(a, rk);
+    } else {
+        if (bsmem > 48 * 1024) APE_CUDA_TRY(cudaFuncSetAttribute(mc_ff_kernel<20, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bsmem));
+        mc_ff_kernel<20, true><<<grid, FF_THREADS, bsmem, (cudaStream_t)stream>>>(a, rk);
+    }
     return check_launch();
 }

@@ -64,6 +64,18 @@ def gather_host_results(local, first_stream, n_streams, group=None):
     return out
 
 
+def ff_window(model_inputs, frame_features, seq_len):
+    """Frames in the input window of a feed-forward model with ``model_inputs`` inputs over frames of ``frame_features`` features:
+    ``seq_len`` for a ``DropoutFF2D`` (the flattened ``[seq_len, frame_features]`` window), 1 for a ``DropoutFF`` (it sees the
+    newest frame only: run on every frame of the window, the estimator keeps the last step)."""
+    if model_inputs == max(1, int(seq_len)) * frame_features:
+        return max(1, int(seq_len))
+    if model_inputs == frame_features:
+        return 1
+    raise UserWarning(f"the estimator produces {frame_features} features per frame ({max(1, int(seq_len))} frames: "
+                      f"{max(1, int(seq_len)) * frame_features} inputs), the feed-forward model takes {model_inputs}")
+
+
 def ring_slots(n_frames_per_call, history):
     """Slots a device ring needs so that one call of ``n_frames_per_call`` frames still finds the ``history - 1``
     frames before its first one (``history`` = sequence_len for features, smooth for predictions)."""
@@ -143,10 +155,19 @@ class BatchedEstimator:
         self.lib = N.load()
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.kind, self.layout = int(kind), int(layout)
-        self.I, self.H, self.L, self.O = nn_models.lstm_dims(state)
-        if KIND_FEATURES[self.kind] != self.I:
-            raise UserWarning(f"estimator kind {kind} produces {KIND_FEATURES[self.kind]} features, the model takes {self.I}")
-        self.T, self.smooth, self.n = max(1, int(seq_len)), max(1, int(smooth)), int(mc_samples)
+        # a DropoutFF / DropoutFF2D state dict (nn_models.py:252-370): stage 2 is ape_mc_ff_ring over the feature ring, L counts
+        # the hidden layers behind the input layer, T is the window the model's input width spans (ff_window)
+        self.ff = "_input_layer.weight" in state
+        if self.ff:
+            I_ff, self.H, self.L, self.O = nn_models.ff_dims(state)
+            self.I = KIND_FEATURES[self.kind]
+            self.T = ff_window(I_ff, self.I, seq_len)
+        else:
+            self.I, self.H, self.L, self.O = nn_models.lstm_dims(state)
+            if KIND_FEATURES[self.kind] != self.I:
+                raise UserWarning(f"estimator kind {kind} produces {KIND_FEATURES[self.kind]} features, the model takes {self.I}")
+            self.T = max(1, int(seq_len))
+        self.smooth, self.n = max(1, int(smooth)), int(mc_samples)
         self.S = self.smooth * self.n
         self.p = float(dropout)
         self.B, self.nF_max = int(n_streams), max(1, int(frames_per_call))
@@ -163,7 +184,7 @@ class BatchedEstimator:
         self.ncols = LAYOUT_NCOLS[self.layout]
         dev, f32 = self.device, torch.float32
         with torch.cuda.device(dev):
-            self.weights = torch.from_numpy(nn_models.pack_lstm_weights(state)).to(dev)
+            self.weights = torch.from_numpy(nn_models.pack_ff_weights(state) if self.ff else nn_models.pack_lstm_weights(state)).to(dev)
             if normalize:
                 self.xx_m = torch.as_tensor(np.asarray(stats["xx_m"], dtype=np.float64)).to(dev)
                 self.xx_s = torch.as_tensor(np.asarray(stats["xx_s"], dtype=np.float64)).to(dev)
@@ -191,8 +212,10 @@ class BatchedEstimator:
             self.copy_done = [None] * NS
             self._use_out(0)
             # sized for the largest call; a shorter call re-tiles its rows, so leave one tile of slack per buffer
-            ws_bytes = N.workspace_bytes(self.I, self.H, self.L, self.T, self.O, B * nF, self.n) + 3 * 64 * self.T * self.H * 4
-            self.workspace = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            self.workspace = None                          # (the feed-forward kernel needs none)
+            if not self.ff:
+                ws_bytes = N.workspace_bytes(self.I, self.H, self.L, self.T, self.O, B * nF, self.n) + 3 * 64 * self.T * self.H * 4
+                self.workspace = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
             # pinned staging for the host-facing calls: N_SLOTS slots, so the next calls can be staged and enqueued while the
             # results of call k are still on their way back (submit() / PendingEstimate.result())
             self.raw_host = [torch.zeros((B, nF, self.ncols), dtype=f32).pin_memory() for _ in range(NS)]
@@ -214,8 +237,11 @@ class BatchedEstimator:
             self.lstm_variant = "fp32"
             if lstm_variant not in ("auto", "fp32", "tc", "tcx"):
                 raise UserWarning(f"lstm_variant must be 'auto', 'fp32', 'tc' or 'tcx', got {lstm_variant!r}")
-            tc_ok = N.tc_supported(self.I, self.H, self.L, self.O) and self.T <= 40
-            tcx_ok = N.split_supported(self.I, self.H, self.L, self.O) and self.T <= 40
+            if self.ff and lstm_variant not in ("auto", "fp32"):
+                raise UserWarning(f"a feed-forward model runs on the fp32 FFMA kernel only: lstm_variant 'auto' or 'fp32', got {lstm_variant!r}")
+            # (a feed-forward model: no tensor-core kernel, so no probe, no small-batch kernel and no cross-call pipeline)
+            tc_ok = not self.ff and N.tc_supported(self.I, self.H, self.L, self.O) and self.T <= 40
+            tcx_ok = not self.ff and N.split_supported(self.I, self.H, self.L, self.O) and self.T <= 40
             if lstm_variant == "tc" and not tc_ok:
                 raise UserWarning(f"the tensor-core LSTM kernel does not support H={self.H}, L={self.L}")
             if lstm_variant == "tcx" and not tcx_ok:
@@ -466,6 +492,25 @@ class BatchedEstimator:
         a.weights_tcx = None if self.tcx_weights is None else self.tcx_weights.data_ptr()
         return a, md
 
+    def _ff_masks(self, nF, masks):
+        """The device copy of a feed-forward model's injected output-dropout masks ``[B, nF, n, H]`` (None without injected masks),
+        kept alive by the caller until the launch is enqueued."""
+        if self.mask_mode != N.MASK_INJECTED:
+            return None
+        if masks is None:
+            raise UserWarning("mask_mode is MASK_INJECTED: pass masks [B, nF, n, H] uint8")
+        md = torch.as_tensor(masks).to(device=self.device, dtype=torch.uint8).contiguous()
+        if md.numel() != self.B * nF * self.n * self.H:
+            raise UserWarning("masks of a feed-forward model must be [B, nF, n, H]")
+        return md
+
+    def _ff_call(self, nF, frame0, sf, md, stream_ptr):
+        """Stage 2 of a feed-forward model: ``ape_mc_ff_ring`` from the feature ring into the prediction ring."""
+        N.check(self.lib.ape_mc_ff_ring(N.ptr(self.weights), self.I, self.T, self.H, self.L, self.O, self.p, N.ptr(self.feats),
+                                        self.feat_ring, self.B, nF, frame0, N.ptr(sf), self.n, self.mask_mode, N.ptr(md),
+                                        self.philox_seed, self.first_stream, N.ptr(self.preds), self.pred_ring, stream_ptr),
+                "ape_mc_ff_ring")
+
     # ---- the reference's three per-frame calls, one by one (estimator.py:174-176) ------------------------------------
     def step_features(self, xx, masks=None):
         """``add_xx_to_row_hist_and_make_prediction`` for all streams: ``xx [B, I]`` float64 rows as ``parse_row_to_xx`` returned
@@ -476,15 +521,19 @@ class BatchedEstimator:
         with torch.cuda.device(self.device):
             st = N.current_stream_ptr()
             xd = torch.from_numpy(xx).to(self.device)
+            md = self._ff_masks(1, masks) if self.ff else None
             N.check(self.lib.ape_features_push(N.ptr(xd), self.I, N.ptr(self.xx_m), N.ptr(self.xx_s), 1 if self.normalize else 0,
                                                N.ptr(self.feats), self.B, self.frame, None, self.feat_ring, st), "ape_features_push")
-            a, md = self._lstm_args(1, self.frame, None, masks)
-            N.check(self._lstm_fn()(a, st), "ape_mc_lstm")
+            if self.ff:
+                self._ff_call(1, self.frame, None, md, st)
+            else:
+                a, md = self._lstm_args(1, self.frame, None, masks)
+                N.check(self._lstm_fn()(a, st), "ape_mc_lstm")
             slots = [max(0, k) % self.pred_ring for k in range(self.frame - self.smooth + 1, self.frame + 1)]
             window = self.preds[:, slots].cpu().numpy().astype(np.float64)          # [B, smooth, n, O]
         if self.normalize:
             window = window * self.yy_s_host + self.yy_m_host                       # estimator.py:108-109
-        self.launches += 1 + self._lstm_launches(a)
+        self.launches += 2 if self.ff else 1 + self._lstm_launches(a)
         self.calls += 1
         self.frame += 1
         return window.reshape(self.B, self.S, self.O)
@@ -525,7 +574,9 @@ class BatchedEstimator:
         frame0, sf = (self.frame, None) if stream_frames is None else (0, stream_frames)
         if sf is not None and (sf.dtype != torch.int32 or sf.numel() != B or not sf.is_cuda):
             raise UserWarning("stream_frames must be a device int32 tensor of B entries")
-        a, md = self._lstm_args(nF, frame0, sf, masks)
+        if self.ff and (layer_ms is not None or trace is not None or timeline is not None):
+            raise UserWarning("layer_ms / trace / timeline are legs of the LSTM kernels")
+        a, md = (None, self._ff_masks(nF, masks)) if self.ff else self._lstm_args(nF, frame0, sf, masks)
         if layer_ms is not None:                     # profiling leg: float32 host array of L entries, filled on return
             a.layer_ms = layer_ms.ctypes.data
         if trace is not None:                        # debugging: device int64[768] of SM-clock stamps (tensor-core path)
@@ -605,9 +656,12 @@ class BatchedEstimator:
                 sf.copy_(_frames_from, non_blocking=True)
             st = N.current_stream_ptr()
             features(st)
-            N.check(self._lstm_fn()(a, st), "ape_mc_lstm")
+            if self.ff:
+                self._ff_call(nF, frame0, sf, md, st)
+            else:
+                N.check(self._lstm_fn()(a, st), "ape_mc_lstm")
             stage3(st)
-        self.launches += 2 + self._lstm_launches(a)
+        self.launches += 2 + (1 if self.ff else self._lstm_launches(a))
         self.calls += 1
         out = EstimateBatch(self._view(self.msg, nF), self._view(self.std, nF), self._view(self.samples, nF),
                             self._view(self.status, nF), self.frame)

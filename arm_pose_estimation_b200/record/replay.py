@@ -116,7 +116,8 @@ def relabel_recordings(recordings, make_estimator, frames_per_call=16, keep_samp
     """Offline relabelling: ``recordings`` = list of ``[frames_i, ncols]`` arrays (or one ``[R, F, ncols]`` array);
     ``make_estimator(n_streams, frames_per_call)`` returns a ``BatchedEstimator``.  Returns a list of dicts with
     ``msg [frames_i, 25]``, ``std [frames_i, 6]`` (and ``samples`` if asked).  The next calls are staged and enqueued while call k runs.
-    ``masks``: explicit dropout masks ``[R, F, L-1, T, n, H]`` for an estimator built with ``MASK_INJECTED`` (parity runs)."""
+    ``masks``: explicit dropout masks ``[R, F, L-1, T, n, H]`` for an estimator built with ``MASK_INJECTED`` (parity runs); for a
+    feed-forward model (``DropoutFF`` / ``DropoutFF2D``) its output-dropout masks ``[R, F, n, H]``."""
     if isinstance(recordings, np.ndarray) and recordings.ndim == 3:
         rows, lengths = np.asarray(recordings, dtype=np.float32), np.full(len(recordings), recordings.shape[1], np.int64)
     else:

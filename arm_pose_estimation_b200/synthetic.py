@@ -80,6 +80,21 @@ def synth_imu_pose_state_dict(I, O, seed=1234):
     return sd
 
 
+def synth_ff_state_dict(I, H, Lh, O, seed=1234):
+    """State dict of the reference's ``DropoutFF`` / ``DropoutFF2D`` (``_input_layer.*``, ``_hidden_layers.{k}.*``,
+    ``_output_layer.*``; a ``DropoutFF2D`` of ``seq_len`` frames of ``input_size`` features has I = seq_len * input_size) with
+    U(-1/sqrt(K), 1/sqrt(K)) float32 numpy values (torch's Linear init, K = the layer's inputs) drawn from ``default_rng(seed)``."""
+    rng = np.random.default_rng(seed)
+    u = lambda k, *shape: rng.uniform(-1 / np.sqrt(k), 1 / np.sqrt(k), size=shape).astype(np.float32)
+    sd = {"_input_layer.weight": u(I, H, I), "_input_layer.bias": u(I, H)}
+    for l in range(Lh):
+        sd[f"_hidden_layers.{l}.weight"] = u(H, H, H)
+        sd[f"_hidden_layers.{l}.bias"] = u(H, H)
+    sd["_output_layer.weight"] = u(H, O, H)
+    sd["_output_layer.bias"] = u(H, O)
+    return sd
+
+
 def write_synthetic_deploy(dst, seed=1234):
     """Create a deploy directory ``dst`` (results.json + stats of this package, plus a seeded synthetic
     ``checkpoint.pt`` per deployed hash, saved as the ``(model_state, optimizer_state)`` tuple the reference's

@@ -238,6 +238,24 @@ int ape_ff_blob_floats(int I, int H, int Lh, int O, int64_t* floats);
 int ape_mc_ff(const float* blob, int I, int H, int Lh, int O, float dropout_p, const float* x, int rows,
               int n_samples, int mask_mode, const uint8_t* masks, uint64_t philox_seed, uint32_t stream_id0,
               uint32_t frame0, float* preds, void* stream);
+/*
+ * ape_mc_ff on the rings of the batched path: stage 2 of a feed-forward model between ape_features and ape_fk_reduce.
+ * E = B * nF rows, row e = b * nF + j is frame f = (stream_frames ? stream_frames[b] : frame0) + j of stream b (a negative
+ * stream_frames[b]: nothing of stream b is written).  Its input is the window of frames f - T + 1 .. f of the feature ring,
+ * time-major (index t * I + k, DropoutFF2D._flatten of x [1, T, I]; T = 1: DropoutFF on the newest frame), frames before 0
+ * read frame 0.  The hidden stack, FMA order and output layer are those of ape_mc_ff; the Philox counters are
+ * (stream_id0 + b, f, sample, gap 15, 0, unit octet), so row e equals ape_mc_ff on its window with stream_id0 + b, frame0 = f.
+ *   blob   pack_ff_weights() of a model with T * I inputs
+ *   feats  [B][feat_ring][I] float32 (ape_features), feat_ring >= nF + T - 1
+ *   masks  APE_MASK_INJECTED: [E][n_samples][H] of {0,1}
+ *   preds  [B][pred_ring][n_samples][O] float32 (ape_fk_reduce's input), slot f % pred_ring, pred_ring >= nF
+ * The batched kernel only: H % 8 != 0, a blob not 16-byte aligned, masks not 8-byte aligned or tiles over 200 KB of
+ * shared memory return APE_ERR_UNSUPPORTED.  O <= 20.  Every refusal comes before any CUDA call.
+ */
+int ape_mc_ff_ring(const float* blob, int I, int T, int H, int Lh, int O, float dropout_p,
+                   const float* feats, int feat_ring, int B, int nF, int frame0, const int32_t* stream_frames,
+                   int n_samples, int mask_mode, const uint8_t* masks, uint64_t philox_seed, uint32_t stream_id0,
+                   float* preds, int pred_ring, void* stream);
 
 /*
  * One dense layer over many rows, y = act(x W^T + b): the input layer of ImuPoseLSTM (nn_models.py:210-249: Linear + relu in front
