@@ -29,7 +29,7 @@ SYMBOLS = (
     "ape_mc_lstm_tcxsl_max_active_clusters", "ape_philox_masks", "ape_ff_blob_floats", "ape_mc_ff", "ape_mc_ff_ring", "ape_dense_act", "ape_fk_reduce", "ape_msg_from_est",
     "ape_pipeline_create", "ape_pipeline_destroy", "ape_pipeline_submit", "ape_pipeline_wait", "ape_pipeline_query", "ape_pipeline_sync",
     "ape_pipeline_fence", "ape_pipeline_stream",
-    "ape_selfcheck_philox", "ape_selfcheck_keep8", "ape_selfcheck_features", "ape_selfcheck_row_pose", "ape_selfcheck_tcs_schedule",
+    "ape_selfcheck_philox", "ape_selfcheck_keep8", "ape_selfcheck_keep_flags", "ape_selfcheck_features", "ape_selfcheck_row_pose", "ape_selfcheck_tcs_schedule",
     "ape_selftest_umma", "ape_selftest_ffma_peak",
 )
 
@@ -201,6 +201,8 @@ def load():
     lib.ape_selfcheck_philox.argtypes = [C.POINTER(u32), C.POINTER(u32), C.POINTER(u32)]
     lib.ape_selfcheck_keep8.restype = i32
     lib.ape_selfcheck_keep8.argtypes = [u64, u32, u32, u32, u32, u32, u32, f32, C.POINTER(u32)]
+    lib.ape_selfcheck_keep_flags.restype = i32
+    lib.ape_selfcheck_keep_flags.argtypes = [C.POINTER(u32), i32, u32, C.POINTER(u32)]
     lib.ape_selfcheck_features.restype = i32
     lib.ape_selfcheck_features.argtypes = [i32, i32, C.POINTER(f32), C.POINTER(C.c_double), C.POINTER(i32)]
     lib.ape_selfcheck_row_pose.restype = i32

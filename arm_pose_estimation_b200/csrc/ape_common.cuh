@@ -129,21 +129,25 @@ APE_HD PhiloxRoundKeys philox_round_keys(uint64_t seed) {
     for (int r = 0; r < 10; ++r) { rk.k[2 * r] = k0; rk.k[2 * r + 1] = k1; k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
     return rk;
 }
-#ifdef __CUDACC__
 // Keep FLAGS of the 8 lanes of a draw: bit 15 (low lane) and bit 31 (high lane) of word i are set iff that 16-bit lane is
 // < keep_thr16 - the same decision as `lane < keep_thr16` above, evaluated for both lanes of a word with three integer
 // operations instead of an emulated SIMD compare (the loader warps of the tensor-core kernels are issue-bound):
 //   lane < thr  <=>  thr.bit15 ? (lane.bit15 == 0 || lane.low15 < thr.low15) : (lane.bit15 == 0 && lane.low15 < thr.low15)
 //   lane.low15 < thr.low15  <=>  bit 15 of (0x7FFF + thr.low15 - lane.low15)   (no borrow between the lanes: 0 <= . <= 0xFFFE)
+// Valid for keep_thr16 <= 0xFFFF; 65536 (p = 0) is the caller's shortcut.  Host and device, so ape_selfcheck_keep_flags can
+// check every lane value on the CPU.
 struct KeepCompare { uint32_t k2, top; };      // k2: (0x7FFF + thr.low15) in both lanes; top: all ones iff thr.bit15
-__device__ __forceinline__ KeepCompare keep_compare(uint32_t keep_thr16) {
+APE_HD KeepCompare keep_compare(uint32_t keep_thr16) {
     const uint32_t k = 0x7FFFu + (keep_thr16 & 0x7FFFu);
     return {k | (k << 16), (keep_thr16 & 0x8000u) ? 0xFFFFFFFFu : 0u};
 }
-__device__ __forceinline__ uint32_t keep_flags_word(uint32_t c, const KeepCompare kc) {
+APE_HD uint32_t keep_flags_word(uint32_t c, const KeepCompare kc) {
     const uint32_t d = kc.k2 - (c & 0x7FFF7FFFu);
     return (~c & d) | (kc.top & (~c | d));     // one LOP3: top ? (~c | d) : (~c & d)
 }
+// the flag words of p = 0 (keep_thr16 == 65536): every lane kept
+constexpr uint32_t KEEP_ALL_FLAGS = 0x80008000u;
+#ifdef __CUDACC__
 // flags (bits 15 / 31) -> half2 AND-mask (0xFFFF per kept lane): one byte permute with sign replication
 __device__ __forceinline__ uint32_t keep_flags_to_halfmask(uint32_t flags) {
     uint32_t m;
@@ -153,7 +157,7 @@ __device__ __forceinline__ uint32_t keep_flags_to_halfmask(uint32_t flags) {
 // the four flag words of one draw (Philox4x32-10 with precomputed round keys; counter layout of philox_keep8)
 __device__ __forceinline__ uint4 philox_keep_flags_rk(const PhiloxRoundKeys& rk, uint32_t stream, uint32_t frame, uint32_t sample,
                                                       uint32_t gap, uint32_t t, uint32_t group, uint32_t keep_thr16) {
-    if (keep_thr16 >= 65536u) return make_uint4(0x80008000u, 0x80008000u, 0x80008000u, 0x80008000u);
+    if (keep_thr16 >= 65536u) return make_uint4(KEEP_ALL_FLAGS, KEEP_ALL_FLAGS, KEEP_ALL_FLAGS, KEEP_ALL_FLAGS);
     const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u;
     uint32_t c0 = stream, c1 = frame, c2 = (sample & 0xFFFFFu) | ((gap & 0xFu) << 20) | ((t & 0xFFu) << 24), c3 = group;
 #pragma unroll

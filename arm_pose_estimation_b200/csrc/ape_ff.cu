@@ -307,6 +307,8 @@ extern "C" int ape_mc_ff(const float* blob, int I, int H, int Lh, int O, float d
     if (mask_mode < APE_MASK_NONE || mask_mode > APE_MASK_PHILOX) return APE_ERR_BAD_ARG;
     if (mask_mode == APE_MASK_INJECTED && !masks) return APE_ERR_BAD_ARG;
     if (mask_mode != APE_MASK_NONE && !(dropout_p >= 0.0f && dropout_p < 1.0f)) return APE_ERR_BAD_ARG;
+    // the Philox counter holds the sample in 20 bits (ape_common.cuh): samples s and s + 2^20 would draw the same mask
+    if (mask_mode == APE_MASK_PHILOX && n_samples > (1 << 20)) return APE_ERR_UNSUPPORTED;
     if (rows == 0) return APE_OK;
     FfArgs a{blob, I, H, Lh, O, x, rows, n_samples, mask_mode, masks, philox_seed, stream_id0, frame0,
              keep_threshold16(dropout_p), mask_mode == APE_MASK_NONE ? 1.0f : 1.0f / (1.0f - dropout_p), preds,
@@ -347,6 +349,7 @@ extern "C" int ape_mc_ff_ring(const float* blob, int I, int T, int H, int Lh, in
     if (mask_mode == APE_MASK_INJECTED && !masks) return APE_ERR_BAD_ARG;
     if (mask_mode != APE_MASK_NONE && !(dropout_p >= 0.0f && dropout_p < 1.0f)) return APE_ERR_BAD_ARG;
     if ((int64_t)I * T > (1 << 20) || (int64_t)B * nF > (1 << 30)) return APE_ERR_BAD_ARG;
+    if (mask_mode == APE_MASK_PHILOX && n_samples > (1 << 20)) return APE_ERR_UNSUPPORTED;     // 20-bit sample field, as ape_mc_ff
     // the batched kernel only (no ring form of the one-CTA-per-row kernel): 16-byte rows of W^T / the masks, tiles in shared memory
     const int OP = O <= 16 ? 16 : 20;
     const size_t bsmem = ff_batched_smem(I * T, H, OP);

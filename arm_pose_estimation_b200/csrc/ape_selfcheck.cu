@@ -19,6 +19,15 @@ extern "C" int ape_selfcheck_keep8(uint64_t seed, uint32_t stream, uint32_t fram
     return APE_OK;
 }
 
+// the branch-free two-lane compare of the tensor-core and batched feed-forward kernels (keep_compare / keep_flags_word) on n
+// Philox output words; keep_thr16 == 65536 gives the all-kept flags philox_keep_flags_rk returns for p = 0
+extern "C" int ape_selfcheck_keep_flags(const uint32_t* words, int n, uint32_t keep_thr16, uint32_t* flags) {
+    if (!words || !flags || n < 0 || keep_thr16 > 65536u) return APE_ERR_BAD_ARG;
+    const ape::KeepCompare kc = ape::keep_compare(keep_thr16);
+    for (int i = 0; i < n; ++i) flags[i] = keep_thr16 == 65536u ? ape::KEEP_ALL_FLAGS : ape::keep_flags_word(words[i], kc);
+    return APE_OK;
+}
+
 namespace {
 struct HostRow {
     const float* p;

@@ -233,6 +233,7 @@ int ape_philox_masks(uint64_t philox_seed, uint32_t stream_id0, int B, int nF, i
  *   x      [rows][I] float32 (DropoutFF2D: the flattened [seq_len * input] window)
  *   masks  APE_MASK_INJECTED: [rows][n_samples][H] of {0,1}
  *   preds  [rows][n_samples][O] float32
+ * APE_MASK_PHILOX with n_samples > 2^20 returns APE_ERR_UNSUPPORTED before any CUDA call (the counter's sample field has 20 bits).
  */
 int ape_ff_blob_floats(int I, int H, int Lh, int O, int64_t* floats);
 int ape_mc_ff(const float* blob, int I, int H, int Lh, int O, float dropout_p, const float* x, int rows,
@@ -250,7 +251,8 @@ int ape_mc_ff(const float* blob, int I, int H, int Lh, int O, float dropout_p, c
  *   masks  APE_MASK_INJECTED: [E][n_samples][H] of {0,1}
  *   preds  [B][pred_ring][n_samples][O] float32 (ape_fk_reduce's input), slot f % pred_ring, pred_ring >= nF
  * The batched kernel only: H % 8 != 0, a blob not 16-byte aligned, masks not 8-byte aligned or tiles over 200 KB of
- * shared memory return APE_ERR_UNSUPPORTED.  O <= 20.  Every refusal comes before any CUDA call.
+ * shared memory return APE_ERR_UNSUPPORTED.  O <= 20.  APE_MASK_PHILOX with n_samples > 2^20: APE_ERR_UNSUPPORTED, as ape_mc_ff.
+ * Every refusal comes before any CUDA call.
  */
 int ape_mc_ff_ring(const float* blob, int I, int T, int H, int Lh, int O, float dropout_p,
                    const float* feats, int feat_ring, int B, int nF, int frame0, const int32_t* stream_frames,
@@ -360,6 +362,10 @@ int ape_pipeline_stream(ape_pipeline* p, int which, void** stream);
 int ape_selfcheck_philox(const uint32_t* ctr4, const uint32_t* key2, uint32_t* out4);
 int ape_selfcheck_keep8(uint64_t seed, uint32_t stream, uint32_t frame, uint32_t sample, uint32_t gap,
                         uint32_t t, uint32_t group, float dropout_p, uint32_t* keep_bits);
+/* The two-lane keep compare of the tensor-core and batched feed-forward kernels on n Philox output words: flags[i] has bit 15 set iff
+ * the low 16-bit lane of words[i] is < keep_thr16 and bit 31 iff the high lane is (the other bits carry no meaning); keep_thr16 <= 65536
+ * (65536: every lane kept). */
+int ape_selfcheck_keep_flags(const uint32_t* words, int n, uint32_t keep_thr16, uint32_t* flags);
 int ape_selfcheck_features(int kind, int layout, const float* row, double* xx, int* n_features);
 int ape_selfcheck_row_pose(int target, const double* preds, const double* body9, int use_float, double* est, int* bad);
 /* The per-step schedule of weight pieces of the H = 256 tensor-core kernel (csrc/ape_lstm_tcs.cu: walk_step) for an x-part of kgx

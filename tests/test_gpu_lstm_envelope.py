@@ -32,7 +32,7 @@ EXACT_TOL = 2e-5                     # fp32 FFMA kernel and split-precision kern
 SINGLE_TOL = 2e-4                    # single-pass fp16 operands, T <= 8
 SINGLE_TOL_LONG = 5e-4               # single-pass fp16 operands, T = 40: fp16 rounding of h_t accumulates over the steps
 TCW_VS_TC = 5e-5                     # wavefront vs one-layer launches (bias inside the accumulator, see test_gpu_tcw.py)
-FLAGS = {"tc": 1, "tcw": 2, "split": 3, "tcl": 4}
+FLAGS = {"tc": 1, "tcw": 2, "split": 3, "tcl": 4, "tcxl": 5, "tcxsl": 5}
 GUARD, PATTERN = 4096, 0xA5
 P = 0.2
 
@@ -91,7 +91,7 @@ def reference(state, x, masks, n, sel, p=P):
 
 def expected_launches(kernel, L, T, all_steps):
     """(launches, layers that start a launch) of ape_mc_lstm_tc pinned to ``kernel``."""
-    if kernel == "tcl":
+    if kernel in ("tcl", "tcxl", "tcxsl"):                 # every layer in one launch
         return 1, [0]
     if kernel == "tcw" and T >= 2:                       # layer 0 alone, then pairs (1, 2), (3, 4) .. and a lone last layer
         starts = [0] + list(range(1, L, 2))
@@ -100,12 +100,17 @@ def expected_launches(kernel, L, T, all_steps):
     return len(starts) + (1 if all_steps else 0), starts
 
 
-def run_lstm(state, x, masks, n, kernel, all_steps=False, p=P):
+def run_lstm(state, x, masks, n, kernel, all_steps=False, p=P, philox=None, nF=1, frame0=0, stream_frames=None):
     """One LSTM call on dense windows x (E, T, I) with injected masks (E, L-1, T, n, H) (None: no dropout), pinned to one kernel:
-    "fp32" (ape_mc_lstm_fma) or "tc" / "tcw" / "split" / "tcl" (ape_mc_lstm_tc with tc_flags 1 / 2 / 3 / 4).  Returns the
-    predictions (E, n, O), or with ``all_steps`` those of every step (E * n, T, O).  Checks the routing and the guard bytes."""
+    "fp32" (ape_mc_lstm_fma), "tc" / "tcw" / "split" / "tcl" / "tcxl" (ape_mc_lstm_tc with tc_flags 1 / 2 / 3 / 4 / 5) or "tcxsl"
+    (ape_mc_lstm_tcxsl).  ``philox`` = (seed, stream_id0): APE_MASK_PHILOX instead (masks None).  The E = B * nF estimates are
+    nF frames of each of B streams, from frame0 or from the host counters ``stream_frames`` [B]; the predictions go through a ring
+    of nF slots.  Returns the predictions (E, n, O), or with ``all_steps`` those of every step (E * n, T, O).  Checks the routing
+    and the guard bytes."""
     I, H, L, O = OL.lstm_dims(state)
     E, T, _ = x.shape
+    assert E % nF == 0 and (masks is None or philox is None) and (nF == 1 or not all_steps)
+    B = E // nF
     dev = torch.device("cuda")
     keep = []
     a = N.LstmArgs()
@@ -114,11 +119,14 @@ def run_lstm(state, x, masks, n, kernel, all_steps=False, p=P):
     a.weights = w.data_ptr()
     if kernel == "fp32":
         ws_bytes = N.workspace_bytes(I, H, L, T, O, E, n)
-    elif kernel == "split":
+    elif kernel in ("split", "tcxl", "tcxsl"):
         wx = torch.from_numpy(nn_models.pack_lstm_weights_tcx(state)).to(dev)
         keep.append(wx)
         a.weights_tcx = wx.data_ptr()
-        ws_bytes = (N.tcx_workspace_bytes if H == 128 else N.tcxs_workspace_bytes)(I, H, L, T, O, E, n, all_steps=all_steps)
+        if kernel == "split":
+            ws_bytes = (N.tcx_workspace_bytes if H == 128 else N.tcxs_workspace_bytes)(I, H, L, T, O, E, n, all_steps=all_steps)
+        else:
+            ws_bytes = (N.tcxl_workspace_bytes if kernel == "tcxl" else N.tcxsl_workspace_bytes)(I, H, L, T, O, E, n)
     else:
         wt = torch.from_numpy(nn_models.pack_lstm_weights_tc(state)).to(dev)
         keep.append(wt)
@@ -135,15 +143,21 @@ def run_lstm(state, x, masks, n, kernel, all_steps=False, p=P):
     a.I, a.H, a.L, a.T, a.O = I, H, L, T, O
     a.dropout_p = p
     a.x_dense, a.feat_ring_buf, a.feat_ring = xd.data_ptr(), None, 0
-    a.B, a.nF, a.frame0, a.n_samples = E, 1, 0, n
-    if masks is None:
+    a.B, a.nF, a.frame0, a.n_samples = B, nF, frame0, n
+    if stream_frames is not None:
+        sfd = torch.tensor(stream_frames, dtype=torch.int32, device=dev)
+        keep.append(sfd)
+        a.stream_frames = sfd.data_ptr()
+    if philox is not None:
+        a.mask_mode, (a.philox_seed, a.stream_id0) = N.MASK_PHILOX, philox
+    elif masks is None:
         a.mask_mode = N.MASK_NONE
     else:
         md = torch.from_numpy(np.ascontiguousarray(masks, dtype=np.uint8)).to(dev)
         keep.append(md)
         a.mask_mode, a.masks = N.MASK_INJECTED, md.data_ptr()
     a.workspace = ws.data_ptr()
-    a.preds, a.pred_ring, a.all_steps = preds.data_ptr(), 1, int(all_steps)
+    a.preds, a.pred_ring, a.all_steps = preds.data_ptr(), nF, int(all_steps)
     lib = N.load()
     if kernel == "fp32":
         N.check(lib.ape_mc_lstm_fma(a, N.current_stream_ptr()), "ape_mc_lstm_fma")
@@ -155,7 +169,8 @@ def run_lstm(state, x, masks, n, kernel, all_steps=False, p=P):
         assert count.value == want_launches, f"{kernel}: {count.value} launches, expected {want_launches}"
         ms = (C.c_float * L)(*([-1.0] * L))
         a.layer_ms = C.addressof(ms)
-        N.check(lib.ape_mc_lstm_tc(a, N.current_stream_ptr()), f"ape_mc_lstm_tc ({kernel})")
+        call = lib.ape_mc_lstm_tcxsl if kernel == "tcxsl" else lib.ape_mc_lstm_tc
+        N.check(call(a, N.current_stream_ptr()), f"ape_mc_lstm_tc ({kernel})")
         for l in range(L):                               # a launch's time goes to its first layer; the second of a pair reads 0
             if l in starts:
                 assert ms[l] > 0.0, f"{kernel}: layer {l} has no launch of its own (time {ms[l]})"
@@ -166,7 +181,11 @@ def run_lstm(state, x, masks, n, kernel, all_steps=False, p=P):
     assert bool((pbuf[4 * n_pred:] == PATTERN).all()), f"{kernel}: bytes behind the predictions were written"
     out = preds.cpu().numpy()
     assert not np.isnan(out).any(), f"{kernel}: {int(np.isnan(out).sum())} predictions were never written"
-    return out.reshape(E * n, T, O) if all_steps else out.reshape(E, n, O)
+    if all_steps:
+        return out.reshape(E * n, T, O)
+    ring = out.reshape(B, nF, n, O)                      # slot f % nF of each stream: back to estimate order
+    fb = np.full(B, frame0) if stream_frames is None else np.asarray(stream_frames)
+    return np.stack([ring[e // nF, (int(fb[e // nF]) + e % nF) % nF] for e in range(E)])
 
 
 def inputs(I, H, L, T, E, n, seed, masked=True):
