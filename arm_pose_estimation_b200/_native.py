@@ -26,9 +26,9 @@ SYMBOLS = (
     "ape_mc_lstm_workspace_bytes", "ape_mc_lstm_fma", "ape_mc_lstm_tc_supported", "ape_lstm_tc_blob_bytes",
     "ape_mc_lstm_tc_workspace_bytes", "ape_mc_lstm_tc_workspace_bytes_all_steps", "ape_mc_lstm_tc", "ape_mc_lstm_tc_launch_count", "ape_mc_lstm_tcx_supported", "ape_lstm_tcx_blob_bytes", "ape_mc_lstm_tcx_workspace_bytes", "ape_mc_lstm_tcx_workspace_bytes_all_steps", "ape_mc_lstm_tcxs_supported", "ape_lstm_tcxs_blob_bytes", "ape_mc_lstm_tcxs_workspace_bytes",
     "ape_mc_lstm_tcxs_workspace_bytes_all_steps", "ape_mc_lstm_tcxl_workspace_bytes", "ape_mc_lstm_tcxsl", "ape_mc_lstm_tcxsl_workspace_bytes",
-    "ape_mc_lstm_tcxsl_max_active_clusters", "ape_philox_masks", "ape_ff_blob_floats", "ape_mc_ff", "ape_mc_ff_ring", "ape_dense_act", "ape_fk_reduce", "ape_msg_from_est",
+    "ape_mc_lstm_tcxsl_max_active_clusters", "ape_philox_masks", "ape_ff_blob_floats", "ape_mc_ff", "ape_mc_ff_ring", "ape_dense_act", "ape_fk_reduce", "ape_fk_reduce_bodies", "ape_msg_from_est",
     "ape_pipeline_create", "ape_pipeline_destroy", "ape_pipeline_submit", "ape_pipeline_wait", "ape_pipeline_query", "ape_pipeline_sync",
-    "ape_pipeline_fence", "ape_pipeline_stream",
+    "ape_pipeline_fence", "ape_pipeline_stream", "ape_pipeline_set_bodies",
     "ape_selfcheck_philox", "ape_selfcheck_keep8", "ape_selfcheck_keep_flags", "ape_selfcheck_features", "ape_selfcheck_row_pose", "ape_selfcheck_tcs_schedule",
     "ape_selftest_umma", "ape_selftest_ffma_peak",
 )
@@ -178,6 +178,8 @@ def load():
     lib.ape_mc_ff_ring.argtypes = [vp, i32, i32, i32, i32, i32, f32, vp, i32, i32, i32, i32, vp, i32, i32, vp, u64, u32, vp, i32, vp]
     lib.ape_fk_reduce.restype = i32
     lib.ape_fk_reduce.argtypes = [vp, i32, vp, vp, vp, i32, i32, i32, i32, i32, vp, i32, i32, vp, vp, vp, vp, vp, vp]
+    lib.ape_fk_reduce_bodies.restype = i32
+    lib.ape_fk_reduce_bodies.argtypes = [vp, i32, vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, i32, i32, vp, vp, vp, vp, vp, vp]
     lib.ape_msg_from_est.restype = i32
     lib.ape_msg_from_est.argtypes = [vp, i32, vp, i32, i32, i32, vp, vp, vp]
     lib.ape_pipeline_create.restype = i32
@@ -196,6 +198,8 @@ def load():
     lib.ape_pipeline_fence.argtypes = [vp, vp]
     lib.ape_pipeline_stream.restype = i32
     lib.ape_pipeline_stream.argtypes = [vp, i32, C.POINTER(vp)]
+    lib.ape_pipeline_set_bodies.restype = i32
+    lib.ape_pipeline_set_bodies.argtypes = [vp, vp, i32]
     # host self-check hooks: used by tests/ only
     lib.ape_selfcheck_philox.restype = i32
     lib.ape_selfcheck_philox.argtypes = [C.POINTER(u32), C.POINTER(u32), C.POINTER(u32)]

@@ -55,8 +55,12 @@ template <typename F> APE_HD Vec3<F> qrot(const Quat<F>& q, const Vec3<F>& v) {
 }
 // qrot for a vector along the x axis, v = (vx, 0, 0) - the default bone vectors (bone_map.py:42-45) - written out: vx times the
 // first column of the (unnormalised) rotation matrix of q.  10 operations instead of 42.
+// The first two squares are ONE fused multiply-add, x^2 fused onto w^2, written out: left to the compiler, which of the two products
+// it fuses depended on the code around the call (the last bit of the stage-3 message moved with an unrelated change of the kernel).
+APE_HD float fmadd(float a, float b, float c) { return fmaf(a, b, c); }
+APE_HD double fmadd(double a, double b, double c) { return fma(a, b, c); }
 template <typename F> APE_HD Vec3<F> qrot_x(const Quat<F>& q, F vx) {
-    return {vx * (q.w * q.w + q.x * q.x - q.y * q.y - q.z * q.z), vx * F(2) * (q.x * q.y + q.w * q.z), vx * F(2) * (q.x * q.z - q.w * q.y)};
+    return {vx * (fmadd(q.x, q.x, q.w * q.w) - q.y * q.y - q.z * q.z), vx * F(2) * (q.x * q.y + q.w * q.z), vx * F(2) * (q.x * q.z - q.w * q.y)};
 }
 // conjugate / squared norm (transformations.py:244-254)
 template <typename F> APE_HD Quat<F> qinv(const Quat<F>& q) {

@@ -28,6 +28,7 @@ struct FkArgs {
     const float* yy_m;
     const float* yy_s;
     const float* body9;
+    int body_stride;                // floats between the skeleton rows of consecutive streams (0: one row for the whole launch)
     int O, B, nF, frame0, n, smooth;
     const int32_t* stream_frames;   // per-stream frame counters (null: frame0 for all); < 0: skip the stream
     float* msg;
@@ -124,12 +125,28 @@ __global__ void __launch_bounds__(FK_WARPS_PER_CTA * 32, APE_FK_MIN_BLOCKS(TARGE
     if (__all_sync(FK_FULL, dead)) return;
     const int S = a.smooth * a.n;
 
-    Body<float> body;
-    body.larm_vec = {a.body9[0], a.body9[1], a.body9[2]};
-    body.uarm_vec = {a.body9[3], a.body9[4], a.body9[5]};
-    body.uarm_orig = {a.body9[6], a.body9[7], a.body9[8]};
-    body.bones_along_x = bones_are_along_x(body);      // (the default skeleton: a uniform branch)
-    const F2 len = pk(body.larm_vec.x, body.uarm_vec.x), len2 = len + len;
+    // This estimate's skeleton: row b of the table (stride 0: the one shared row), staged in shared memory by the sub-warp's first nine
+    // lanes.  A sub-warp past the end keeps b = 0 and an idle stream's b is in range, so no lane reads outside the table.  Only the two
+    // bone lengths of the x-axis rotation stay in registers; the rest of the row is read back (volatile: not hoisted into registers)
+    // where it is used - a per-lane row held in registers costs ~10 registers more than the one row the whole launch shared, which the
+    // compiler kept in uniform registers, and spills at the launch bounds above.
+    // The two estimates of a warp may have different skeletons, one on the short x-axis rotation and one on the general qrot: those
+    // branches hold no shuffle, every full-mask shuffle comes before or after them.
+    __shared__ float s_body[FK_WARPS_PER_CTA * FK_SUB][9];
+    volatile float* sb = s_body[warp * FK_SUB + half];
+    if (lane < 9) sb[lane] = __ldg(a.body9 + (size_t)b * a.body_stride + lane);
+    __syncwarp();
+    auto body_vec = [&](int k) { return Vec3<float>{sb[k], sb[k + 1], sb[k + 2]}; };     // 0: larm_vec, 3: uarm_vec, 6: uarm_orig
+    auto body_row = [&]() {
+        Body<float> r;
+        r.larm_vec = body_vec(0);
+        r.uarm_vec = body_vec(3);
+        r.uarm_orig = body_vec(6);
+        r.bones_along_x = bones_are_along_x(r);
+        return r;
+    };
+    const bool along_x = body_row().bones_along_x;
+    const F2 len = pk(sb[0], sb[3]), len2 = len + len;
 
     const F2 zero2 = splat(0.0f);
     Quat2 q0{zero2, zero2, zero2, zero2}, sq{zero2, zero2, zero2, zero2};          // lo: lower arm, hi: upper arm
@@ -200,7 +217,7 @@ __global__ void __launch_bounds__(FK_WARPS_PER_CTA * 32, APE_FK_MIN_BLOCKS(TARGE
     unsigned long long* smp = a.samples ? reinterpret_cast<unsigned long long*>(a.samples + ((size_t)e * S + lane) * 6) : nullptr;   // this lane's row of the pass
     Quat2 q{splat(1.0f), zero2, zero2, zero2};
     Quat<float> hips{1.0f, 0.0f, 0.0f, 0.0f};
-    Vec3<float> shoulder = body.uarm_orig;
+    Vec3<float> shoulder = body_vec(6);
     F2 P[3] = {zero2, zero2, zero2};
     for (int i0 = 0; i0 < S; i0 += FK_LANES) {
         const int i = i0 + lane;
@@ -224,17 +241,19 @@ __global__ void __launch_bounds__(FK_WARPS_PER_CTA * 32, APE_FK_MIN_BLOCKS(TARGE
             bad |= rb && live;
             if (HIPS) {
                 hips = hips_quat(p[OH], p[OH + 1]);
-                shoulder = qrot(hips, body.uarm_orig);
+                shoulder = qrot(hips, body_vec(6));
             }
             if (POS) {                                               // positions are network outputs
                 P[0] = pk(p[0], p[1]); P[1] = pk(p[2], p[9]); P[2] = pk(p[10], p[11]);
-            } else if (body.bones_along_x) {                         // shoulder -> elbow -> hand (estimate_joints.py:61-63 / :84-85)
+            } else if (along_x) {                                    // shoulder -> elbow -> hand (estimate_joints.py:61-63 / :84-85)
+                if (!HIPS) shoulder = body_vec(6);
                 F2 vx, vy, vz;
                 qrot_x2(q, len, len2, vx, vy, vz);
                 const float ex = hi(vx) + shoulder.x, ey = hi(vy) + shoulder.y, ez = hi(vz) + shoulder.z;
                 P[0] = pk(lo(vx) + ex, lo(vy) + ey); P[1] = pk(lo(vz) + ez, ex); P[2] = pk(ey, ez);
             } else {
-                const Vec3<float> el = vadd(qrot(q_hi(q), body.uarm_vec), shoulder), ha = vadd(qrot(q_lo(q), body.larm_vec), el);
+                if (!HIPS) shoulder = body_vec(6);
+                const Vec3<float> el = vadd(qrot(q_hi(q), body_vec(3)), shoulder), ha = vadd(qrot(q_lo(q), body_vec(0)), el);
                 P[0] = pk(ha.x, ha.y); P[1] = pk(ha.z, el.x); P[2] = pk(el.y, el.z);
             }
         }
@@ -294,7 +313,7 @@ __global__ void __launch_bounds__(FK_WARPS_PER_CTA * 32, APE_FK_MIN_BLOCKS(TARGE
         m.elbow = {hi(psum[1]), lo(psum[2]), hi(psum[2])};
         m.shoulder = {pshl[0], pshl[1], pshl[2]};
     } else if (S > 1) {
-        chain(TARGET, body, m);                                               // FK again from the means
+        chain(TARGET, body_row(), m);                                               // FK again from the means
     } else {                                                                  // one row: copied as is (compose_msg.py:62-66)
         m.hand = {lo(piv[0]), hi(piv[0]), lo(piv[1])};
         m.elbow = {hi(piv[1]), lo(piv[2]), hi(piv[2])};
@@ -333,13 +352,14 @@ __global__ void __launch_bounds__(FK_WARPS_PER_CTA * 32, APE_FK_MIN_BLOCKS(TARGE
 
 }  // namespace ape
 
-extern "C" int ape_fk_reduce(const float* preds, int pred_ring, const float* yy_m, const float* yy_s,
-                             const float* body9, int target, int O, int B, int nF, int frame0, const int32_t* stream_frames, int n_samples,
-                             int smooth, float* msg, float* samples, float* stdev, float* est_rows,
-                             int32_t* status, void* stream) {
+extern "C" int ape_fk_reduce_bodies(const float* preds, int pred_ring, const float* yy_m, const float* yy_s,
+                                    const float* bodies, int body_stride, int target, int O, int B, int nF, int frame0,
+                                    const int32_t* stream_frames, int n_samples, int smooth, float* msg, float* samples, float* stdev,
+                                    float* est_rows, int32_t* status, void* stream) {
     using namespace ape;
-    if (!preds || !body9 || !msg || B < 0 || nF < 0 || frame0 < 0 || n_samples < 1 || smooth < 1 || pred_ring < 1)
+    if (!preds || !bodies || !msg || B < 0 || nF < 0 || frame0 < 0 || n_samples < 1 || smooth < 1 || pred_ring < 1)
         return APE_ERR_BAD_ARG;
+    if (body_stride < 0 || (body_stride > 0 && body_stride < 9)) return APE_ERR_BAD_ARG;   // rows of 9 floats must not overlap
     if (target < APE_TARGET_ORI_CAL_LARM_UARM || target > APE_TARGET_ORI_POS_CAL_LARM_UARM_HIPS) return APE_ERR_BAD_ARG;
     if (O != target_num_outputs(target)) return APE_ERR_BAD_ARG;
     if ((yy_m == nullptr) != (yy_s == nullptr)) return APE_ERR_BAD_ARG;
@@ -347,7 +367,8 @@ extern "C" int ape_fk_reduce(const float* preds, int pred_ring, const float* yy_
     const long long E = (long long)B * nF;
     if (E == 0) return APE_OK;
     if (E > 0x7fffffffLL || (long long)smooth * n_samples > 0x7fffffffLL) return APE_ERR_BAD_ARG;
-    FkArgs a{preds, pred_ring, yy_m, yy_s, body9, O, B, nF, frame0, n_samples, smooth, stream_frames, msg, samples, stdev, est_rows, status, nullptr};
+    FkArgs a{preds, pred_ring, yy_m, yy_s, bodies, body_stride, O, B, nF, frame0, n_samples, smooth, stream_frames, msg, samples, stdev,
+             est_rows, status, nullptr};
     const int grid = (int)((E + FK_SUB * FK_WARPS_PER_CTA - 1) / (FK_SUB * FK_WARPS_PER_CTA));
     cudaStream_t st = (cudaStream_t)stream;
     if (target == APE_TARGET_ORI_CAL_LARM_UARM)
@@ -359,6 +380,15 @@ extern "C" int ape_fk_reduce(const float* preds, int pred_ring, const float* yy_
     return check_launch();
 }
 
+// one skeleton for every stream: the table form with stride 0 (the same kernel, the same arithmetic)
+extern "C" int ape_fk_reduce(const float* preds, int pred_ring, const float* yy_m, const float* yy_s,
+                             const float* body9, int target, int O, int B, int nF, int frame0, const int32_t* stream_frames, int n_samples,
+                             int smooth, float* msg, float* samples, float* stdev, float* est_rows,
+                             int32_t* status, void* stream) {
+    return ape_fk_reduce_bodies(preds, pred_ring, yy_m, yy_s, body9, 0, target, O, B, nF, frame0, stream_frames, n_samples, smooth,
+                                msg, samples, stdev, est_rows, status, stream);
+}
+
 extern "C" int ape_msg_from_est(const float* est, int W, const float* body9, int target, int E, int S, float* msg,
                                 float* stdev, void* stream) {
     using namespace ape;
@@ -366,7 +396,7 @@ extern "C" int ape_msg_from_est(const float* est, int W, const float* body9, int
     if (target < APE_TARGET_ORI_CAL_LARM_UARM || target > APE_TARGET_ORI_POS_CAL_LARM_UARM_HIPS) return APE_ERR_BAD_ARG;
     if (W != (target == APE_TARGET_ORI_CAL_LARM_UARM ? 14 : 21)) return APE_ERR_BAD_ARG;
     if (E == 0) return APE_OK;
-    FkArgs a{nullptr, 1, nullptr, nullptr, body9, target_num_outputs(target), E, 1, 0, S, 1, nullptr, msg, nullptr, stdev, nullptr, nullptr, est};
+    FkArgs a{nullptr, 1, nullptr, nullptr, body9, 0, target_num_outputs(target), E, 1, 0, S, 1, nullptr, msg, nullptr, stdev, nullptr, nullptr, est};
     const int grid = (E + FK_SUB * FK_WARPS_PER_CTA - 1) / (FK_SUB * FK_WARPS_PER_CTA);
     cudaStream_t st = (cudaStream_t)stream;
     if (target == APE_TARGET_ORI_CAL_LARM_UARM)

@@ -46,6 +46,8 @@ struct ape_pipeline {
     // frames_host[prev_slot], which the next n_slots - 1 calls leave alone)
     bool prev_valid, prev_sf;
     int prev_nF, prev_frame0, prev_slot;
+    const float* bodies;        // stage 3's skeleton table (ape_pipeline_set_bodies; desc.body9 with stride 0 until then)
+    int body_stride;
 };
 
 #define PIPE_TRY(expr) do { int _rc = (expr); if (_rc != APE_OK) return _rc; } while (0)
@@ -82,6 +84,8 @@ extern "C" int ape_pipeline_create(const ape_pipeline_desc* d, ape_pipeline** ou
     p->last_lane = 0;
     p->calls = p->submits = 0;
     p->prev_valid = false;
+    p->bodies = d->body9;
+    p->body_stride = 0;
     *out = p;
     return APE_OK;
 }
@@ -125,6 +129,14 @@ extern "C" int ape_pipeline_fence(ape_pipeline* p, void* stream) {
     APE_CUDA_TRY(cudaStreamWaitEvent(p->side, p->ev_in, 0));
     APE_CUDA_TRY(cudaStreamWaitEvent(p->lane[0], p->ev_in, 0));
     APE_CUDA_TRY(cudaStreamWaitEvent(p->lane[1], p->ev_in, 0));
+    return APE_OK;
+}
+
+// stage 3 of the calls submitted from now on reads this table (nothing is copied: the caller keeps it unchanged while calls may read it)
+extern "C" int ape_pipeline_set_bodies(ape_pipeline* p, const float* bodies, int body_stride) {
+    if (!p || body_stride < 0 || (body_stride > 0 && body_stride < 9)) return APE_ERR_BAD_ARG;
+    p->bodies = bodies ? bodies : p->d.body9;
+    p->body_stride = bodies ? body_stride : 0;
     return APE_OK;
 }
 
@@ -219,8 +231,9 @@ extern "C" int ape_pipeline_submit(ape_pipeline* p, const float* rows_host, cons
     p->last_lane = parity;
     float* out = d.out_dev[slot];
     float* samples = d.emit_samples ? out + Em * 32 : nullptr;
-    PIPE_TRY(ape_fk_reduce(d.lstm.preds, d.lstm.pred_ring, d.yy_m, d.yy_s, d.body9, d.target, d.lstm.O, d.B, nF, f0, sf_dev,
-                           d.lstm.n_samples, d.smooth, out, samples, out + Em * 25, nullptr, (int32_t*)(out + Em * 31), lane));
+    PIPE_TRY(ape_fk_reduce_bodies(d.lstm.preds, d.lstm.pred_ring, d.yy_m, d.yy_s, p->bodies, p->body_stride, d.target, d.lstm.O, d.B,
+                                  nF, f0, sf_dev, d.lstm.n_samples, d.smooth, out, samples, out + Em * 25, nullptr,
+                                  (int32_t*)(out + Em * 31), lane));
     APE_CUDA_TRY(cudaEventRecord(p->done[bufset], lane));
     p->done_valid[bufset] = true;
     if (flags & APE_PIPE_CALLER_WAITS) APE_CUDA_TRY(cudaStreamWaitEvent(caller, p->done[bufset], 0));

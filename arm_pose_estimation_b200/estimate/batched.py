@@ -18,7 +18,7 @@ import numpy as np
 import torch
 
 from arm_pose_estimation_b200 import _native as N
-from arm_pose_estimation_b200.data_types.bone_map import body_measurements_row
+from arm_pose_estimation_b200.data_types.bone_map import body_measurements_rows
 from arm_pose_estimation_b200.estimate import nn_models
 from arm_pose_estimation_b200.utility.names import NNS_TARGETS
 
@@ -36,7 +36,9 @@ LAYOUT_NCOLS = {N.LAYOUT_WATCH_ONLY: 28, N.LAYOUT_WATCH_PHONE: 55}
 
 def shard_streams(n_streams, world_size, rank):
     """Static contiguous split of the stream axis: ``(first_stream, count)`` of ``rank`` (SURVEY.md §8e).
-    The first ``n_streams % world_size`` ranks take one extra stream; no stream is shared, no exchange follows."""
+    The first ``n_streams % world_size`` ranks take one extra stream; no stream is shared, no exchange follows.
+    Per-stream skeletons split the same way: a rank builds its ``BatchedEstimator`` with ``first_stream=first`` and
+    ``bonemaps=bonemaps[first:first + count]``, the skeletons of its own streams."""
     if world_size < 1 or not 0 <= rank < world_size or n_streams < 0:
         raise ValueError(f"bad shard request: n_streams={n_streams} world_size={world_size} rank={rank}")
     base, extra = divmod(n_streams, world_size)
@@ -149,7 +151,11 @@ class BatchedEstimator:
                  smooth=1, dropout=0.2, bonemap=None, frames_per_call=1, emit_samples=True, normalize=True,
                  mask_mode=N.MASK_PHILOX, philox_seed=0, first_stream=0, device=None,
                  lstm_variant="auto", tc_min_rows=1, tc_tolerance_m=5e-5, pipeline=True, lanes=True, tc_flags=None,
-                 native_pipeline=None, small_batch_kernel=True, split_small_batch_kernel=False):
+                 native_pipeline=None, small_batch_kernel=True, split_small_batch_kernel=False, bonemaps=None):
+        """``bonemap``: one skeleton for every stream; ``bonemaps``: one per stream (B entries for ``body_measurements_rows``, or a
+        ``[B, 9]`` array), not both.  Either way stage 3 reads a device table ``[B, 9]`` (``set_bonemaps`` / ``set_bonemap`` rewrite
+        it).  The tensor-core precision probe runs at construction on the row with the longest arm (``|larm| + |uarm|``: the
+        position error grows with bone length); a later ``set_bonemap`` does not probe again."""
         if not torch.cuda.is_available():
             raise RuntimeError("BatchedEstimator needs a CUDA device (sm_100a); there is no CPU fallback")
         self.lib = N.load()
@@ -193,7 +199,14 @@ class BatchedEstimator:
                 self.yy_m_host, self.yy_s_host = np.asarray(stats["yy_m"], dtype=np.float64), np.asarray(stats["yy_s"], dtype=np.float64)
             else:
                 self.xx_m = self.xx_s = self.yy_m = self.yy_s = None
-            self.body = torch.as_tensor(body_measurements_row(bonemap).astype(np.float32).ravel()).to(dev)
+            if bonemap is not None and bonemaps is not None:
+                raise UserWarning("pass one skeleton for every stream (bonemap) or one per stream (bonemaps), not both")
+            # stage 3's skeleton table, one row per stream (row 0 stands in for an estimator of no streams); its address never
+            # changes, so a captured step_graph graph stays valid when set_bonemap rewrites it
+            rows = body_measurements_rows([bonemap] * self.B if bonemaps is None else bonemaps, self.B)
+            self.bodies = torch.zeros((max(1, self.B), 9), dtype=f32, device=dev)
+            self.bodies[: self.B] = torch.from_numpy(rows.astype(np.float32)).to(dev)
+            torch.cuda.current_stream(dev).synchronize()     # (read by the native pipeline's own streams, which do not wait for this one)
             self.feat_ring = ring_slots(self.nF_max, self.T)
             # (two calls' worth of frames: with the two-lane pipeline the last layer of call k+1 may write its predictions
             # while stage 3 of call k still reads the smoothing window of call k)
@@ -331,7 +344,7 @@ class BatchedEstimator:
         d.raw, d.feats, d.feat_ring = self.raw.data_ptr(), self.feats.data_ptr(), self.feat_ring
         d.lstm = self._lstm_args(self.nF_max, 0, None, None)[0]
         d.lane_workspace[0], d.lane_workspace[1] = self.lane_ws[0].data_ptr(), self.lane_ws[1].data_ptr()
-        d.yy_m, d.yy_s, d.body9 = self.yy_m.data_ptr(), self.yy_s.data_ptr(), self.body.data_ptr()
+        d.yy_m, d.yy_s, d.body9 = self.yy_m.data_ptr(), self.yy_s.data_ptr(), self.bodies.data_ptr()
         d.target, d.smooth, d.emit_samples = self.target, self.smooth, 1 if self.emit_samples else 0
         d.B, d.nF_max, d.n_slots = self.B, self.nF_max, self.N_SLOTS
         self.frames_host = [torch.zeros(self.B, dtype=torch.int32).pin_memory() for _ in range(self.N_SLOTS)]
@@ -344,6 +357,7 @@ class BatchedEstimator:
         handle = ctypes.c_void_p(None)
         N.check(self.lib.ape_pipeline_create(ctypes.byref(d), ctypes.byref(handle)), "ape_pipeline_create")
         self._pipe, self._pipe_desc = handle, d
+        N.check(self.lib.ape_pipeline_set_bodies(handle, self.bodies.data_ptr(), 9), "ape_pipeline_set_bodies")
 
     def __del__(self):
         pipe, self._pipe = getattr(self, "_pipe", None), None
@@ -406,8 +420,11 @@ class BatchedEstimator:
     def _probe_tc_error(self, which="tc", n_est=16, n_samples=64):
         """Max |position| difference (metres) between a tensor-core LSTM kernel (``which``: "tc" single pass | "tcx" split precision)
         and the fp32 kernel on a probe batch: N(0,1) normalised windows, the same Philox masks for both (the keying does not depend
-        on the kernel)."""
+        on the kernel).  Stage 3 uses the skeleton with the longest arm, where a rotation error moves the hand farthest."""
         dev = self.device
+        rows = self.bodies[: max(1, self.B)].double()
+        arm = rows[:, 0:3].norm(dim=1) + rows[:, 3:6].norm(dim=1)
+        body = self.bodies[int(torch.argmax(arm).item())]
         g = torch.Generator(device="cpu").manual_seed(1234)
         x = torch.randn((n_est, self.T, self.I), generator=g, dtype=torch.float32).to(dev)
         ws = torch.empty(max(N.workspace_bytes(self.I, self.H, self.L, self.T, self.O, n_est, n_samples),
@@ -432,7 +449,7 @@ class BatchedEstimator:
             N.check(self._lstm_fn(variant)(a, N.current_stream_ptr()), f"ape_mc_lstm ({variant} probe)")
             est = torch.empty((n_est, n_samples, EST_WIDTH[self.target]), dtype=torch.float32, device=dev)
             msg = torch.empty((n_est, 25), dtype=torch.float32, device=dev)
-            N.check(self.lib.ape_fk_reduce(N.ptr(preds), 1, N.ptr(self.yy_m), N.ptr(self.yy_s), N.ptr(self.body), self.target,
+            N.check(self.lib.ape_fk_reduce(N.ptr(preds), 1, N.ptr(self.yy_m), N.ptr(self.yy_s), N.ptr(body), self.target,
                                            self.O, n_est, 1, 0, None, n_samples, 1, N.ptr(msg), None, None, N.ptr(est), None,
                                            N.current_stream_ptr()), "ape_fk_reduce (probe)")
             outs.append(est[..., :9 if EST_WIDTH[self.target] == 21 else 6].clone())
@@ -460,6 +477,33 @@ class BatchedEstimator:
     def reset(self):
         """Forget all history, like ``Estimator.reset`` (estimator.py:88-91): the next row is frame 0 again."""
         self.frame = 0
+
+    # ---- per-stream skeletons (the reference's per-instance bonemap, estimator.py:57-68) --------------------------------
+    def set_bonemaps(self, bonemaps):
+        """Give every stream its skeleton (B entries, see ``body_measurements_rows``).  Waits for the calls in flight, which keep
+        the skeletons they were submitted with; every call submitted after this returns uses the new ones."""
+        self._write_bodies(slice(0, self.B), body_measurements_rows(bonemaps, self.B))
+
+    def set_bonemap(self, b, bonemap):
+        """Give stream ``b`` its own skeleton (a BoneMap-like object, ``None`` for the default, or nine floats), e.g. when a new user
+        takes over the stream; same ordering as ``set_bonemaps``.  The tensor-core precision probe is not repeated."""
+        if not 0 <= int(b) < self.B:
+            raise UserWarning(f"stream {b} is not one of the {self.B} streams")
+        self._write_bodies(slice(int(b), int(b) + 1), body_measurements_rows([bonemap], 1))
+
+    def _write_bodies(self, rows, values):
+        with torch.cuda.device(self.device):
+            if self._pipe is not None and self._pipe_busy:
+                N.check(self.lib.ape_pipeline_sync(self._pipe), "ape_pipeline_sync")
+                self._pipe_busy = False
+            torch.cuda.synchronize(self.device)           # (the Python-level path's side, lane, copy and caller streams)
+            self.bodies[rows] = torch.from_numpy(values.astype(np.float32)).to(self.device)
+            torch.cuda.current_stream().synchronize()     # the table is in place before any stream of a later call reads it
+
+    @property
+    def body_rows(self):
+        """Host copy ``[B, 9]`` float32 of the skeleton table stage 3 reads (larm_vec, uarm_vec, uarm_orig_rh per stream)."""
+        return self.bodies[: self.B].cpu().numpy()
 
     # ---- device path -----------------------------------------------------------------------------------
     def _lstm_args(self, nF, frame0, sf, masks):
@@ -590,10 +634,10 @@ class BatchedEstimator:
                     "ape_features")
 
         def stage3(stream_ptr):
-            N.check(lib.ape_fk_reduce(N.ptr(self.preds), self.pred_ring, N.ptr(self.yy_m), N.ptr(self.yy_s), N.ptr(self.body),
-                                      self.target, self.O, B, nF, frame0, N.ptr(sf), self.n, self.smooth,
-                                      N.ptr(self.msg), N.ptr(self.samples), N.ptr(self.std), None, N.ptr(self.status), stream_ptr),
-                    "ape_fk_reduce")
+            N.check(lib.ape_fk_reduce_bodies(N.ptr(self.preds), self.pred_ring, N.ptr(self.yy_m), N.ptr(self.yy_s),
+                                             N.ptr(self.bodies), 9, self.target, self.O, B, nF, frame0, N.ptr(sf), self.n, self.smooth,
+                                             N.ptr(self.msg), N.ptr(self.samples), N.ptr(self.std), None, N.ptr(self.status),
+                                             stream_ptr), "ape_fk_reduce_bodies")
 
         if self.pipeline and self._pipe is None and layer_ms is None and trace is None and not _plain:
             # buffer set of this call: lane (stream + workspace) = call & 1; with lanes each workspace's two copies of layer 0's

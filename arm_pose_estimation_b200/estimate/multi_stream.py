@@ -63,6 +63,12 @@ class MultiStreamEstimator:
         """One stream reconnected: its next row starts a fresh window; the others are not disturbed."""
         self._frames[b] = 0
 
+    def set_bonemap(self, b, bonemap):
+        """Stream ``b`` gets its own skeleton (the reference's per-socket ``bonemap``, estimator.py:57-68): the engine's
+        ``set_bonemap``, which applies from the next tick on.  A new user on a stream is ``reset_stream(b); set_bonemap(b, bm)``:
+        from then on the stream sees exactly what a single-stream estimator built with ``bonemap=bm`` would produce."""
+        self._engine.set_bonemap(b, bonemap)
+
     def get_last_msg(self, b):
         return self._last_msg[b]
 

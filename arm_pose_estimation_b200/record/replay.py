@@ -112,12 +112,14 @@ def pad_recordings(recordings):
     return out, lengths
 
 
-def relabel_recordings(recordings, make_estimator, frames_per_call=16, keep_samples=False, masks=None):
+def relabel_recordings(recordings, make_estimator, frames_per_call=16, keep_samples=False, masks=None, bonemaps=None):
     """Offline relabelling: ``recordings`` = list of ``[frames_i, ncols]`` arrays (or one ``[R, F, ncols]`` array);
     ``make_estimator(n_streams, frames_per_call)`` returns a ``BatchedEstimator``.  Returns a list of dicts with
     ``msg [frames_i, 25]``, ``std [frames_i, 6]`` (and ``samples`` if asked).  The next calls are staged and enqueued while call k runs.
     ``masks``: explicit dropout masks ``[R, F, L-1, T, n, H]`` for an estimator built with ``MASK_INJECTED`` (parity runs); for a
-    feed-forward model (``DropoutFF`` / ``DropoutFF2D``) its output-dropout masks ``[R, F, n, H]``."""
+    feed-forward model (``DropoutFF`` / ``DropoutFF2D``) its output-dropout masks ``[R, F, n, H]``.  ``bonemaps``: one skeleton per
+    recording (R entries for ``body_measurements_rows``: recordings of different subjects), set on the estimator before its first
+    call; ``None`` keeps the estimator's own."""
     if isinstance(recordings, np.ndarray) and recordings.ndim == 3:
         rows, lengths = np.asarray(recordings, dtype=np.float32), np.full(len(recordings), recordings.shape[1], np.int64)
     else:
@@ -127,6 +129,8 @@ def relabel_recordings(recordings, make_estimator, frames_per_call=16, keep_samp
         return [dict(msg=np.zeros((0, 25)), std=np.zeros((0, 6))) for _ in range(R)]
     be = make_estimator(R, min(frames_per_call, F))
     be.reset()
+    if bonemaps is not None:
+        be.set_bonemaps(bonemaps)
     msg = np.empty((R, F, 25), np.float32)
     std = np.empty((R, F, 6), np.float32)
     samples = np.empty((R, F, be.S, 6), np.float32) if keep_samples else None

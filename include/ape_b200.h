@@ -285,6 +285,16 @@ int ape_dense_act(const float* wt, const float* bias, const float* x, float* y, 
 int ape_fk_reduce(const float* preds, int pred_ring, const float* yy_m, const float* yy_s, const float* body9,
                   int target, int O, int B, int nF, int frame0, const int32_t* stream_frames, int n_samples, int smooth,
                   float* msg, float* samples, float* stdev, float* est_rows, int32_t* status, void* stream);
+/*
+ * ape_fk_reduce with one skeleton PER STREAM (the reference gives every estimator its own bonemap, estimator.py:57-68):
+ *   bodies       [B][body_stride] float32, row b = the nine floats of body9 for stream b (the local index of this launch);
+ *                body_stride 0: one row for every stream, which is ape_fk_reduce itself (the same kernel and arithmetic)
+ * Every other argument and output is that of ape_fk_reduce.  A null bodies, a negative stride or a stride of 1 to 8 returns
+ * APE_ERR_BAD_ARG before any CUDA call.  Rows of idle streams (stream_frames[b] < 0) are not used.
+ */
+int ape_fk_reduce_bodies(const float* preds, int pred_ring, const float* yy_m, const float* yy_s, const float* bodies,
+                         int body_stride, int target, int O, int B, int nF, int frame0, const int32_t* stream_frames, int n_samples,
+                         int smooth, float* msg, float* samples, float* stdev, float* est_rows, int32_t* status, void* stream);
 
 /*
  * compose_msg.msg_from_nn_targets_est (compose_msg.py:13-108) on rows that already hold quaternions + origins:
@@ -356,6 +366,13 @@ int ape_pipeline_fence(ape_pipeline* p, void* stream);         /* later submits 
 /* The pipeline's CUDA streams (which: 0 side, 1 lane 0, 2 lane 1, 3 copy) as cudaStream_t, for a caller that orders its own work
    against one of them; the pipeline keeps owning them.  APE_ERR_BAD_ARG for a null pointer or another `which`. */
 int ape_pipeline_stream(ape_pipeline* p, int which, void** stream);
+/*
+ * Per-stream skeletons for stage 3: every call submitted after this returns runs ape_fk_reduce_bodies on `bodies` ([B][body_stride]
+ * float32 on the device, body_stride 0 or >= 9); a null `bodies` goes back to desc.body9.  The call does not synchronise and the
+ * pipeline copies nothing: the caller must not overwrite a table that submitted calls may still read (ape_pipeline_sync first).
+ * APE_ERR_BAD_ARG for a null p, a negative stride or a stride of 1 to 8.
+ */
+int ape_pipeline_set_bodies(ape_pipeline* p, const float* bodies, int body_stride);
 
 /* ---- host self-check hooks (tests only; one row per call, never used by the product path) ------ */
 /* The __host__ __device__ row math of the kernels, compiled for the host so a CPU-only box can pin it. */
