@@ -606,12 +606,9 @@ static int tc_kgx(int layer, int I, int H) { return layer == 0 ? ape_pack_kin_pa
 static size_t tc_layer_bytes(int layer, int I, int H) {
     return (size_t)2 * (H / 32) * (tc_kgx(layer, I, H) + H / 8) * 64 * 16 + (size_t)4 * H * 4;
 }
-// fp16 output-layer tiles (TcLayerArgs::Wo16) after the layers: 2 CTAs x [H/8][16 | 32 (H = 256) columns][8] halfs
-static size_t tc_wo16_bytes(int H) { return (size_t)2 * (H / 8) * (H > 128 ? 32 : 16) * 16; }
-// bytes of layer l in the single-pass blob (weights_tc) or in the split-precision blob (weights_tcx: per layer the pieces of
-// ape_lstm_tcx.cu, H = 256 ape_lstm_tcxs.cu, then the kernel's output-layer tiles)
+// bytes of layer l in the single-pass blob (weights_tc) or in the split-precision blob (weights_tcx, ape_lstm_tc_args.cuh: tcx_blob)
 static size_t blob_layer_bytes(bool split, int layer, int I, int H) {
-    return !split ? tc_layer_bytes(layer, I, H) : H == 256 ? ape::tcxs::layer_bytes(layer, I) : ape::tcx::layer_bytes(layer, I);
+    return split ? ape::tcx_blob::layer_bytes(H, layer, I) : tc_layer_bytes(layer, I, H);
 }
 
 // bytes of the fp16 weight blob of the tensor-core path: per layer the two CTAs' weight tiles, then the scaled bias; then the
@@ -620,7 +617,7 @@ extern "C" int ape_lstm_tc_blob_bytes(int I, int H, int L, int64_t* bytes) {
     if (!bytes || I < 1 || H < 32 || H % 32 != 0 || L < 1) return APE_ERR_BAD_ARG;
     int64_t total = 0;
     for (int l = 0; l < L; ++l) total += (int64_t)tc_layer_bytes(l, I, H);
-    total += (int64_t)tc_wo16_bytes(H);
+    total += (int64_t)ape::tc::wo16_bytes(H);
     if (L >= 3) total += (int64_t)(L - 1) * (int64_t)ape::tcw::layer_bytes(H);   // wavefront kernel's pieces of layers >= 1 (H = 128)
     *bytes = total;
     return APE_OK;
@@ -635,6 +632,24 @@ extern "C" int ape_mc_lstm_tc_supported(int I, int H, int L, int O) {
 // shapes of the split-precision kernels (tc_flags == 3)
 static bool split_supported(int I, int H, int L, int O) {
     return L >= 2 && I >= 1 && O >= 1 && (H == 256 ? ape::tcxs::supported(H, I, O) : ape::tcx::supported(H, I, O));
+}
+
+// The small-batch cluster kernels (tc_flags == 4: ape_lstm_tcl.cu; tc_flags == 5: ape_lstm_tcxl.cu at H = 128, ape_lstm_tcxsl.cu at
+// H = 256) run every layer of a call in one launch, one cluster per 128 rows (E x n_samples), up to 64 clusters.
+constexpr long long CLUSTER_MAX_ROWS = (long long)ape::tc::CLUSTER_ROWS * 64;
+static bool cluster_rows_fit(int H, long long E, int n_samples) {
+    return (H == 128 || H == 256) && E >= 0 && n_samples >= 1 && E * n_samples <= CLUSTER_MAX_ROWS;
+}
+static bool cluster_supported(int I, int H, int L, int T, int O, long long E, int n_samples) {
+    return cluster_rows_fit(H, E, n_samples) && L >= 2 && L <= ape::tc::CLUSTER_MAX_L && T >= 1 && T <= 40 && I >= 1 &&
+           ape_pack_kin_pad(0, I, H) <= H && O >= 1 && O <= (H > 128 ? 32 : 16);
+}
+// Workspace of a cluster launch: per cluster the exchange buffer of h_t [2][planes][H/8][128] and two layer sequences
+// [2][T][planes][H/8][128] (planes: 1, split precision 2 - hi and lo), for every cluster of the largest call (rows), + 256 for the alignment
+static size_t cluster_bytes(int H, int T, size_t planes) { return (size_t)(2 + 2 * T) * planes * (H / 8) * ape::tc::CLUSTER_ROWS * 16; }
+static size_t cluster_workspace_bytes(int H, int T, long long rows, size_t planes) {
+    const long long clusters = rows <= 0 ? 1 : (rows + ape::tc::CLUSTER_ROWS - 1) / ape::tc::CLUSTER_ROWS;
+    return cluster_bytes(H, T, planes) * (size_t)clusters + 256;
 }
 
 // Workspace layout of the tensor-core path, computed from the LARGEST call that will use the workspace (ws_E) so that calls of
@@ -664,9 +679,10 @@ static TcWsLayout tc_ws_layout(bool split, int H, int L, int T, long long E, int
     const int n_u1 = L - 2 + (all_steps ? 1 : 0);
     const size_t planes = split ? 2 : 1;
     w.total = 2 * w.scratch_region + 2 * planes * w.u0 + (size_t)(n_u1 > 2 ? 2 : (n_u1 < 0 ? 0 : n_u1)) * planes * w.u1 + 512;
-    // the small-batch cluster kernel (tc_flags == 4) keeps its exchange buffers where the layer kernels keep their units: one set per cluster
-    if (!split && !all_steps && (H == 128 || H == 256) && E * n_samples <= 128LL * 64) {
-        const size_t need = 2 * w.scratch_region + ape::tcl::workspace_bytes(H, T, E * n_samples) + 512;
+    // the small-batch cluster kernel (tc_flags == 4) keeps its exchange buffers where the layer kernels keep their units: one set per
+    // cluster (sized for every call whose rows fit a launch: the query's other arguments do not enter)
+    if (!split && !all_steps && cluster_rows_fit(H, E, n_samples)) {
+        const size_t need = 2 * w.scratch_region + cluster_workspace_bytes(H, T, E * n_samples, 1) + 512;
         if (need > w.total) w.total = need;
     }
     return w;
@@ -690,7 +706,7 @@ extern "C" int ape_mc_lstm_tc_workspace_bytes_all_steps(int I, int H, int L, int
 // The split-precision queries: the tcx_* symbols answer for the H = 128 kernel, the tcxs_* symbols for the H = 256 one.
 static int split_blob_query(int kernel_H, int I, int H, int L, int64_t* bytes) {
     if (!bytes || H != kernel_H || !split_supported(I, H, L, 1)) return APE_ERR_BAD_ARG;
-    int64_t total = (int64_t)(H == 256 ? ape::tcxs::wo16_bytes() : ape::tcx::wo16_bytes());
+    int64_t total = (int64_t)ape::tc::wo16_bytes(H);
     for (int l = 0; l < L; ++l) total += (int64_t)blob_layer_bytes(true, l, I, H);
     *bytes = total;
     return APE_OK;
@@ -746,35 +762,86 @@ extern "C" int ape_mc_lstm_tc_launch_count(const ape_lstm_args* g, int* launches
     return APE_OK;
 }
 
-// Workspace of the split-precision small-batch kernel (tc_flags == 5): the exchange buffer and layer sequences (hi and lo) of one
-// cluster per 128 rows of the largest call
-extern "C" int ape_mc_lstm_tcxl_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
+// Workspace of the split-precision small-batch kernels (tc_flags == 5): the exchange buffer and layer sequences (hi and lo) of one
+// cluster per 128 rows of the largest call.  The tcxl symbol answers for the H = 128 kernel, the tcxsl symbol for the H = 256 one.
+static int cluster_workspace_query(int kernel_H, int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
     if (!bytes || T < 1 || E < 0 || n_samples < 1) return APE_ERR_BAD_ARG;
-    if (!ape::tcxl::supported(H, I, L, T, O, E, n_samples)) return APE_ERR_UNSUPPORTED;
-    *bytes = ape::tcxl::workspace_bytes(T, (long long)E * n_samples);
+    if (H != kernel_H || !cluster_supported(I, H, L, T, O, E, n_samples)) return APE_ERR_UNSUPPORTED;
+    *bytes = cluster_workspace_bytes(H, T, (long long)E * n_samples, 2);
     return APE_OK;
 }
+extern "C" int ape_mc_lstm_tcxl_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
+    return cluster_workspace_query(128, I, H, L, T, O, E, n_samples, bytes);
+}
+extern "C" int ape_mc_lstm_tcxsl_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
+    return cluster_workspace_query(256, I, H, L, T, O, E, n_samples, bytes);
+}
 
-// tc_flags == 5: every layer of a call of <= 8192 rows of a split-precision H = 128 model in ONE launch (csrc/ape_lstm_tcxl.cu).  Every
-// refusal comes before the first CUDA call.
-static int tcxl_call(const ape_lstm_args* g, cudaStream_t st) {
+// The argument block of a cluster kernel for the call `g`: the layers of `blob` (single pass: weights_tc, each layer closed by its
+// scaled bias; split: weights_tcx) and the exchange buffers of every cluster in `workspace`
+static ape::tc::ClusterArgs cluster_args(const ape_lstm_args* g, bool split, const uint8_t* blob, void* workspace) {
+    ape::tc::ClusterArgs a{};
+    const int H = g->H;
+    const uint8_t* p = blob;
+    for (int l = 0; l < g->L; ++l) {
+        a.W[l] = p;
+        a.kgx[l] = tc_kgx(l, g->I, H);
+        p += blob_layer_bytes(split, l, g->I, H);
+        if (!split) a.bias_s[l] = (const float*)(p - (size_t)4 * H * 4);
+    }
     const long long E = (long long)g->B * g->nF;
-    if (g->h0 || g->all_steps || g->layer_begin != 0 || g->layer_end != 0) return APE_ERR_UNSUPPORTED;
-    if (!ape::tcxl::supported(g->H, g->I, g->L, g->T, g->O, E, g->n_samples)) return APE_ERR_UNSUPPORTED;
-    if (!g->weights_tcx || !g->workspace || (g->ws_E != 0 && g->ws_E < E)) return APE_ERR_BAD_ARG;
-    if (E == 0) return APE_OK;
-    ape::LayerTimer timer(g->layer_ms, g->L, st);              // the one launch is reported as layer 0's time
+    a.L = g->L; a.T = g->T; a.I = g->I; a.E = (int)E; a.n = g->n_samples; a.nF = g->nF; a.frame0 = g->frame0; a.feat_ring = g->feat_ring;
+    a.dense = g->x_dense != nullptr;
+    a.in = g->x_dense ? g->x_dense : g->feat_ring_buf;
+    a.stream_frames = g->stream_frames;
+    a.mask_mode = g->mask_mode; a.masks = g->masks;
+    a.rk = ape::philox_round_keys(g->philox_seed);
+    a.stream_id0 = g->stream_id0;
+    a.keep_thr16 = ape::keep_threshold16(g->dropout_p);
+    a.scale = g->mask_mode == APE_MASK_NONE ? 1.0f : 1.0f / (1.0f - g->dropout_p);
+    const size_t planes = split ? 2 : 1;
+    char* ws = (char*)(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
+    a.hx = (uint4*)ws;
+    a.seq = (uint4*)(ws + 2 * planes * (H / 8) * ape::tc::CLUSTER_ROWS * 16);
+    a.ws_stride = cluster_bytes(H, g->T, planes) / 16;
+    a.Wo16 = p;                                                // the output-layer tiles follow the last layer
+    a.bo = g->weights + ape_pack_out_offset(g->I, H, g->L) + (size_t)g->O * H;
+    a.O = g->O;
+    a.preds = g->preds; a.pred_ring = g->pred_ring;
+    a.stamps = (!split && g->trace && g->trace_layer == -2) ? (long long*)g->trace : nullptr;
+    return a;
+}
+
+// one launch of a cluster kernel for all layers of the call `g`, reported as layer 0's time
+static int cluster_launch(const ape_lstm_args* g, bool split, const uint8_t* blob, void* workspace, cudaStream_t st) {
+    const ape::tc::ClusterArgs a = cluster_args(g, split, blob, workspace);
+    const int clusters = (int)(((long long)a.E * a.n + ape::tc::CLUSTER_ROWS - 1) / ape::tc::CLUSTER_ROWS);
+    ape::LayerTimer timer(g->layer_ms, g->L, st);
     int rc = timer.start();
-    if (rc == APE_OK) rc = ape::tcxl::run(g, (const uint8_t*)g->weights_tcx, g->workspace, st);
+    if (rc == APE_OK) rc = !split ? ape::tcl::run(g->H, a, clusters, st) : g->H == 256 ? ape::tcxsl::run(a, clusters, st)
+                                                                                       : ape::tcxl::run(a, clusters, st);
     if (rc == APE_OK) rc = timer.mark(g->L);
     return rc == APE_OK ? timer.finish() : rc;
+}
+
+// tc_flags == 5: every layer of a call of <= 8192 rows of a split-precision model in ONE launch of the small-batch kernel for kernel_H
+// (ape_lstm_tcxl.cu: ape_mc_lstm_tc, H = 128; ape_lstm_tcxsl.cu: ape_mc_lstm_tcxsl, H = 256).  Every refusal comes before the first
+// CUDA call; then `available` (or null) may refuse a device that cannot run the kernel.
+static int split_cluster_call(const ape_lstm_args* g, int kernel_H, cudaStream_t st, int (*available)()) {
+    const long long E = (long long)g->B * g->nF;
+    if (g->h0 || g->all_steps || g->layer_begin != 0 || g->layer_end != 0) return APE_ERR_UNSUPPORTED;
+    if (g->H != kernel_H || !cluster_supported(g->I, g->H, g->L, g->T, g->O, E, g->n_samples)) return APE_ERR_UNSUPPORTED;
+    if (!g->weights_tcx || !g->workspace || (g->ws_E != 0 && g->ws_E < E)) return APE_ERR_BAD_ARG;
+    if (E == 0) return APE_OK;
+    const int rc = available ? available() : APE_OK;
+    return rc == APE_OK ? cluster_launch(g, true, (const uint8_t*)g->weights_tcx, g->workspace, st) : rc;
 }
 
 extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
     using namespace ape;
     int rc = check_lstm_args(g);                               // (h0 / c0: both or neither, and n_samples == 1)
     if (rc != APE_OK) return rc;
-    if (g->tc_flags == 5) return tcxl_call(g, (cudaStream_t)stream);
+    if (g->tc_flags == 5) return split_cluster_call(g, 128, (cudaStream_t)stream, nullptr);
     // an initial state runs on the one-layer kernels (tc_flags 0 and 1) and on the H = 256 split-precision kernel; the wavefront,
     // small-batch and H = 128 split-precision kernels take none
     if (g->h0 && (g->tc_flags == 2 || (g->tc_flags == 3 && g->H != 256) || g->tc_flags == 4)) return APE_ERR_UNSUPPORTED;
@@ -791,7 +858,21 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
     const long long E = (long long)g->B * g->nF;
     if (E == 0) return APE_OK;
     if (!g->workspace || (g->ws_E != 0 && g->ws_E < E)) return APE_ERR_BAD_ARG;
+    const int l_begin = (g->layer_begin == 0 && g->layer_end == 0) ? 0 : g->layer_begin;
+    const int l_end = (g->layer_begin == 0 && g->layer_end == 0) ? g->L : g->layer_end;
+    if (l_begin < 0 || l_end > g->L || l_begin >= l_end) return APE_ERR_BAD_ARG;
+    if (g->tc_flags < 0 || g->tc_flags > 5) return APE_ERR_BAD_ARG;
     cudaStream_t st = (cudaStream_t)stream;
+    const bool all_steps = g->all_steps != 0;
+    const TcWsLayout wl = tc_ws_layout(split, g->H, g->L, g->T, g->ws_E > 0 ? g->ws_E : E, g->n_samples, all_steps);
+    char* wsp = (char*)(((uintptr_t)g->workspace + 255) & ~(uintptr_t)255);
+    if (g->tc_flags == 4) {
+        // small-batch kernel: every layer of a call of <= 8192 rows in ONE launch, one 8-CTA cluster per 128 rows (csrc/ape_lstm_tcl.cu),
+        // its buffers behind the scratch regions
+        if (l_begin != 0 || l_end != g->L || all_steps || !cluster_supported(g->I, g->H, g->L, g->T, g->O, E, g->n_samples))
+            return APE_ERR_UNSUPPORTED;
+        return cluster_launch(g, false, blob, wsp + 2 * wl.scratch_region, st);
+    }
     int dev = 0, sm_count = 0;
     APE_CUDA_TRY(cudaGetDevice(&dev));
     APE_CUDA_TRY(cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev));
@@ -800,34 +881,10 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
     const long long rows = E * g->n_samples;
     const int rpc0 = tc_rpc0(split, E);
     const int tiles0 = (int)((E + 2 * rpc0 - 1) / (2 * rpc0)), tiles1 = (int)((rows + 255) / 256);
-    const bool all_steps = g->all_steps != 0;
-    const TcWsLayout wl = tc_ws_layout(split, H, g->L, g->T, g->ws_E > 0 ? g->ws_E : E, g->n_samples, all_steps);
-    char* wsp = (char*)(((uintptr_t)g->workspace + 255) & ~(uintptr_t)255);
     // per-CTA cell-state scratch at the front (a position that does not depend on the call's size)
     char* scratch = wsp;
     if (wl.scratch_region && sm_count > TC_MAX_SMS) return APE_ERR_UNSUPPORTED;
     wsp += 2 * wl.scratch_region;
-    const int l_begin = (g->layer_begin == 0 && g->layer_end == 0) ? 0 : g->layer_begin;
-    const int l_end = (g->layer_begin == 0 && g->layer_end == 0) ? g->L : g->layer_end;
-    if (l_begin < 0 || l_end > g->L || l_begin >= l_end) return APE_ERR_BAD_ARG;
-    if (g->tc_flags < 0 || g->tc_flags > 5) return APE_ERR_BAD_ARG;
-    if (g->tc_flags == 4) {
-        // small-batch kernel: every layer of a call of <= 128 rows in ONE launch of one 8-CTA cluster (csrc/ape_lstm_tcl.cu)
-        if (l_begin != 0 || l_end != g->L || g->L > 4) return APE_ERR_UNSUPPORTED;
-        const uint8_t* lw[4] = {};
-        const float* lb[4] = {};
-        const uint8_t* p = blob;
-        for (int l = 0; l < g->L; ++l) {
-            lw[l] = p;
-            p += tc_layer_bytes(l, g->I, g->H);
-            lb[l] = (const float*)(p - (size_t)4 * g->H * 4);
-        }
-        LayerTimer timer(g->layer_ms, g->L, st);               // the one launch is reported as layer 0's time
-        rc = timer.start();
-        if (rc == APE_OK) rc = ape::tcl::run(g, lw, lb, p, wsp, st);
-        if (rc == APE_OK) rc = timer.mark(g->L);
-        return rc == APE_OK ? timer.finish() : rc;
-    }
     // SMs the launches of layers >= 1 leave free (a whole number of SM pairs): a concurrent stage 1 + layer 0 of the NEXT call - a few
     // CTAs on a high-priority stream - then never has to wait for a persistent launch to retire CTAs
     if (g->reserve_sms < 0 || g->reserve_sms > sm_count - 2) return APE_ERR_BAD_ARG;
@@ -847,7 +904,7 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
     };
     const uint8_t* wo16 = layer_w(g->L);                                    // the fp16 output-layer tile sits after all layers,
     const size_t ww_layer = !split && g->L >= 3 ? tcw::layer_bytes(H) : 0;  // ... then the wavefront kernel's pieces of layers 1 .. L-1
-    const uint8_t* ww = wo16 + tc_wo16_bytes(H);
+    const uint8_t* ww = wo16 + tc::wo16_bytes(H);
     const float scale = g->mask_mode == APE_MASK_NONE ? 1.0f : 1.0f / (1.0f - g->dropout_p);
     auto layer_args = [&](int l) {
         const bool last = l == g->L - 1;
@@ -921,41 +978,23 @@ extern "C" int ape_mc_lstm_tc(const ape_lstm_args* g, void* stream) {
     return rc == APE_OK ? timer.finish() : rc;
 }
 
-// Workspace of the H = 256 split-precision small-batch kernel (ape_mc_lstm_tcxsl): the exchange buffer and layer sequences (hi and lo)
-// of one 16-CTA cluster per 128 rows of the largest call
-extern "C" int ape_mc_lstm_tcxsl_workspace_bytes(int I, int H, int L, int T, int O, int E, int n_samples, uint64_t* bytes) {
-    if (!bytes || T < 1 || E < 0 || n_samples < 1) return APE_ERR_BAD_ARG;
-    if (!ape::tcxsl::supported(H, I, L, T, O, E, n_samples)) return APE_ERR_UNSUPPORTED;
-    *bytes = ape::tcxsl::workspace_bytes(T, (long long)E * n_samples);
-    return APE_OK;
-}
-
 extern "C" int ape_mc_lstm_tcxsl_max_active_clusters(int* clusters) {
     if (!clusters) return APE_ERR_BAD_ARG;
     *clusters = 0;
     return ape::tcxsl::max_active_clusters(clusters);
 }
 
+// a device that cannot hold one 16-CTA cluster of the H = 256 split-precision small-batch kernel refuses the call
+static int tcxsl_available() {
+    int clusters = 0;
+    const int rc = ape::tcxsl::max_active_clusters(&clusters);
+    return rc != APE_OK ? rc : clusters < 1 ? APE_ERR_UNSUPPORTED : APE_OK;
+}
+
 // Every layer of a call of <= 8192 rows of a split-precision H = 256 model in ONE launch (csrc/ape_lstm_tcxsl.cu), tc_flags == 5.
-// Every refusal comes before the first CUDA call; then a device that cannot hold one 16-CTA cluster of the kernel refuses the call.
 extern "C" int ape_mc_lstm_tcxsl(const ape_lstm_args* g, void* stream) {
-    using namespace ape;
-    int rc = check_lstm_args(g);
+    const int rc = ape::check_lstm_args(g);
     if (rc != APE_OK) return rc;
     if (g->tc_flags != 5) return APE_ERR_BAD_ARG;
-    const long long E = (long long)g->B * g->nF;
-    if (g->h0 || g->all_steps || g->layer_begin != 0 || g->layer_end != 0) return APE_ERR_UNSUPPORTED;
-    if (!tcxsl::supported(g->H, g->I, g->L, g->T, g->O, E, g->n_samples)) return APE_ERR_UNSUPPORTED;
-    if (!g->weights_tcx || !g->workspace || (g->ws_E != 0 && g->ws_E < E)) return APE_ERR_BAD_ARG;
-    if (E == 0) return APE_OK;
-    int clusters = 0;
-    rc = tcxsl::max_active_clusters(&clusters);
-    if (rc != APE_OK) return rc;
-    if (clusters < 1) return APE_ERR_UNSUPPORTED;
-    cudaStream_t st = (cudaStream_t)stream;
-    LayerTimer timer(g->layer_ms, g->L, st);                   // the one launch is reported as layer 0's time
-    rc = timer.start();
-    if (rc == APE_OK) rc = tcxsl::run(g, (const uint8_t*)g->weights_tcx, g->workspace, st);
-    if (rc == APE_OK) rc = timer.mark(g->L);
-    return rc == APE_OK ? timer.finish() : rc;
+    return split_cluster_call(g, 256, (cudaStream_t)stream, tcxsl_available);
 }

@@ -7,6 +7,7 @@
 #pragma once
 #include "ape_f32x2.cuh"
 #include "ape_common.cuh"
+#include "ape_lstm_pack.h"
 #include "ape_umma.cuh"
 
 namespace ape {
@@ -112,6 +113,18 @@ __device__ __forceinline__ void lstm_cell(float pi, float pf, float pg, float po
     h = (1.0f - ec) * rcp_approx((1.0f + eo) * (1.0f + ec));
 }
 
+// Split-precision kernels: accumulator -> ex2 argument (the i, f, o weights are stored halved)
+constexpr float NEG2LOG2E = -2.0f * LOG2E;
+
+// v -> fp16 pair: hi = fp16(v), lo = fp16(v - hi), for two values at once (packed as half2 words)
+__device__ __forceinline__ void split2(float a, float b, uint32_t& hi, uint32_t& lo) {
+    const __half2 h = __floats2half2_rn(a, b);
+    const float2 hf = __half22float2(h);
+    const __half2 l = __floats2half2_rn(a - hf.x, b - hf.y);
+    hi = *reinterpret_cast<const uint32_t*>(&h);
+    lo = *reinterpret_cast<const uint32_t*>(&l);
+}
+
 // Two cells at once in packed fp32 pairs (ape_f32x2.cuh): the same operations as lstm_cell component by component (the clamps and the
 // MUFU calls stay scalar), 15 issue slots for the arithmetic of two cells instead of 30.
 __device__ __forceinline__ void lstm_cell2(F2 pi, F2 pf, F2 pg, F2 po, F2& c, F2& h) {
@@ -134,7 +147,51 @@ __device__ __forceinline__ void lstm_cell2(F2 pi, F2 pf, F2 pg, F2 po, F2& c, F2
 int launch_units_output(const uint4* units, const uint4* units_lo, const float* Wo, float* preds, long long rows, int T, int H, int O,
                         cudaStream_t st);
 
+// bytes of the fp16 output-layer tiles after the last layer of either blob (TcLayerArgs::Wo16), both CTAs
+__host__ __device__ constexpr uint32_t wo16_bytes(int H) { return 2u * (uint32_t)(H / 8) * (H > 128 ? 32u : 16u) * 16u; }
+
+// Argument block of the small-batch cluster kernels (ape_lstm_tcl.cu; split precision: ape_lstm_tcxl.cu, ape_lstm_tcxsl.cu): all layers of
+// a call in one launch, one cluster per CLUSTER_ROWS rows
+constexpr int CLUSTER_ROWS = 128, CLUSTER_MAX_L = 4;
+struct ClusterArgs {
+    const uint8_t* W[CLUSTER_MAX_L];        // layer l of the blob: single pass [cta 2][chunk H/32][kgx + H/8 k-groups][64][8]; split
+                                            // [pair cta 2][chunk H/32][Wx_hi + bias | Wx_lo | Wh_hi | Wh_lo] (tcx_blob)
+    const float* bias_s[CLUSTER_MAX_L];     // single pass: [4H] column 4u + g, 0.5 b (i, f, o), b (g); split: null (the bias is in the blob)
+    int kgx[CLUSTER_MAX_L];
+    int L, T, I, E, n, nF, frame0, feat_ring, dense;
+    const float* in;                        // feature ring [B][feat_ring][I] or dense windows [E][T][I]
+    const int32_t* stream_frames;
+    int mask_mode;
+    const uint8_t* masks;                   // injected: [E][L-1][T][n][H]
+    PhiloxRoundKeys rk;
+    uint32_t stream_id0, keep_thr16;
+    float scale;                            // 1 / (1 - p) (1 with no dropout): applied to a layer's output sequence BEFORE the fp16 rounding
+    uint4* hx;                              // [2][planes][H/8][128] exchange buffer of h_t (operand layout), by step parity
+    uint4* seq;                             // [2][T][planes][H/8][128] a layer's output sequence (the next layer's input), by layer parity
+    size_t ws_stride;                       // uint4s between the hx / seq buffers of consecutive clusters
+    const uint8_t* Wo16;                    // [2][H/8][16 | 32 (H = 256)][8]: fp16(W_o), remainder
+    const float* bo;
+    int O;
+    float* preds;
+    int pred_ring;
+    long long* stamps;                      // single pass, debugging: null, or [L * T][8] globaltimer ns of CTA 0 (tools/tcl_trace.py;
+                                            // ape_lstm_args.trace, trace_layer = -2); split: null
+};
+
 }  // namespace tc
+
+namespace tcx_blob {
+// The split-precision blob (weights_tcx) of tcx, tcxs, tcxl and tcxsl: per layer [pair cta 2][chunk H/32] of four 64-column pieces for an
+// x-part of kgx k-groups - Wx_hi + the bias K step, Wx_lo, Wh_hi, Wh_lo - then the output-layer tiles (tc::wo16_bytes)
+constexpr uint32_t KG_BYTES = 64 * 16;                                                           // one k-group of a piece
+__host__ __device__ constexpr uint32_t p0_bytes(int kgx) { return (uint32_t)(kgx + 2) * KG_BYTES; }   // Wx_hi + bias K step
+__host__ __device__ constexpr uint32_t p1_bytes(int kgx) { return (uint32_t)kgx * KG_BYTES; }         // Wx_lo
+__host__ __device__ constexpr uint32_t ph_bytes(int H) { return (uint32_t)(H / 8) * KG_BYTES; }       // Wh_hi or Wh_lo
+__host__ __device__ constexpr uint32_t chunk_bytes(int H, int kgx) { return p0_bytes(kgx) + p1_bytes(kgx) + 2 * ph_bytes(H); }
+inline size_t layer_bytes(int H, int layer, int I) {                                            // both CTAs
+    return (size_t)2 * (H / 32) * chunk_bytes(H, ape_pack_kin_pad(layer, I, H) / 8);
+}
+}  // namespace tcx_blob
 
 namespace tcs {
 // streamed-weights kernel (ape_lstm_tcs.cu)
@@ -153,18 +210,13 @@ int launch_pair(const tc::TcLayerArgs& a, const tc::TcLayerArgs& b, int sm_count
 
 namespace tcl {
 // small-batch kernel (ape_lstm_tcl.cu): all layers of a call in one launch, one cluster of 8 CTAs per 128 rows (hidden units split
-// across the cluster, h_t exchanged once per step); up to 64 clusters
-bool supported(int H, int I, int L, int O, long long E, int n);
-size_t workspace_bytes(int H, int T, long long rows);     // rows = E * n_samples of the largest call (one cluster per 128 rows)
-int run(const ape_lstm_args* g, const uint8_t* const* layer_w, const float* const* layer_bias, const uint8_t* wo16, void* workspace,
-        cudaStream_t st);
+// across the cluster, h_t exchanged once per step), H = 128 / 256
+int run(int H, const tc::ClusterArgs& a, int clusters, cudaStream_t st);
 }  // namespace tcl
 
 namespace tcx {
 // split-precision kernel (ape_lstm_tcx.cu): every operand an fp16 pair hi + lo, three tensor-core passes per product, ex2 / rcp cell
 bool supported(int H, int I, int O);
-size_t layer_bytes(int layer, int I);            // bytes of one layer's pieces (TcLayerArgs::Ww), both CTAs
-size_t wo16_bytes();                             // bytes of the output-layer tiles after the last layer (TcLayerArgs::Wo16), both CTAs
 size_t scratch_bytes(int sm_count);              // per-CTA cell-state scratch of one launch
 int launch_layer(const tc::TcLayerArgs& a, int sm_count, cudaStream_t st);
 }  // namespace tcx
@@ -173,8 +225,6 @@ namespace tcxs {
 // split-precision kernel for H = 256 (ape_lstm_tcxs.cu): the arithmetic and blob layout of tcx, h_t staged through L2 into
 // single-buffered TMEM operands
 bool supported(int H, int I, int O);
-size_t layer_bytes(int layer, int I);
-size_t wo16_bytes();
 size_t scratch_bytes(int sm_count);              // per-CTA cell state and h_t staging of one launch
 int launch_layer(const tc::TcLayerArgs& a, int sm_count, cudaStream_t st);    // a.h0 / a.c0: the state variant
 }  // namespace tcxs
@@ -182,17 +232,13 @@ int launch_layer(const tc::TcLayerArgs& a, int sm_count, cudaStream_t st);    //
 namespace tcxl {
 // split-precision small-batch kernel (ape_lstm_tcxl.cu, H = 128): all layers of a call in one launch, one 8-CTA cluster per 128 rows,
 // the arithmetic of tcx on the tcx blob
-bool supported(int H, int I, int L, int T, int O, long long E, int n);
-size_t workspace_bytes(int T, long long rows);             // rows = E * n_samples of the largest call (one cluster per 128 rows)
-int run(const ape_lstm_args* g, const uint8_t* blob, void* workspace, cudaStream_t st);
+int run(const tc::ClusterArgs& a, int clusters, cudaStream_t st);
 }  // namespace tcxl
 
 namespace tcxsl {
 // split-precision small-batch kernel for H = 256 (ape_lstm_tcxsl.cu): all layers of a call in one launch, one 16-CTA cluster per
 // 128 rows, the arithmetic of tcxs on the tcx blob
-bool supported(int H, int I, int L, int T, int O, long long E, int n);
-size_t workspace_bytes(int T, long long rows);             // rows = E * n_samples of the largest call (one cluster per 128 rows)
 int max_active_clusters(int* clusters);                    // 16-CTA clusters of this launch the current device holds at once
-int run(const ape_lstm_args* g, const uint8_t* blob, void* workspace, cudaStream_t st);
+int run(const tc::ClusterArgs& a, int clusters, cudaStream_t st);
 }  // namespace tcxsl
 }  // namespace ape

@@ -30,7 +30,7 @@ namespace tcl {
 
 using tc::tanh_approx;
 
-constexpr int NCTA = 8, ROWS = 128, MAX_L = 4, MAX_CLUSTERS = 64;
+constexpr int NCTA = 8, ROWS = tc::CLUSTER_ROWS;
 // 12 loader warps: three per TMEM lane quarter, each taking every third k-group of its 32 rows (building x_t for a layer >= 1 is 32 L2
 // loads + 32 Philox draws per row at H = 256; with one warp per quarter it took 7.5 - 12 us, twice the rest of a step)
 // 8 epilogue warps: two per TMEM lane quarter, each taking every second k-group (8 units) of its 32 rows' cells
@@ -39,28 +39,6 @@ constexpr int CTRL_WARP = EPI_WARPS + LOAD_WARPS;
 constexpr uint32_t BLK_COLS = 64, KG_BYTES_B = BLK_COLS * 16;    // a weight tile of the blob: [k-group][64 gate columns][8 halfs]
 constexpr uint32_t ACC_COL = 0, X_COL = 128, OUT_COL = 384, TMEM_COLS = 512;
 
-struct Args {
-    const uint8_t* W[MAX_L];        // layer l of the fp16 blob: [cta 2][chunk H/32][kgx + KG k-groups][64][8]
-    const float* bias_s[MAX_L];     // [4H] column 4u + g, 0.5 b (i, f, o), b (g)
-    int kgx[MAX_L];
-    int L, T, I, E, n, nF, frame0, feat_ring, dense;
-    const float* in;                // feature ring [B][feat_ring][I] or dense windows [E][T][I]
-    const int32_t* stream_frames;
-    int mask_mode;
-    const uint8_t* masks;           // injected: [E][L-1][T][n][H]
-    PhiloxRoundKeys rk;
-    uint32_t stream_id0, keep_thr16;
-    float scale;                    // 1 / (1 - p) (1 with no dropout): applied to a layer's output sequence BEFORE the fp16 rounding
-    uint4* hx;                      // [2][H/8][128] exchange buffer of h_t (operand layout), by step parity
-    uint4* seq;                     // [2][T][H/8][128] a layer's output sequence (the next layer's input), by layer parity
-    size_t ws_stride;               // uint4s between the hx / seq buffers of consecutive clusters
-    const uint8_t* Wo16;            // [2][H/8][NO][8]: fp16(W_o), remainder
-    const float* bo;
-    int O;
-    float* preds;
-    int pred_ring;
-    long long* stamps;              // debugging: null, or [L * T][8] globaltimer ns of CTA 0 (tools/tcl_trace.py; ape_lstm_args.trace, trace_layer = -2)
-};
 __device__ __forceinline__ void stamp(long long* st, int step, int ev) {
     if (st) st[step * 8 + ev] = tc::globaltimer_ns();
 }
@@ -68,7 +46,7 @@ __device__ __forceinline__ void stamp(long long* st, int step, int ev) {
 enum { BAR_W = 0, BAR_X = 1, BAR_ACC = 3, BAR_H = 4, BAR_OUT = 5, BAR_COUNT = 6 };
 
 template <int H>
-__global__ void __cluster_dims__(NCTA, 1, 1) __launch_bounds__(THREADS, 1) lstm_small_kernel(const __grid_constant__ Args a) {
+__global__ void __cluster_dims__(NCTA, 1, 1) __launch_bounds__(THREADS, 1) lstm_small_kernel(const __grid_constant__ tc::ClusterArgs a) {
     using namespace umma;
     constexpr int KG = H / 8, NU = H / NCTA, NB = NU / 16, NCOL = 4 * NU;       // this CTA: NU units = NB weight tiles = NCOL gate columns
     constexpr int NO = H > 128 ? 32 : 16;                                      // columns of an output tile
@@ -372,18 +350,7 @@ __global__ void __cluster_dims__(NCTA, 1, 1) __launch_bounds__(THREADS, 1) lstm_
     if (warp == CTRL_WARP) tmem_dealloc<1>(tmem, TMEM_COLS);
 }
 
-bool supported(int H, int I, int L, int O, long long E, int n) {
-    return (H == 128 || H == 256) && L >= 2 && L <= MAX_L && E >= 1 && n >= 1 && E * n <= (long long)ROWS * MAX_CLUSTERS &&
-           ape_pack_kin_pad(0, I, H) <= H && O <= (H > 128 ? 32 : 16);
-}
-
-static size_t cluster_ws_bytes(int H, int T) { return (size_t)(2 + 2 * T) * (H / 8) * ROWS * 16; }      // hx + seq of one cluster
-size_t workspace_bytes(int H, int T, long long rows) {
-    const long long clusters = rows <= 0 ? 1 : (rows + ROWS - 1) / ROWS;
-    return cluster_ws_bytes(H, T) * (size_t)clusters + 256;
-}
-
-template <int H> static int launch_t(const Args& a, int clusters, cudaStream_t st) {
+template <int H> static int launch_t(const tc::ClusterArgs& a, int clusters, cudaStream_t st) {
     constexpr int KG = H / 8, NB = H / NCTA / 16;
     const size_t smem = (size_t)NB * 2 * KG * KG_BYTES_B + (size_t)KG * ROWS * 16 + (size_t)4 * (H / NCTA) * 4 + 64;
     APE_CUDA_TRY(cudaFuncSetAttribute(lstm_small_kernel<H>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -391,37 +358,8 @@ template <int H> static int launch_t(const Args& a, int clusters, cudaStream_t s
     return check_launch();
 }
 
-// all layers of the call `g` (ape_mc_lstm_tc with tc_flags == 4); blob / bias pointers per layer from the fp16 blob `weights_tc`
-int run(const ape_lstm_args* g, const uint8_t* const* layer_w, const float* const* layer_bias, const uint8_t* wo16, void* workspace,
-        cudaStream_t st) {
-    const long long E = (long long)g->B * g->nF;
-    if (!supported(g->H, g->I, g->L, g->O, E, g->n_samples)) return APE_ERR_UNSUPPORTED;
-    if (g->all_steps || g->h0 || g->c0 || g->T > 40 || g->T < 1) return APE_ERR_UNSUPPORTED;
-    Args a{};
-    for (int l = 0; l < g->L; ++l) {
-        a.W[l] = layer_w[l]; a.bias_s[l] = layer_bias[l];
-        a.kgx[l] = l == 0 ? ape_pack_kin_pad(0, g->I, g->H) / 8 : g->H / 8;
-    }
-    a.L = g->L; a.T = g->T; a.I = g->I; a.E = (int)E; a.n = g->n_samples; a.nF = g->nF; a.frame0 = g->frame0; a.feat_ring = g->feat_ring;
-    a.dense = g->x_dense != nullptr;
-    a.in = g->x_dense ? g->x_dense : g->feat_ring_buf;
-    a.stream_frames = g->stream_frames;
-    a.mask_mode = g->mask_mode; a.masks = g->masks;
-    a.rk = philox_round_keys(g->philox_seed);
-    a.stream_id0 = g->stream_id0;
-    a.keep_thr16 = keep_threshold16(g->dropout_p);
-    a.scale = g->mask_mode == APE_MASK_NONE ? 1.0f : 1.0f / (1.0f - g->dropout_p);
-    char* ws = (char*)(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-    a.hx = (uint4*)ws;
-    a.seq = (uint4*)(ws + (size_t)2 * (g->H / 8) * ROWS * 16);
-    a.ws_stride = cluster_ws_bytes(g->H, g->T) / 16;
-    const int clusters = (int)((E * g->n_samples + ROWS - 1) / ROWS);
-    a.Wo16 = wo16;
-    a.bo = g->weights + ape_pack_out_offset(g->I, g->H, g->L) + (size_t)g->O * g->H;
-    a.O = g->O;
-    a.preds = g->preds; a.pred_ring = g->pred_ring;
-    a.stamps = (g->trace && g->trace_layer == -2) ? (long long*)g->trace : nullptr;
-    return g->H == 256 ? launch_t<256>(a, clusters, st) : launch_t<128>(a, clusters, st);
+int run(int H, const tc::ClusterArgs& a, int clusters, cudaStream_t st) {
+    return H == 256 ? launch_t<256>(a, clusters, st) : launch_t<128>(a, clusters, st);
 }
 
 }  // namespace tcl

@@ -51,28 +51,15 @@ constexpr uint32_t SMEM = 2 * A_BYTES + NP * SLOT_BYTES + ONES_BYTES + BAR_BLOCK
 constexpr uint32_t HH_COL = 256, HL_COL = 384, H_COLS = H / 2, TMEM_COLS = 512;
 constexpr size_t CSTATE_FLOATS = (size_t)H * ROWS;         // per CTA: [k-group * 2 + half][row] float4
 static_assert(SMEM <= 227 * 1024, "shared memory budget");
-constexpr float NEG2LOG2E = -2.0f * 1.4426950408889634f;   // accumulator -> ex2 argument (i, f, o weights are stored halved)
+using tc::NEG2LOG2E;
+using tc::split2;
+static_assert(2 * OUT_BYTES == tc::wo16_bytes(H), "the output-layer tiles of the tcx blob");
 
 enum {
     BAR_X_READY = 0, BAR_X_DONE = 1, BAR_ACC_READY = 2, BAR_SLOT_FREE = 4, BAR_H_READY = 6, BAR_W_FULL = BAR_H_READY + NCHL,
     BAR_W_EMPTY = BAR_W_FULL + NFULL, BAR_OUT_READY = BAR_W_EMPTY + NP, BAR_COUNT = BAR_OUT_READY + 1
 };
 static_assert(BAR_COUNT * 8 + 16 <= BAR_BLOCK_BYTES, "barrier block too small");
-
-// bytes of the four pieces of one chunk for an x-part of kgx k-groups
-__host__ __device__ constexpr uint32_t p0_bytes(int kgx) { return (uint32_t)(kgx + 2) * KG_BYTES_B; }
-__host__ __device__ constexpr uint32_t p1_bytes(int kgx) { return (uint32_t)kgx * KG_BYTES_B; }
-constexpr uint32_t PH_BYTES = KG * KG_BYTES_B;
-__host__ __device__ constexpr uint32_t chunk_bytes(int kgx) { return p0_bytes(kgx) + p1_bytes(kgx) + 2 * PH_BYTES; }
-
-// v -> fp16 pair: hi = fp16(v), lo = fp16(v - hi), for two values at once (packed as half2 words)
-__device__ __forceinline__ void split2(float a, float b, uint32_t& hi, uint32_t& lo) {
-    const __half2 h = __floats2half2_rn(a, b);
-    const float2 hf = __half22float2(h);
-    const __half2 l = __floats2half2_rn(a - hf.x, b - hf.y);
-    hi = *reinterpret_cast<const uint32_t*>(&h);
-    lo = *reinterpret_cast<const uint32_t*>(&l);
-}
 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 1)
 lstm_layer_tcx_kernel(const __grid_constant__ TcLayerArgs a) {
@@ -459,7 +446,7 @@ lstm_layer_tcx_kernel(const __grid_constant__ TcLayerArgs a) {
         }
       } else if (warp == TMA_WARP && lane == 0) {
         // =================================== weight-ring producer (one lane per CTA) =====================================
-        const uint32_t p0b = p0_bytes(kgx), p1b = p1_bytes(kgx), cb = chunk_bytes(kgx);
+        const uint32_t p0b = tcx_blob::p0_bytes(kgx), p1b = tcx_blob::p1_bytes(kgx), phb = tcx_blob::ph_bytes(H), cb = tcx_blob::chunk_bytes(H, kgx);
         const uint8_t* Wl = a.Ww + (size_t)rank * NCHL * cb;   // this CTA's half of the layer's pieces
         uint32_t wslot = 0, wphase = 0, gpiece = 0;
         bool wrapped = false;
@@ -479,7 +466,7 @@ lstm_layer_tcx_kernel(const __grid_constant__ TcLayerArgs a) {
                 const uint8_t* c0 = Wl + (size_t)cl * cb;
                 put(c0, p0b);
                 put(c0 + p0b, p1b);
-                if (t > 0) { put(c0 + p0b + p1b, PH_BYTES); put(c0 + p0b + p1b + PH_BYTES, PH_BYTES); }
+                if (t > 0) { put(c0 + p0b + p1b, phb); put(c0 + p0b + p1b + phb, phb); }
             }
         }
         if (has_out) put(a.Wo16 + (size_t)rank * OUT_BYTES, OUT_BYTES);
@@ -493,8 +480,6 @@ lstm_layer_tcx_kernel(const __grid_constant__ TcLayerArgs a) {
 }
 
 bool supported(int Hh, int I, int O) { return Hh == H && ape_pack_kin_pad(0, I, Hh) <= Hh && O <= (int)OUT_N / 2; }
-
-size_t layer_bytes(int layer, int I) { return (size_t)2 * NCHL * chunk_bytes(layer == 0 ? ape_pack_kin_pad(0, I, H) / 8 : KG); }
 
 size_t scratch_bytes(int sm_count) { return (size_t)sm_count * CSTATE_FLOATS * sizeof(float); }
 
@@ -510,8 +495,6 @@ int launch_layer(const TcLayerArgs& a, int sm_count, cudaStream_t st) {
     lstm_layer_tcx_kernel<<<2 * clusters, THREADS, SMEM, st>>>(a);
     return check_launch();
 }
-
-size_t wo16_bytes() { return (size_t)2 * OUT_BYTES; }
 
 }  // namespace tcx
 }  // namespace ape

@@ -54,7 +54,9 @@ constexpr uint32_t HH_COL = 256, HL_COL = 384, TMEM_COLS = 512;
 static_assert(HL_COL + H / 2 <= TMEM_COLS, "two accumulator slots + h_hi + h_lo");
 constexpr size_t CSTATE_FLOATS = (size_t)H * ROWS;         // per CTA: cell state [k-group * 2 + half][row] float4
 constexpr size_t SCRATCH_FLOATS = 2 * CSTATE_FLOATS;       // ... followed by the h_t staging area [chunk][hi, lo][s][row] uint4
-constexpr float NEG2LOG2E = -2.0f * 1.4426950408889634f;   // accumulator -> ex2 argument (i, f, o weights are stored halved)
+using tc::NEG2LOG2E;
+using tc::split2;
+static_assert(2 * OUT_BYTES == tc::wo16_bytes(H), "the output-layer tiles of the tcx blob");
 
 enum {
     BAR_X_READY = 0, BAR_X_DONE = 1, BAR_ACC_READY = 2, BAR_SLOT_FREE = 4, BAR_H_READY = 6, BAR_OUT_READY = 7, BAR_W_FULL = 8,
@@ -62,26 +64,12 @@ enum {
 };
 static_assert(BAR_COUNT * 8 + 16 <= BAR_BLOCK_BYTES, "barrier block too small");
 
-// bytes of the four parts of one chunk for an x-part of kgx k-groups (the layout of ape_lstm_tcx.cu)
-__host__ __device__ constexpr uint32_t p0_bytes(int kgx) { return (uint32_t)(kgx + 2) * KG_BYTES_B; }
-__host__ __device__ constexpr uint32_t p1_bytes(int kgx) { return (uint32_t)kgx * KG_BYTES_B; }
-constexpr uint32_t PH_BYTES = KG * KG_BYTES_B;
-__host__ __device__ constexpr uint32_t chunk_bytes(int kgx) { return p0_bytes(kgx) + p1_bytes(kgx) + 2 * PH_BYTES; }
 // ring pieces per chunk: x-part pieces (Wx_hi, then the same count of Wx_lo) and, for a step with a recurrent half, 2 Wh_hi + 2 Wh_lo
 __host__ __device__ constexpr int x_pieces(int kgx) { return (kgx + PIECE_KG - 1) / PIECE_KG; }
 constexpr int H_PIECES = KG / PIECE_KG;
 // Ring pieces of one chunk of step t.  A step has a recurrent half when t > 0 or, with a caller-supplied initial state, at t = 0
 // too (on h_0).  The producer, both issuers and the peer's forwarder walk the ring by this one count.
 __host__ __device__ constexpr int chunk_pieces(int kgx, int t, bool state) { return 2 * x_pieces(kgx) + (t > 0 || state ? 2 * H_PIECES : 0); }
-
-// v -> fp16 pair: hi = fp16(v), lo = fp16(v - hi), for two values at once (packed as half2 words)
-__device__ __forceinline__ void split2(float a, float b, uint32_t& hi, uint32_t& lo) {
-    const __half2 h = __floats2half2_rn(a, b);
-    const float2 hf = __half22float2(h);
-    const __half2 l = __floats2half2_rn(a - hf.x, b - hf.y);
-    hi = *reinterpret_cast<const uint32_t*>(&h);
-    lo = *reinterpret_cast<const uint32_t*>(&l);
-}
 
 // STATE: a caller-supplied initial state (a.h0, a.c0).  At the start of every tile the epilogue writes h_0 as fp16 pairs into the h
 // buffers step 0 reads and publishes it on BAR_H0_READY; the cell starts from c_0; step 0 runs its recurrent half after the
@@ -544,7 +532,7 @@ lstm_layer_tcxs_kernel(const __grid_constant__ TcLayerArgs a) {
         }
       } else if (warp == TMA_WARP && lane == 0) {
         // =================================== weight-ring producer (one lane per CTA) =====================================
-        const uint32_t p0b = p0_bytes(kgx), p1b = p1_bytes(kgx), cb = chunk_bytes(kgx);
+        const uint32_t p0b = tcx_blob::p0_bytes(kgx), p1b = tcx_blob::p1_bytes(kgx), cb = tcx_blob::chunk_bytes(H, kgx);
         const uint8_t* Wl = a.Ww + (size_t)rank * NCH * cb;    // this CTA's half of the layer's pieces
         uint32_t wslot = 0, wphase = 0, gpiece = 0;
         bool wrapped = false;
@@ -585,8 +573,6 @@ lstm_layer_tcxs_kernel(const __grid_constant__ TcLayerArgs a) {
 
 bool supported(int Hh, int I, int O) { return Hh == H && I >= 1 && ape_pack_kin_pad(0, I, Hh) <= Hh && O >= 1 && O <= (int)OUT_N / 2; }
 
-size_t layer_bytes(int layer, int I) { return (size_t)2 * NCH * chunk_bytes(layer == 0 ? ape_pack_kin_pad(0, I, H) / 8 : KG); }
-
 size_t scratch_bytes(int sm_count) { return (size_t)sm_count * SCRATCH_FLOATS * sizeof(float); }
 
 int launch_layer(const TcLayerArgs& a, int sm_count, cudaStream_t st) {
@@ -603,8 +589,6 @@ int launch_layer(const TcLayerArgs& a, int sm_count, cudaStream_t st) {
     kernel<<<2 * clusters, THREADS, SMEM, st>>>(a);
     return check_launch();
 }
-
-size_t wo16_bytes() { return (size_t)2 * OUT_BYTES; }
 
 }  // namespace tcxs
 }  // namespace ape

@@ -31,65 +31,32 @@
 namespace ape {
 namespace tcxsl {
 
-constexpr int H = 256, KG = H / 8, NCHL = H / 32, NCTA = 16, NU = H / NCTA, NCOL = 4 * NU, ROWS = 128, MAX_L = 4, MAX_CLUSTERS = 64;
+constexpr int H = 256, KG = H / 8, NCHL = H / 32, NCTA = 16, NU = H / NCTA, NCOL = 4 * NU, ROWS = tc::CLUSTER_ROWS;
 // 8 epilogue warps (two per TMEM lane quarter, one k-group = 8 units each), 12 loader warps (three per quarter), one controller warp
 constexpr int EPI_WARPS = 8, LOAD_PARTS = 3, LOAD_WARPS = 4 * LOAD_PARTS, THREADS = (EPI_WARPS + LOAD_WARPS + 1) * 32;
 constexpr int CTRL_WARP = EPI_WARPS + LOAD_WARPS;
 constexpr int PIECE_KG = 16;                               // tcxs's weight pieces: the unit of its MMA order
 constexpr uint32_t KG_BYTES_B = NCOL * 16;                 // one k-group of a 64-column weight piece
-constexpr uint32_t PH_BYTES = KG * KG_BYTES_B;             // Wh_hi or Wh_lo
-__host__ __device__ constexpr uint32_t p0_bytes(int kgx) { return (uint32_t)(kgx + 2) * KG_BYTES_B; }   // Wx_hi + bias K step
-__host__ __device__ constexpr uint32_t p1_bytes(int kgx) { return (uint32_t)kgx * KG_BYTES_B; }         // Wx_lo
-__host__ __device__ constexpr uint32_t chunk_bytes(int kgx) { return p0_bytes(kgx) + p1_bytes(kgx) + 2 * PH_BYTES; }
-constexpr uint32_t W_BYTES = chunk_bytes(KG);              // 130 KB: a slot of a layer >= 1 (the largest)
+constexpr uint32_t W_BYTES = tcx_blob::chunk_bytes(H, KG); // 130 KB: a slot of a layer >= 1 (the largest)
 constexpr uint32_t H_BYTES = KG * ROWS * 16;               // one h operand tile (64 KB)
 constexpr uint32_t ONES_BYTES = 2 * ROWS * 16;             // A operand of the bias K step
 constexpr int NO = 32;                                     // columns of an output tile (O <= 32)
-constexpr uint32_t OT_BYTES = KG * NO * 16;
+constexpr uint32_t OT_BYTES = tc::wo16_bytes(H) / 2;
 constexpr uint32_t BAR_BLOCK_BYTES = 128;                 // the mbarriers, then the TMEM base address tcgen05.alloc writes
 constexpr uint32_t SMEM = W_BYTES + H_BYTES + ONES_BYTES + BAR_BLOCK_BYTES;
 constexpr uint32_t ACC_COL = 0, XH_COL = 64, XL_COL = XH_COL + H / 2, HL_COL = XL_COL + H / 2, OUT_COL = HL_COL + H / 2, TMEM_COLS = 512;
 static_assert(SMEM <= 227 * 1024, "shared memory budget");
 static_assert(ACC_COL + NCOL <= XH_COL && OUT_COL + 2 * NO <= TMEM_COLS, "tensor memory plan");
 static_assert(2 * OT_BYTES <= W_BYTES, "the output tiles take the weights' place");
-constexpr float NEG2LOG2E = -2.0f * 1.4426950408889634f;   // accumulator -> ex2 argument (i, f, o weights are stored halved)
-
-struct Args {
-    const uint8_t* W[MAX_L];        // layer l of the split blob: [pair cta 2][chunk H/32][Wx_hi + bias | Wx_lo | Wh_hi | Wh_lo]
-    int kgx[MAX_L];
-    int L, T, I, E, n, nF, frame0, feat_ring, dense;
-    const float* in;                // feature ring [B][feat_ring][I] or dense windows [E][T][I]
-    const int32_t* stream_frames;
-    int mask_mode;
-    const uint8_t* masks;           // injected: [E][L-1][T][n][H]
-    PhiloxRoundKeys rk;
-    uint32_t stream_id0, keep_thr16;
-    float scale;                    // 1 / (1 - p) (1 with no dropout): applied to a layer's output sequence BEFORE the split
-    uint4* hx;                      // [2][hi | lo][H/8][128] exchange buffer of h_t (operand layout), by step parity
-    uint4* seq;                     // [2][T][hi | lo][H/8][128] a layer's output sequence (the next layer's input), by layer parity
-    size_t ws_stride;               // uint4s between the hx / seq buffers of consecutive clusters
-    const uint8_t* Wo16;            // [2][H/8][32][8]: fp16(W_o), remainder
-    const float* bo;
-    int O;
-    float* preds;
-    int pred_ring;
-};
+using tc::NEG2LOG2E;
+using tc::split2;
 
 enum { BAR_W = 0, BAR_X = 1, BAR_XFREE = 2, BAR_ACC = 3, BAR_H = 4, BAR_HLO = 5, BAR_OUT = 7, BAR_COUNT = 8 };   // BAR_HLO + half
 static_assert(BAR_COUNT * 8 + 16 <= BAR_BLOCK_BYTES, "barrier block too small");
 
-// v -> fp16 pair: hi = fp16(v), lo = fp16(v - hi), for two values at once (ape_lstm_tcxs.cu)
-__device__ __forceinline__ void split2(float a, float b, uint32_t& hi, uint32_t& lo) {
-    const __half2 h = __floats2half2_rn(a, b);
-    const float2 hf = __half22float2(h);
-    const __half2 l = __floats2half2_rn(a - hf.x, b - hf.y);
-    hi = *reinterpret_cast<const uint32_t*>(&h);
-    lo = *reinterpret_cast<const uint32_t*>(&l);
-}
-
 __device__ __forceinline__ uint4 and4(uint4 v, uint4 m) { return make_uint4(v.x & m.x, v.y & m.y, v.z & m.z, v.w & m.w); }
 
-__global__ void __launch_bounds__(THREADS, 1) lstm_small_tcxs_kernel(const __grid_constant__ Args a) {
+__global__ void __launch_bounds__(THREADS, 1) lstm_small_tcxs_kernel(const __grid_constant__ tc::ClusterArgs a) {
     using namespace umma;
     constexpr uint32_t LBO_A = ROWS * 16, LBO_B = KG_BYTES_B, SBO = 128;
 
@@ -142,7 +109,7 @@ __global__ void __launch_bounds__(THREADS, 1) lstm_small_tcxs_kernel(const __gri
         auto pull = [&](int t) { return t + 1 < T || (last_layer && a.preds && rank == 0); };
         // ---- this CTA's slot of layer l -> shared memory (every MMA of the previous layer has completed: see the barrier below) ----
         if (warp == CTRL_WARP && lane == 0) {
-            const uint32_t cb = chunk_bytes(kgx);
+            const uint32_t cb = tcx_blob::chunk_bytes(H, kgx);
             mbar_arrive_expect_tx(&bars[BAR_W], cb);
             bulk_g2s(sW, a.W[l] + ((size_t)(rank & 1) * NCHL + (rank >> 1)) * cb, cb, &bars[BAR_W]);
         }
@@ -329,8 +296,8 @@ __global__ void __launch_bounds__(THREADS, 1) lstm_small_tcxs_kernel(const __gri
             const uint64_t dHh = make_desc(smem_u32(sH), LBO_A, SBO);
             const uint64_t dOnes = make_desc(smem_u32(sOnes), LBO_A, SBO);
             const uint64_t dWxh = make_desc(smem_u32(sW), LBO_B, SBO);                         // Wx_hi, then the bias K step
-            const uint64_t dWxl = desc_advance(dWxh, p0_bytes(kgx));                              // Wx_lo
-            const uint64_t dWhh = desc_advance(dWxl, p1_bytes(kgx)), dWhl = desc_advance(dWhh, PH_BYTES);   // Wh_hi, Wh_lo
+            const uint64_t dWxl = desc_advance(dWxh, tcx_blob::p0_bytes(kgx));                              // Wx_lo
+            const uint64_t dWhh = desc_advance(dWxl, tcx_blob::p1_bytes(kgx)), dWhl = desc_advance(dWhh, tcx_blob::ph_bytes(H));   // Wh_hi, Wh_lo
             const uint32_t xh = tmem + XH_COL, xl = tmem + XL_COL, hl = tmem + HL_COL;
             const uint32_t nxp = (uint32_t)(kgx + PIECE_KG - 1) / PIECE_KG;
             constexpr uint32_t KS_B = 2 * LBO_B >> 4, KS_A = 2 * LBO_A >> 4;                      // descriptor steps of one K = 16
@@ -423,19 +390,6 @@ __global__ void __launch_bounds__(THREADS, 1) lstm_small_tcxs_kernel(const __gri
     if (warp == CTRL_WARP) tmem_dealloc<1>(tmem, TMEM_COLS);
 }
 
-bool supported(int Hh, int I, int L, int T, int O, long long E, int n) {
-    return Hh == H && L >= 2 && L <= MAX_L && T >= 1 && T <= 40 && I >= 1 && ape_pack_kin_pad(0, I, H) <= H && O >= 1 && O <= NO &&
-           E >= 0 && n >= 1 && E * n <= (long long)ROWS * MAX_CLUSTERS;
-}
-
-static size_t cluster_ws_bytes(int T) { return (size_t)(2 + 2 * T) * 2 * KG * ROWS * 16; }      // hx + seq (hi and lo) of one cluster
-size_t workspace_bytes(int T, long long rows) {
-    const long long clusters = rows <= 0 ? 1 : (rows + ROWS - 1) / ROWS;
-    return cluster_ws_bytes(T) * (size_t)clusters + 256;
-}
-
-static size_t layer_bytes(int layer, int I) { return (size_t)2 * NCHL * chunk_bytes(layer == 0 ? ape_pack_kin_pad(0, I, H) / 8 : KG); }
-
 // the launch configuration of `clusters` clusters (a 16-CTA cluster is a non-portable size: the kernel opts in first)
 static cudaError_t launch_config(int clusters, cudaStream_t st, cudaLaunchConfig_t& cfg, cudaLaunchAttribute* attr) {
     cudaError_t e = cudaFuncSetAttribute(lstm_small_tcxs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM);
@@ -465,34 +419,7 @@ int max_active_clusters(int* clusters) {
     return APE_OK;
 }
 
-// all layers of the call `g` (ape_mc_lstm_tcxsl) from the split blob `blob` (weights_tcx); shapes already checked
-int run(const ape_lstm_args* g, const uint8_t* blob, void* workspace, cudaStream_t st) {
-    Args a{};
-    const uint8_t* p = blob;
-    for (int l = 0; l < g->L; ++l) {
-        a.W[l] = p;
-        a.kgx[l] = l == 0 ? ape_pack_kin_pad(0, g->I, H) / 8 : KG;
-        p += layer_bytes(l, g->I);
-    }
-    const long long E = (long long)g->B * g->nF;
-    a.L = g->L; a.T = g->T; a.I = g->I; a.E = (int)E; a.n = g->n_samples; a.nF = g->nF; a.frame0 = g->frame0; a.feat_ring = g->feat_ring;
-    a.dense = g->x_dense != nullptr;
-    a.in = g->x_dense ? g->x_dense : g->feat_ring_buf;
-    a.stream_frames = g->stream_frames;
-    a.mask_mode = g->mask_mode; a.masks = g->masks;
-    a.rk = philox_round_keys(g->philox_seed);
-    a.stream_id0 = g->stream_id0;
-    a.keep_thr16 = keep_threshold16(g->dropout_p);
-    a.scale = g->mask_mode == APE_MASK_NONE ? 1.0f : 1.0f / (1.0f - g->dropout_p);
-    char* ws = (char*)(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-    a.hx = (uint4*)ws;
-    a.seq = (uint4*)(ws + (size_t)2 * 2 * KG * ROWS * 16);
-    a.ws_stride = cluster_ws_bytes(g->T) / 16;
-    const int clusters = (int)((E * g->n_samples + ROWS - 1) / ROWS);
-    a.Wo16 = p;                                          // the output-layer tiles follow the last layer
-    a.bo = g->weights + ape_pack_out_offset(g->I, g->H, g->L) + (size_t)g->O * g->H;
-    a.O = g->O;
-    a.preds = g->preds; a.pred_ring = g->pred_ring;
+int run(const tc::ClusterArgs& a, int clusters, cudaStream_t st) {
     cudaLaunchConfig_t cfg;
     cudaLaunchAttribute attr[1];
     APE_CUDA_TRY(launch_config(clusters, st, cfg, attr));

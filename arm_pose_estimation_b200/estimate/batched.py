@@ -263,7 +263,6 @@ class BatchedEstimator:
                 self.tc_weights = torch.from_numpy(nn_models.pack_lstm_weights_tc(state)).to(dev)
                 assert self.tc_weights.numel() == N.tc_blob_bytes(self.I, self.H, self.L)
                 ws_tc = N.workspace_bytes(self.I, self.H, self.L, self.T, self.O, B * nF, self.n, tensor_core=True) + 3 * 256 * self.T * self.H * 4
-                ws_tc += (2 + 2 * self.T) * (self.H // 8) * 2048 + 512          # (the small-batch kernel's exchange buffer and layer sequences)
                 if ws_tc > self.workspace.numel():
                     self.workspace = torch.empty(ws_tc, dtype=torch.uint8, device=dev)
                 self.tc_probe_error_m = self._probe_tc_error()
